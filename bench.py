@@ -4,12 +4,13 @@
     python bench.py [--gpus N] [--steps K] [--warmup W]          # this repo's CUDA path
     python bench.py --impl reference [...]                        # the reference's CPU algorithm
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N  # one rank per GPU (N > 1)
+    python bench.py ... --dump-outputs DIR                        # also save the last timed step's outputs (.npy)
 
 A step = DarkPose target encoding (joints -> targets, weights), masked-MSE forward+backward (pred, targets, weights ->
 loss, grad) and GaussTaylor decode (pred, trans_inv -> keypoints, scores) of the same predicted heatmaps (K = 17, 64x48
 float32), issued as BATCH-sized launches of the one-launch step kernel (sp_step_f32) over distinct buffer sets (working
-set >> the 126 MB L2, so every launch streams from HBM); ceil(500 / --steps) passes over the buffer sets make one step, so
-that the timed region lasts about half a second whatever --steps is. With N > 1 every rank does the same amount of work
+set >> the 126 MB L2, so every launch streams from HBM); one pass over the buffer sets (--persons persons per GPU) makes
+one step, and exactly --steps steps are timed. With N > 1 every rank does the same amount of work
 on its own persons (weak scaling) and the decoded keypoints of a step are all-gathered over NCCL (double-buffered,
 overlapped with the next step).
 
@@ -33,6 +34,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # a benchmark run leaves the tree as it found it (it may be read-only)
 
 import torch  # noqa: E402
 
@@ -56,6 +58,8 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-eval", action="store_true", help="skip the cfg-5 eval job")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (see dump_outputs)")
     return ap.parse_args()
 
 
@@ -232,6 +236,8 @@ def cpu_reference_rates(persons, height, width, threads, reps=3, encode_workers=
 
 
 def run_reference(args):
+    if args.dump_outputs:
+        raise SystemExit("bench.py: --dump-outputs writes the outputs of this repo's CUDA path; the reference arm has none")
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
@@ -241,17 +247,9 @@ def run_reference(args):
     ref = CpuReference(sample, args.height, args.width, cores, encode_workers=workers)
     try:
         ref.prepare_pred()
-        t0 = time.perf_counter()
         for _ in range(args.warmup):
             ref.timed_step()
-            if time.perf_counter() - t0 > 60:
-                break
-        times = []
-        t0 = time.perf_counter()
-        for _ in range(args.steps):
-            times.append(ref.timed_step())
-            if time.perf_counter() - t0 > 180:
-                break
+        times = [ref.timed_step() for _ in range(args.steps)]
     finally:
         ref.close()
     total = sum(t["step"] for t in times)
@@ -604,13 +602,12 @@ def eval_job_numbers(device, world, rank, persons=104000, mean_group=20.0, heigh
             "decode_read_GBps_per_gpu": (n * (17 * height * width * 4)) / (ms * 1e-3) / 1e9}
 
 
-def step_cycles(steps):
-    """Passes over the rotating buffer sets per step, chosen from --steps alone (both arms and every rank derive the
-    same number) so that the timed region of the product arm lasts about half a second even when few steps are asked
-    for (the driver's --steps 20 used to time 27 ms, two clock samples)."""
-    if os.environ.get("SP_BENCH_CYCLES"):          # profiling aid (ncu launch lists): fewer launches per step
+def step_cycles():
+    """Passes over the rotating buffer sets per step: one, so that a step is a fixed amount of work (--persons persons
+    per GPU) and --steps sets how much work is timed. SP_BENCH_CYCLES overrides it (a profiling aid)."""
+    if os.environ.get("SP_BENCH_CYCLES"):
         return max(1, int(os.environ["SP_BENCH_CYCLES"]))
-    return max(1, -(-500 // max(1, int(steps))))
+    return 1
 
 
 def bench_config(args, world):
@@ -618,7 +615,7 @@ def bench_config(args, world):
     from simple_pose_b200.pipeline import ALGO_BYTES
     H, W, B = args.height, args.width, args.batch
     base = max(B, (args.persons // B) * B)
-    cycles = step_cycles(args.steps)
+    cycles = step_cycles()
     per_person = ALGO_BYTES["encode"](17, H, W) + ALGO_BYTES["loss"](17, H, W) + ALGO_BYTES["decode"](17, H, W)
     return {"workload": "cfg2+cfg1 step: DarkPose target encoding + masked joints-MSE fwd/bwd + GaussTaylor decode of the same "
                         "predicted heatmaps (+ NCCL all-gather of the keypoints when N>1), K=17, %dx%d float32" % (H, W),
@@ -627,6 +624,51 @@ def bench_config(args, world):
             "l2": "inputs larger than L2: %d distinct buffer sets of %d persons, %.0f MB of separate-kernel traffic per pass" %
                   (base // B, B, base * per_person / 1e6),
             "parallelism": "persons sharded, dp%d" % world}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_sample_size(world, P, B, H, W):
+    """Persons in the targets / gradient sample of `dump_outputs`: what fits in 64 MB beside the keypoints, losses and
+    weights (4 KB kept for the .npy headers). Every rank calls it before the timed steps, so a table too large to dump
+    stops all ranks there."""
+    fixed = world * P * 17 * 3 * 4 + (P // B) * 4 + P * 17 * 4
+    n = min(P, (DUMP_LIMIT_BYTES - 4096 - fixed) // (2 * 17 * H * W * 4 + 8))
+    if n < 1:
+        raise SystemExit("bench.py: --dump-outputs: the keypoint table alone exceeds 64 MB; use fewer --persons")
+    return n
+
+
+def dump_outputs(out_dir, paths, keypoints, world, P, N, cycles, B, H, W):
+    """Writes what the last timed step handed its caller, as float32 / float64 .npy files in `out_dir`:
+
+        coords [world*P, 17, 2], maxval [world*P, 17, 1]   decoded keypoints of the step's last pass (every rank's when
+                                                           world > 1: the all-gathered table; earlier passes repeat them)
+        loss [P // B]                                      per-launch loss of this rank
+        weights [P, 17]                                    this rank's target weights
+        targets_sample, grad_sample [n, 17, H, W]          targets and loss gradient of n persons of this rank, a fixed
+        sample_persons [n] (float64)                       seeded sample (person indices) sized to keep the total <= 64 MB
+
+    The inputs depend on the flags only (seeded), so two builds run with the same flags can be compared array by array."""
+    import numpy as np
+    last = slice((cycles - 1) * P, cycles * P)
+    blocks = keypoints.view(world, N * 17 * 3)
+    out = {"coords": blocks[:, :N * 17 * 2].reshape(world, N, 17, 2)[:, last].reshape(world * P, 17, 2),
+           "maxval": blocks[:, N * 17 * 2:].reshape(world, N, 17, 1)[:, last].reshape(world * P, 17, 1),
+           "loss": torch.stack([p.loss for p in paths]),
+           "weights": torch.cat([p.weights for p in paths])}
+    out = {k: v.cpu().numpy() for k, v in out.items()}
+    n = dump_sample_size(world, P, B, H, W)
+    idx = np.sort(np.random.default_rng(2024).choice(P, size=n, replace=False))
+    out["targets_sample"] = torch.stack([paths[j // B].targets[j % B] for j in idx]).cpu().numpy()
+    out["grad_sample"] = torch.stack([paths[j // B].grad[j % B] for j in idx]).cpu().numpy()
+    out["sample_persons"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        assert a.dtype in (np.float32, np.float64), name
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    print("bench.py: wrote %s to %s" % (", ".join(sorted(out)), out_dir), file=sys.stderr, flush=True)
 
 
 def run_ours(args):
@@ -650,7 +692,9 @@ def run_ours(args):
     H, W, B = args.height, args.width, args.batch
     P = max(B, (args.persons // B) * B)          # persons per pass over the buffer sets
     nb = P // B
-    cycles = step_cycles(args.steps)
+    cycles = step_cycles()
+    if args.dump_outputs:
+        dump_sample_size(world, P, B, H, W)
 
     sets = make_inputs(P, B, H, W, device, seed=rank * 7919)
     # decoded keypoints of all batches of all passes of a step land in one flat send buffer: [N*17*2 coords | N*17
@@ -739,6 +783,9 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     ms_per_step = timed(step, args.steps)                         # THE timed region: exactly --steps steps
+    if args.dump_outputs and rank == 0:                           # before anything below overwrites the step's outputs
+        side = (state["step"] - 1) & 1
+        dump_outputs(args.dump_outputs, paths, kp_all[side] if world > 1 else kp_local[side], world, P, N, cycles, B, H, W)
     value = world * P * cycles / (ms_per_step * 1e-3)
     # per-kernel durations, still under the clock sampler
     rounds = max(3, min(20, args.steps))
