@@ -53,16 +53,12 @@ void load_tuning_locked() {
     t.loss_chunk_quads = env_or_unset("SP_LOSS_CHUNK_QUADS");
     t.loss_ring = env_or_unset("SP_LOSS_RING");
     t.loss_warps = env_or_unset("SP_LOSS_WARPS");
-    t.loss_bulk_store = env_or_unset("SP_LOSS_BULK_STORE");
     t.train_force_ldg = env_or_unset("SP_TRAIN_FORCE_LDG");
     t.train_chunk_quads = env_or_unset("SP_TRAIN_CHUNK_QUADS");
     t.train_no_tile = env_or_unset("SP_TRAIN_NO_TILE");
-    t.train_tile_cfg = env_or_unset("SP_TRAIN_TILE_CFG");
-    t.train_depth = env_or_unset("SP_TRAIN_DEPTH");
     t.train_static_pct = env_or_unset("SP_TRAIN_STATIC_PCT");
     t.train_warps = env_or_unset("SP_TRAIN_WARPS");
     t.train_ring = env_or_unset("SP_TRAIN_RING");
-    t.train_bulk_store = env_or_unset("SP_TRAIN_BULK_STORE");
     t.decode_force_generic = env_or_unset("SP_DECODE_FORCE_GENERIC");
     t.decode_warps = env_or_unset("SP_DECODE_WARPS");
     t.decode_stages = env_or_unset("SP_DECODE_STAGES");

@@ -34,9 +34,8 @@ static inline int sp_sm_count() {
 struct SpTuning {
     int no_pdl;
     int encode_warps, encode_parts;
-    int loss_force_ldg, loss_chunk_quads, loss_ring, loss_warps, loss_bulk_store;
-    int train_force_ldg, train_chunk_quads, train_no_tile, train_tile_cfg, train_depth, train_static_pct,
-        train_warps, train_ring, train_bulk_store;
+    int loss_force_ldg, loss_chunk_quads, loss_ring, loss_warps;
+    int train_force_ldg, train_chunk_quads, train_no_tile, train_static_pct, train_warps, train_ring;
     int decode_force_generic, decode_warps, decode_stages, decode_grid_wide, decode_runtime_ksize, decode_static_pct;
     int step_warps, step_static_pct;
     int nms_serial;
@@ -152,19 +151,6 @@ __device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gmem_src, u
         "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar))
         : "memory");
 }
-
-// ---- 1-D bulk copy shared -> global (the TMA store path), tracked by bulk async-groups -------------------
-// The shared-memory source must have been written (generic proxy) and fenced with fence_proxy_async_smem()
-// before the copy is issued, and must not be overwritten until wait_group_read says the engine has read it.
-__device__ __forceinline__ void bulk_s2g(void* gmem_dst, const void* smem_src, uint32_t bytes) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gmem_dst), "r"(smem_u32(smem_src)), "r"(bytes)
-                 : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
-template <int N>
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group %0;" ::"n"(N) : "memory"); }
 
 // ---- NaN-propagating max (max.NaN.f32) ------------------------------------------------------
 __device__ __forceinline__ float fmax_nan(float a, float b) {

@@ -169,12 +169,9 @@ mse_mixed_kernel(const PT* __restrict__ pred, const float* __restrict__ target, 
 // dynamic smem: [mbarriers 1024 B][per warp: ring x (pred chunk | target chunk)]
 constexpr int kRingBarBytes = 1024;
 
-// BULK_STORE: the gradient leaves through the TMA as well. A lane overwrites the pred quad it has just consumed
-// with the gradient quad (a 16-byte shared store instead of a 16-byte global store), and once the chunk is done
-// lane 0 hands the whole 3 KB to the copy engine (cp.async.bulk shared -> global, one bulk group per chunk). The
-// slot is re-armed one iteration later, after cp.async.bulk.wait_group.read has confirmed that the engine has read
-// it -- so of `ring` slots one is being consumed, one is draining and ring - 2 are being filled.
-template <bool WRITE_GRAD, bool BULK_STORE>
+// A variant that sent the gradient out through the TMA too (written into the drained slot, cp.async.bulk shared -> global)
+// was within 1-2 % either way warm and 12 % slower from a cold cache, so the gradient stays on register stores (DESIGN.md, section 4).
+template <bool WRITE_GRAD>
 __global__ void __launch_bounds__(1024, 1)
 mse_ring_kernel(const float* __restrict__ pred, const float* __restrict__ target, const float* __restrict__ mask,
                 float* __restrict__ grad, float* __restrict__ loss, MseWorkspace* __restrict__ ws,
@@ -216,11 +213,10 @@ mse_ring_kernel(const float* __restrict__ pred, const float* __restrict__ target
     double sum_sq = 0.0;
     int cs = 0;
     uint32_t parity = 0;
-    bool draining = false;          // BULK_STORE: the slot consumed in the previous iteration awaits its refill
     for (long long i = lo + warp; i < hi; i += nwarps) {
         const float mk = __ldg(mask + i / chunks_per_map);          // latency hidden behind the wait below
         sp::mbar_wait(bars + cs, parity);
-        float4* p4 = reinterpret_cast<float4*>(slots + (size_t)cs * 2 * chunk_bytes);
+        const float4* p4 = reinterpret_cast<const float4*>(slots + (size_t)cs * 2 * chunk_bytes);
         const float4* t4 = reinterpret_cast<const float4*>(slots + (size_t)cs * 2 * chunk_bytes + chunk_bytes);
         float4* g4 = reinterpret_cast<float4*>(grad + i * chunk_floats);
         float acc = 0.f;
@@ -234,30 +230,16 @@ mse_ring_kernel(const float* __restrict__ pred, const float* __restrict__ target
             d = sq_err_and_grad(p.y, t.y, mk, norm, half_scale, g.y); acc = fmaf(d, d, acc);
             d = sq_err_and_grad(p.z, t.z, mk, norm, half_scale, g.z); acc = fmaf(d, d, acc);
             d = sq_err_and_grad(p.w, t.w, mk, norm, half_scale, g.w); acc = fmaf(d, d, acc);
-            if (WRITE_GRAD) {
-                if (BULK_STORE) p4[q] = g;      // the quad this lane has just read
-                else            g4[q] = g;
-            }
+            if (WRITE_GRAD) g4[q] = g;
         }
         sum_sq += (double)acc;
         __syncwarp();
         if (lane == 0) {
             sp::fence_proxy_async_smem();
-            if (BULK_STORE && WRITE_GRAD) {
-                sp::bulk_s2g(g4, p4, chunk_bytes);
-                sp::bulk_commit();
-                if (draining) {
-                    sp::bulk_wait_read<1>();                        // the previous chunk's store has left shared memory
-                    issue_next();                                   // refills the slot drained one iteration ago
-                }
-            } else {
-                issue_next();                                       // refills the slot just drained
-            }
+            issue_next();                                           // refills the slot just drained
         }
-        draining = true;
         if (++cs == ring) { cs = 0; parity ^= 1u; }
     }
-    if (BULK_STORE && WRITE_GRAD && lane == 0) sp::bulk_wait_all<0>();   // all gradient bytes are in global memory
 #ifdef SP_TRAIN_TRACE
     if (lane == 0 && g_loss_trace_ptr) {
         unsigned smid;
@@ -330,15 +312,11 @@ extern "C" int sp_mse_fwd_bwd_f32(const float* pred, const float* target, const 
                 const long long nchunks = (long long)nmaps * (nq / chunk_quads);
                 int grid = sp_sm_count();
                 if ((long long)grid * nwarps > nchunks) grid = (int)((nchunks + nwarps - 1) / nwarps);
-                const bool bulk = sp_knob(tune.loss_bulk_store, 0) == 1 && ring >= 2;
-                if (grad && bulk) {
-                    SP_CUDA(sp_launch_smem(mse_ring_kernel<true, true>, dim3(grid), dim3(nwarps * 32), smem, st, pred, target, mask, grad, loss, ws,
-                                      nchunks, chunk_quads, nq / chunk_quads, nwarps, ring, norm, half_scale, 1.0 / count));
-                } else if (grad) {
-                    SP_CUDA(sp_launch_smem(mse_ring_kernel<true, false>, dim3(grid), dim3(nwarps * 32), smem, st, pred, target, mask, grad, loss, ws,
+                if (grad) {
+                    SP_CUDA(sp_launch_smem(mse_ring_kernel<true>, dim3(grid), dim3(nwarps * 32), smem, st, pred, target, mask, grad, loss, ws,
                                       nchunks, chunk_quads, nq / chunk_quads, nwarps, ring, norm, half_scale, 1.0 / count));
                 } else {
-                    SP_CUDA(sp_launch_smem(mse_ring_kernel<false, false>, dim3(grid), dim3(nwarps * 32), smem, st, pred, target, mask, grad, loss, ws,
+                    SP_CUDA(sp_launch_smem(mse_ring_kernel<false>, dim3(grid), dim3(nwarps * 32), smem, st, pred, target, mask, grad, loss, ws,
                                       nchunks, chunk_quads, nq / chunk_quads, nwarps, ring, norm, half_scale, 1.0 / count));
                 }
                 return 0;

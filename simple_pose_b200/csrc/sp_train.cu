@@ -191,10 +191,11 @@ encode_mse_ring_kernel(const MapIo io, float* __restrict__ loss, MseWorkspace* _
 // Why it matters: with 16 warps per SM each warp issues about one instruction every 8 cycles, so
 // the kernel's time is (instructions per quad) x latency until the copy engine becomes the limit.
 // dynamic smem: same layout as variant B
-template <int QPR, int PPC, int RING, bool ACC, bool BULK = false>
+template <int QPR, int PPC, int RING, bool ACC>
 __global__ void __launch_bounds__(512, 1)
 encode_mse_tile_kernel(const MapIo io, float* __restrict__ loss, MseWorkspace* __restrict__ ws, double inv_count, int nwarps,
-                       int depth, int static_maps) {
+                       int depth,   // == RING; making it compile-time reschedules the kernel, a change to measure on its own
+                       int static_maps) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr int CHUNK_BYTES = PPC * 32 * Tile<QPR>::PERIOD * 16;
     const int lane = threadIdx.x & 31;
@@ -213,7 +214,7 @@ encode_mse_tile_kernel(const MapIo io, float* __restrict__ loss, MseWorkspace* _
     rg.bar0 = base + (uint32_t)(warp * RING * 8);
     rg.slot0 = base + (uint32_t)(kRingHeader + (size_t)nwarps * fac_bytes + (size_t)warp * RING * CHUNK_BYTES);
     rg.cs = 0; rg.parity = 0; rg.ps = 0; rg.tail = 0; rg.left = 0; rg.pnext = -1; rg.src = nullptr;
-    rg.inflight = 0; rg.depth = depth; rg.stores = 0;
+    rg.inflight = 0; rg.depth = depth;
     rg.fifo = fifo; rg.next_work = &ws->next_work;
     rg.nmaps = io.nmaps;
     rg.static_stride = (int)gridDim.x * nwarps;
@@ -257,18 +258,17 @@ encode_mse_tile_kernel(const MapIo io, float* __restrict__ loss, MseWorkspace* _
         const JointVerdict jv = prepare_map<QPR>(io, m, jc, ex, ey, lane);
         float acc;
         if (jv.draw && jv.weight == 1.0f && (!ACC || io.analytic_ok))
-            acc = tile_map<QPR, PPC, ACC, 0, BULK, true, false>(io, m, jv, ex, ey, rg, pd, lane);
+            acc = tile_map<QPR, PPC, ACC, 0>(io, m, jv, ex, ey, rg, pd, lane);
         else if (!jv.draw && jv.weight == 0.0f)
-            acc = tile_map<QPR, PPC, ACC, 1, BULK, true, false>(io, m, jv, ex, ey, rg, pd, lane);
+            acc = tile_map<QPR, PPC, ACC, 1>(io, m, jv, ex, ey, rg, pd, lane);
         else
-            acc = tile_map<QPR, PPC, ACC, 2, BULK, true, false>(io, m, jv, ex, ey, rg, pd, lane);
+            acc = tile_map<QPR, PPC, ACC, 2>(io, m, jv, ex, ey, rg, pd, lane);
         sum_sq += (double)acc;
         __syncwarp();
         ++head;
         m = m_next;
     }
     if (ACC) flush_pending(io, pd, lane);
-    if (BULK && lane == 0) sp::bulk_wait_all<0>();           // every gradient byte of this warp is in global memory
 #ifdef SP_TRAIN_TRACE
     tr[3] = gtime(); tr[5] = head; tr[6] = clock64() - c0;
     { unsigned smid; asm volatile("mov.u32 %0, %%smid;" : "=r"(smid)); tr[7] = smid; }
@@ -374,19 +374,8 @@ static int encode_mse_launch(const float* joints, const void* pred_raw, int pred
     if (plain_f32 && (qpr == 12 || qpr == 18) && grad && !targets && !force_ldg && sp_knob(tune.train_no_tile, 0) == 0) {
         const int period = (qpr == 12) ? Tile<12>::PERIOD : Tile<18>::PERIOD;
         const int rows = (qpr == 12) ? Tile<12>::ROWS : Tile<18>::ROWS;
-        // tuned layouts (PPC periods per chunk, ring depth); SP_TRAIN_TILE_CFG picks another compiled one
-        const int cfg = sp_knob(tune.train_tile_cfg, 0);
-        int ppc = 1, ring = 2;
-        if (qpr == 12) {
-            if (cfg == 1) { ppc = 1; ring = 2; } else if (cfg == 2) { ppc = 2; ring = 2; } else if (cfg == 3) { ppc = 4; ring = 1; }
-            else if (cfg == 4) { ppc = 2; ring = 3; } else if (cfg == 5) { ppc = 2; ring = 4; } else { ppc = 2; ring = 1; }
-        } else {
-            if (cfg == 1) { ppc = 1; ring = 1; } else if (cfg == 2) { ppc = 1; ring = 3; } else if (cfg == 3) { ppc = 1; ring = 4; } else { ppc = 1; ring = 2; }
-        }
-        // copies kept in flight per warp in steady state (the whole ring is used once a warp is on its last map)
-        int depth = sp_knob(tune.train_depth, ring);
-        if (depth < 1) depth = 1;
-        if (depth > ring) depth = ring;
+        // the tuned layouts (PPC periods per chunk, RING slots per warp): (2, 1) at W = 48, (1, 2) at W = 72
+        const int ppc = (qpr == 12) ? 2 : 1, ring = (qpr == 12) ? 1 : 2;
         const int periods = nq / (32 * period);
         if (H % rows == 0 && periods % ppc == 0) {
             const size_t chunk_bytes = (size_t)ppc * 32 * period * 16;
@@ -412,32 +401,13 @@ static int encode_mse_launch(const float* joints, const void* pred_raw, int pred
 #define SP_LAUNCH_TILE(Q, P, R)                                                                                              \
     do {                                                                                                                     \
         if (pred_xy) {                                                                                                       \
-            SP_CUDA(sp_launch_smem(encode_mse_tile_kernel<Q, P, R, true>, dim3(grid), dim3(nwarps * 32), smem, st, io, loss, ws, 1.0 / count, nwarps, depth, static_maps)); \
+            SP_CUDA(sp_launch_smem(encode_mse_tile_kernel<Q, P, R, true>, dim3(grid), dim3(nwarps * 32), smem, st, io, loss, ws, 1.0 / count, nwarps, ring, static_maps)); \
         } else {                                                                                                             \
-            SP_CUDA(sp_launch_smem(encode_mse_tile_kernel<Q, P, R, false>, dim3(grid), dim3(nwarps * 32), smem, st, io, loss, ws, 1.0 / count, nwarps, depth, static_maps)); \
+            SP_CUDA(sp_launch_smem(encode_mse_tile_kernel<Q, P, R, false>, dim3(grid), dim3(nwarps * 32), smem, st, io, loss, ws, 1.0 / count, nwarps, ring, static_maps)); \
         }                                                                                                                    \
     } while (0)
-                // SP_TRAIN_BULK_STORE=1: the gradient leaves through the TMA too (ring >= 2; the start-up depth is the whole ring)
-                const bool bulk = sp_knob(tune.train_bulk_store, 0) == 1 && ring >= 2 && ((qpr == 12 && ppc == 2 && ring <= 4) || (qpr == 18 && ring <= 3));
-                if (bulk) {
-#define SP_LAUNCH_TILE_BULK(Q, P, R)                                                                                         \
-    do {                                                                                                                     \
-        if (pred_xy) SP_CUDA(sp_launch_smem(encode_mse_tile_kernel<Q, P, R, true, true>, dim3(grid), dim3(nwarps * 32), smem, st, io, loss, ws, 1.0 / count, nwarps, R, static_maps)); \
-        else         SP_CUDA(sp_launch_smem(encode_mse_tile_kernel<Q, P, R, false, true>, dim3(grid), dim3(nwarps * 32), smem, st, io, loss, ws, 1.0 / count, nwarps, R, static_maps)); \
-    } while (0)
-                    if (qpr == 12) { if (ring == 2) SP_LAUNCH_TILE_BULK(12, 2, 2); else if (ring == 3) SP_LAUNCH_TILE_BULK(12, 2, 3); else SP_LAUNCH_TILE_BULK(12, 2, 4); }
-                    else           { if (ring == 2) SP_LAUNCH_TILE_BULK(18, 1, 2); else SP_LAUNCH_TILE_BULK(18, 1, 3); }
-#undef SP_LAUNCH_TILE_BULK
-                    return 0;
-                }
-                if (qpr == 12) {
-                    if (ppc == 1) SP_LAUNCH_TILE(12, 1, 2); else if (ppc == 2 && ring == 2) SP_LAUNCH_TILE(12, 2, 2);
-                    else if (ppc == 2 && ring == 3) SP_LAUNCH_TILE(12, 2, 3); else if (ppc == 2 && ring == 4) SP_LAUNCH_TILE(12, 2, 4);
-                    else if (ppc == 4) SP_LAUNCH_TILE(12, 4, 1); else SP_LAUNCH_TILE(12, 2, 1);
-                } else {
-                    if (ring == 1) SP_LAUNCH_TILE(18, 1, 1); else if (ring == 3) SP_LAUNCH_TILE(18, 1, 3);
-                    else if (ring == 4) SP_LAUNCH_TILE(18, 1, 4); else SP_LAUNCH_TILE(18, 1, 2);
-                }
+                if (qpr == 12) SP_LAUNCH_TILE(12, 2, 1);
+                else           SP_LAUNCH_TILE(18, 1, 2);
 #undef SP_LAUNCH_TILE
                 return 0;
             }

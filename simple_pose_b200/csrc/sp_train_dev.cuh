@@ -298,7 +298,7 @@ __device__ __forceinline__ JointVerdict prepare_map(const MapIo& io, int m, cons
 }
 
 
-// ---- period-tiled map body (variant C of sp_train.cu; also the loss pass of the step kernel, sp_step.cu) ----------
+// ---- period-tiled map body (variant C of sp_train.cu) ----------------------------------------------------------------
 constexpr int kFifo = 16;          // entries per warp; the producer is never more than ring+2 <= 10 maps ahead
 constexpr int kRingHeader = 1024 + 2048 + 64;
 
@@ -413,30 +413,6 @@ struct TileRing {
         }
         return slot0 + cs * (uint32_t)CHUNK_BYTES;
     }
-    // BULK variant of release: the lanes have overwritten the chunk in place with the gradient; lane 0 hands the
-    // slot to the copy engine (cp.async.bulk shared -> global) and, one release later, re-arms it -- after
-    // cp.async.bulk.wait_group.read 1 has confirmed that every store but the newest has left shared memory.
-    // Of RING slots one is being consumed, one is draining, RING - 2 are being filled.
-    int stores;
-    __device__ __forceinline__ void release_store(int lane, void* gdst) {
-        __syncwarp();
-        if (lane == 0) {
-            sp::fence_proxy_async_smem();
-            const uint32_t src_slot = slot0 + cs * (uint32_t)CHUNK_BYTES;
-            asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(src_slot), "n"(CHUNK_BYTES) : "memory");
-            sp::bulk_commit();
-            --inflight;
-            if (stores++ > 0) {
-                sp::bulk_wait_read<1>();
-                issue_next();
-            }
-        }
-        if (RING > 1) {
-            if (++cs == RING) { cs = 0; parity ^= 1u; }
-        } else {
-            parity ^= 1u;
-        }
-    }
     __device__ __forceinline__ void release(int lane) {
         __syncwarp();
         if (lane == 0) {
@@ -468,27 +444,14 @@ __device__ __forceinline__ void flush_pending(const MapIo& io, PendingAxis& pd, 
     pd.m = -1;
 }
 
+// One map, its chunks arriving through the warp's TileRing: writes the gradient (never the targets), returns this
+// lane's share of sum((m*p - m*t)^2) and, with ACC, the HeatMapAcc coordinates.
 // MODE 0: Gaussian drawn, mask == 1, argmax tracked iff ACC (the common case);
 // MODE 1: nothing drawn and mask == 0 (invisible / culled joint): target 0, no tracking;
 // MODE 2: anything else (odd mask values, sigma outside the analytic range): run-time flags.
-__device__ __forceinline__ void sts128(uint32_t addr, float4 v) {
-    asm volatile("st.shared.v4.f32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-}
-
-// The whole predicted map already staged in shared memory (the step kernel): same interface as TileRing, no copies.
-template <int CHUNK_BYTES>
-struct StagedMap {
-    uint32_t next;               // shared address of the next chunk
-    __device__ __forceinline__ uint32_t wait() { return next; }
-    __device__ __forceinline__ void release(int) { next += (uint32_t)CHUNK_BYTES; }
-    __device__ __forceinline__ void release_store(int, void*) { next += (uint32_t)CHUNK_BYTES; }
-};
-
-// Ring = TileRing<RING, chunk bytes> (chunks arrive through the per-warp TMA ring) or StagedMap<chunk bytes>.
-// WRITE_GRAD / WRITE_TARGETS: which of the two map-sized outputs are stored (the training kernel: grad only).
-template <int QPR, int PPC, bool ACC, int MODE, bool BULK, bool WRITE_GRAD, bool WRITE_TARGETS, typename Ring>
+template <int QPR, int PPC, bool ACC, int MODE, int RING, int CHUNK_BYTES>
 __device__ __forceinline__ float tile_map(const MapIo& io, int m, const JointVerdict& jv, const double* ex, const double* ey,
-                                          Ring& rg, PendingAxis& pd, int lane) {
+                                          TileRing<RING, CHUNK_BYTES>& rg, PendingAxis& pd, int lane) {
     using T = Tile<QPR>;
     constexpr int PERIOD = T::PERIOD, ROWS = T::ROWS;
     constexpr int CHUNK_QUADS = PPC * 32 * PERIOD;
@@ -524,7 +487,6 @@ __device__ __forceinline__ float tile_map(const MapIo& io, int m, const JointVer
     int bq = lane, tbq = lane;
     int qlane = lane;                                   // this lane's quad at step 0 of the current chunk
     float4* g4 = reinterpret_cast<float4*>(io.grad + (size_t)m * hw) + lane;
-    float4* t4 = reinterpret_cast<float4*>(io.targets + (size_t)m * hw) + lane;
     const int chunks = (hw >> 2) / CHUNK_QUADS;
 
 #pragma unroll 1
@@ -534,8 +496,6 @@ __device__ __forceinline__ float tile_map(const MapIo& io, int m, const JointVer
         for (int it = 0; it < PPC; ++it) {
 #pragma unroll
             for (int j = 0; j < PERIOD; ++j) {
-                constexpr int kDummy = 0;
-                (void)kDummy;
                 const int step = it * PERIOD + j;
                 const float4 p = lds128(chunk + 512u * step);
                 float4 t = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -562,19 +522,15 @@ __device__ __forceinline__ float tile_map(const MapIo& io, int m, const JointVer
                 acc = fmaf(dy, dy, acc);
                 acc = fmaf(dz, dz, acc);
                 acc = fmaf(dw, dw, acc);
-                if (WRITE_GRAD) {
-                    float4 g;
-                    g.x = __fmul_rn(__fmul_rn(norm, dx), half_scale);
-                    g.y = __fmul_rn(__fmul_rn(norm, dy), half_scale);
-                    g.z = __fmul_rn(__fmul_rn(norm, dz), half_scale);
-                    g.w = __fmul_rn(__fmul_rn(norm, dw), half_scale);
-                    if (!unit) {
-                        g.x = __fmul_rn(g.x, mk); g.y = __fmul_rn(g.y, mk); g.z = __fmul_rn(g.z, mk); g.w = __fmul_rn(g.w, mk);
-                    }
-                    if (BULK) sts128(chunk + 512u * step, g);      // in place: this lane has just read these 16 bytes
-                    else      g4[32 * step] = g;
+                float4 g;
+                g.x = __fmul_rn(__fmul_rn(norm, dx), half_scale);
+                g.y = __fmul_rn(__fmul_rn(norm, dy), half_scale);
+                g.z = __fmul_rn(__fmul_rn(norm, dz), half_scale);
+                g.w = __fmul_rn(__fmul_rn(norm, dw), half_scale);
+                if (!unit) {
+                    g.x = __fmul_rn(g.x, mk); g.y = __fmul_rn(g.y, mk); g.z = __fmul_rn(g.z, mk); g.w = __fmul_rn(g.w, mk);
                 }
-                if (WRITE_TARGETS) t4[32 * step] = t;
+                g4[32 * step] = g;
                 if (track) {
                     const float m4 = sp::fmax_nan(sp::fmax_nan(px, py), sp::fmax_nan(pz, pw));
                     if (m4 > best) bq = qlane + 32 * step;
@@ -586,10 +542,8 @@ __device__ __forceinline__ float tile_map(const MapIo& io, int m, const JointVer
                 }
             }
         }
-        if (BULK) rg.release_store(lane, g4 - lane);
-        else      rg.release(lane);
+        rg.release(lane);
         g4 += CHUNK_QUADS;
-        t4 += CHUNK_QUADS;
         qlane += CHUNK_QUADS;
 #pragma unroll
         for (int j = 0; j < PERIOD; ++j) eya[j] += 8u * (uint32_t)(PPC * ROWS);

@@ -951,15 +951,11 @@ def test_cfg5_coco_val_sized_job_properties(api):
                                  {"SP_TRAIN_RING": "1"}, {"SP_TRAIN_RING": "4", "SP_TRAIN_CHUNK_QUADS": "64"},
                                  {"SP_TRAIN_CHUNK_QUADS": "768", "SP_TRAIN_RING": "1"}, {"SP_TRAIN_WARPS": "1", "SP_TRAIN_RING": "8"},
                                  {"SP_TRAIN_NO_TILE": "1"}, {"SP_TRAIN_NO_TILE": "1", "SP_TRAIN_RING": "3", "SP_TRAIN_WARPS": "5"},
-                                 {"SP_TRAIN_TILE_CFG": "1"}, {"SP_TRAIN_TILE_CFG": "2", "SP_TRAIN_WARPS": "3"},
-                                 {"SP_TRAIN_TILE_CFG": "3", "SP_TRAIN_WARPS": "7"}, {"SP_TRAIN_WARPS": "1"}, {"SP_NO_PDL": "1"},
-                                 # the gradient leaving through the TMA (cp.async.bulk shared -> global), rings of 2 / 3 / 4 slots
-                                 {"SP_TRAIN_BULK_STORE": "1", "SP_TRAIN_TILE_CFG": "2"}, {"SP_TRAIN_BULK_STORE": "1", "SP_TRAIN_TILE_CFG": "4"},
-                                 {"SP_TRAIN_BULK_STORE": "1", "SP_TRAIN_TILE_CFG": "5", "SP_TRAIN_WARPS": "3"}])
+                                 {"SP_TRAIN_WARPS": "3"}, {"SP_TRAIN_WARPS": "7"}, {"SP_TRAIN_WARPS": "1"}, {"SP_NO_PDL": "1"}])
 @pytest.mark.parametrize("hw", [(64, 48), (96, 72)])
 def test_fused_kernel_variants_agree(api, env, hw):
-    """Every chunk/ring/warp layout of the period-tiled kernel, the generic TMA ring and the
-    plain-load variant give identical outputs (weights 0, 1 and odd values all present)."""
+    """The period-tiled kernel with full and partial CTAs, every chunk/ring/warp layout of the generic
+    TMA ring and the plain-load variant give identical outputs (weights 0, 1 and odd values all present)."""
     h, w = hw
     joints = synth.joints(40, height=h, width=w, seed=81)
     joints[3, :, 2] = 2.0
@@ -1040,9 +1036,7 @@ def test_fused_label_argmax_ties_and_outside_centres(api):
                                  {"SP_LOSS_WARPS": "7", "SP_LOSS_RING": "4", "SP_LOSS_CHUNK_QUADS": "64"},
                                  {"SP_LOSS_WARPS": "32", "SP_LOSS_RING": "2", "SP_LOSS_CHUNK_QUADS": "96"},
                                  {"SP_LOSS_CHUNK_QUADS": "768", "SP_LOSS_RING": "8"},
-                                 {"SP_LOSS_CHUNK_QUADS": "100"}, {"SP_NO_PDL": "1"},
-                                 {"SP_LOSS_BULK_STORE": "1"}, {"SP_LOSS_BULK_STORE": "1", "SP_LOSS_RING": "2", "SP_LOSS_WARPS": "1"},
-                                 {"SP_LOSS_BULK_STORE": "1", "SP_LOSS_RING": "5", "SP_LOSS_CHUNK_QUADS": "96"}])
+                                 {"SP_LOSS_CHUNK_QUADS": "100"}, {"SP_NO_PDL": "1"}])
 @pytest.mark.parametrize("b,hw", [(40, (64, 48)), (3, (96, 72)), (9, (20, 12))])
 def test_loss_kernel_variants_agree(api, env, b, hw):
     """Every chunk/ring/warp layout of the TMA-ring loss kernel, the plain-load fallback and the
