@@ -18,7 +18,7 @@
  *     SP_ERR_* codes (< 0) for argument errors; sp_error_string() names any of them.
  *     No exception crosses the boundary;
  *   - stateless and re-entrant; the only per-call scratch is the workspace the caller hands
- *     to sp_mse_fwd_bwd_f32.
+ *     to the entry points that take one.
  */
 #ifndef SIMPLE_POSE_B200_H
 #define SIMPLE_POSE_B200_H
@@ -288,6 +288,44 @@ int sp_eval_rows_nms_fanout_f32(float* rows, int row_stride, const double* box_s
  * rows [N, 3K+1] f32 = (x, y, conf) * K from coords [N,K,2] / maxval [N,K], then the person score
  * mean(conf) + max(conf) (mean accumulated in float64, rounded once; NaN propagates). */
 int sp_person_rows_f32(const float* coords, const float* maxval, float* rows, int N, int K, void* stream);
+
+/* ------------------------------------------------------------------------------------------
+ * A11 COCO keypoint AP: pycocotools' COCOeval(cocoGt, cocoDt, 'keypoints') with the keypoint defaults,
+ *     catIds = [1] and maxDets = [20] -- evaluate(), accumulate() and the ten statistics of summarize()
+ *     (eval.py:13-27, metrics/pose_metrics.py:182-209), without the result JSON file.
+ *
+ * Detections (N):
+ *   det_rows   [N, det_stride] f32: x of joint k at 3k, y at 3k+1 (the eval table, stride 3K+3, and the
+ *              kps_to_dict_ table, stride 3K+1, both fit); det_stride >= 3K
+ *   det_scores [N] f64; det_img [N] i32: position of the detection's image in the evaluated image list;
+ *              a detection with a position outside [0, I) is not evaluated; det_keep [N] u8 (NULL = all; 0 = not
+ *              evaluated). Within an image the input order decides equal scores, as the results-list order does.
+ * Ground truth (G persons, I evaluated images in params.imgIds order, parsed on the host once):
+ *   gt_seg [I+1] i32 offsets (image i owns GT gt_seg[i]..gt_seg[i+1]-1, in annotation-file order);
+ *   gt_kps [G, 3K] f64 (x, y, v); gt_area [G] f64; gt_bbox [G, 4] f64 (x, y, w, h);
+ *   gt_flags [G] u8: bit 0 = ignore (iscrowd or num_keypoints == 0), bit 1 = iscrowd.
+ * Parameters, computed on the host with NumPy exactly as Params.setKpParams does: iou_thrs [T] f64,
+ *   rec_thrs [R] f64, area_rng [A, 2] f64. Anything but K = 17, T = 10, R = 101, A = 3, max_dets = 20:
+ *   SP_ERR_UNSUPPORTED.
+ * Outputs (f64, device): precision [T, R, A] and recall [T, A] (COCOeval's eval['precision'][:, :, 0, :, 0] and
+ *   eval['recall'][:, 0, :, 0]; -1 where an area range has no non-ignored GT), stats [10] (summarize()).
+ * Optional diagnostics (NULL = not written): oks_out [20 * G] f64: image i's [D_i, G_i] OKS matrix (detections
+ *   ranked by score and cut to 20, GT in file order) row-major from oks_out + 20 * gt_seg[i]; det_flags_out
+ *   [I * 20] u64 and det_order_out [I * 20] i32 per slot i * 20 + rank: bit (a * T + t) of the low word = matched
+ *   at area range a and threshold t, of the high word = ignored; the detection's index (-1 = empty slot).
+ * workspace: sp_coco_eval_workspace_bytes(N, I, G) bytes (0 = invalid sizes or no CUDA device), 16-byte aligned.
+ *   Its contents on entry do not matter (every call writes what it reads), so it need not be zeroed; calls that
+ *   may run concurrently need separate workspaces. No host synchronisation. */
+size_t sp_coco_eval_workspace_bytes(int num_dets, int num_images, int num_gts);
+int sp_coco_eval_kps_f32(const float* det_rows, int det_stride, const double* det_scores, const int* det_img,
+                         const unsigned char* det_keep, int num_dets,
+                         const double* gt_kps, const double* gt_area, const double* gt_bbox,
+                         const unsigned char* gt_flags, const int* gt_seg, int num_images, int num_gts,
+                         const double* iou_thrs, const double* rec_thrs, const double* area_rng,
+                         int K, int T, int R, int A, int max_dets,
+                         double* precision, double* recall, double* stats,
+                         double* oks_out, unsigned long long* det_flags_out, int* det_order_out,
+                         void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Eval-side caller of the decoder (SURVEY 8, "next": the data either side of the path):

@@ -62,6 +62,11 @@ SIGNATURES = {
     "sp_rescore_f64": (c_int, [c_void, c_void, c_void, c_int, c_int, c_dbl, c_void]),
     "sp_pack_kps_f64": (c_int, [c_void, c_void, c_void, c_int, c_int, c_void]),
     "sp_pack_rows_f32": (c_int, [c_void, c_void, c_void, c_void, c_void, c_int, c_int, c_void]),
+    "sp_coco_eval_workspace_bytes": (c_size, [c_int, c_int, c_int]),
+    "sp_coco_eval_kps_f32": (c_int, [c_void, c_int, c_void, c_void, c_void, c_int,
+                                     c_void, c_void, c_void, c_void, c_void, c_int, c_int,
+                                     c_void, c_void, c_void, c_int, c_int, c_int, c_int, c_int,
+                                     c_void, c_void, c_void, c_void, c_void, c_void, c_void, c_size, c_void]),
     "sp_box_affine_f64": (c_int, [c_void, c_int, c_void, c_void, c_void, c_void, c_void, c_void, c_int, c_dbl, c_int, c_int, c_flt, c_void]),
     "sp_center_scale_affine_f64": (c_int, [c_void, c_void, c_void, c_void, c_void, c_int, c_int, c_int, c_void]),
     "sp_center_scale_rot_affine_f64": (c_int, [c_void, c_void, c_void, c_void, c_void, c_void, c_int, c_int, c_int, c_void]),

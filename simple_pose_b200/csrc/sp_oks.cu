@@ -11,6 +11,7 @@
 // keeps the reference's operation order, including NumPy's 8-accumulator pairwise summation,
 // so that the `oks > thresh` decisions agree.
 #include "sp_common.cuh"
+#include "sp_numpy_sum.cuh"
 #include <math_constants.h>
 
 namespace {
@@ -21,41 +22,7 @@ constexpr int kMaxJoints = 64;
 __device__ __constant__ double kCocoSigmas[17] = {.26, .25, .25, .35, .35, .79, .79, .72, .72,
                                                   .62, .62, 1.07, 1.07, .87, .87, .89, .89};
 
-// NumPy's pairwise sum for n <= 128 fed one value at a time (numpy/core/src/umath/loops_utils:
-// 8 running accumulators, tree-combined, then the n % 8 tail added in order; for n < 8 a plain
-// running sum). The reduction starts from the identity: result = 0 + pairwise(values).
-struct NumpySum {
-    double r[8];
-    double tail;
-    int n_main, seen, n;
-    __device__ void begin(int count) {
-        n = count;
-        n_main = (count < 8) ? 0 : count - (count % 8);
-        seen = 0;
-        tail = 0.0;
-#pragma unroll
-        for (int j = 0; j < 8; ++j) r[j] = 0.0;
-    }
-    __device__ void push(double v) {
-        if (seen < n_main) {
-            const int j = seen & 7;
-            // first round initialises the accumulator (r[j] = a[j]), later rounds add
-            double cur = 0.0;
-#pragma unroll
-            for (int q = 0; q < 8; ++q) if (q == j) cur = r[q];
-            cur = (seen < 8) ? v : __dadd_rn(cur, v);
-#pragma unroll
-            for (int q = 0; q < 8; ++q) if (q == j) r[q] = cur;
-            if (seen + 1 == n_main)
-                tail = __dadd_rn(__dadd_rn(__dadd_rn(r[0], r[1]), __dadd_rn(r[2], r[3])),
-                                 __dadd_rn(__dadd_rn(r[4], r[5]), __dadd_rn(r[6], r[7])));
-        } else {
-            tail = __dadd_rn(tail, v);
-        }
-        ++seen;
-    }
-    __device__ double result() const { return __dadd_rn(0.0, tail); }
-};
+using sp::NumpySum;
 
 struct OksParams {
     const double* sigmas;    // NULL -> COCO table

@@ -2,7 +2,8 @@
 
 Used by the parity tests (generated on CPU so the oracle and the kernels see identical
 bits), by ``bench.py`` (generated directly on the GPU for the large configurations) and
-by ``__graft_entry__.smoke()``. Pure torch; no oracle and no CUDA extension involved.
+by ``__graft_entry__.smoke()``. Pure torch (NumPy for the COCO annotation sets); no oracle and no CUDA
+extension involved.
 """
 import math
 
@@ -290,3 +291,138 @@ def table_checksum(rows):
     weight = (torch.arange(n, device=rows.device, dtype=torch.int64)[:, None] * 1000003 +
               torch.arange(w, device=rows.device, dtype=torch.int64)[None, :] * 7919 + 1)
     return int((bits * weight).sum().item())
+
+
+def coco_keypoint_set(images=200, seed=0, variant="all", max_gt=4, fp=(0, 3), crowded_frac=0.05, zero_kp_frac=0.3):
+    """A seeded COCO-shaped keypoint set for the COCO evaluator: (annotation dict, results list).
+
+    Per image 0-``max_gt`` person GTs (normal ones with some unlabeled joints, ``zero_kp_frac`` with no keypoints,
+    a few crowds; areas include exactly 32^2 and 96^2) and a non-person annotation now and then; per GT 0-3
+    detections at graded distances (the ones of zero-keypoint GTs land around the box: the box-distance branch of
+    computeOks), ``fp`` false positives per image, ``crowded_frac`` of the images with 25 more (over maxDets = 20);
+    images with GT only and with detections only; scores with ties inside and across images, many exactly 0.0;
+    detections whose keypoint extent is exactly 32 x 32 or 96 x 96. ``variant`` "medium" / "large" keeps every GT
+    area inside [32^2, 96^2] / above 96^2, so that the other range has no GT. Image ids are not in sorted order in
+    the ``images`` list; the results list is shuffled across images. Keypoints of results are float32 values."""
+    import numpy as np
+    rng = np.random.default_rng(seed)
+    img_ids = (rng.permutation(3 * images)[:images] + 1).tolist()
+    dataset = {"images": [{"id": i, "width": 640, "height": 480} for i in img_ids], "annotations": [],
+               "categories": [{"id": 1, "name": "person"}]}
+    results = []
+    ann_id = 7
+
+    def det(kps_xy, score, img):
+        k = np.asarray(kps_xy, dtype=np.float32).reshape(17, 2)
+        conf = rng.random(17).astype(np.float32)
+        row = np.stack([k[:, 0], k[:, 1], conf], 1).reshape(-1)
+        results.append({"image_id": img, "category_id": 1, "keypoints": [float(v) for v in row], "score": score})
+
+    def score():
+        u = rng.random()
+        if u < 0.15:
+            return 0.0
+        if u < 0.55:
+            return float(rng.integers(0, 21)) / 20.0
+        return float(rng.random())
+
+    for img in img_ids:
+        kind = rng.random()
+        n_gt = 0 if kind < 0.1 else int(rng.integers(1, max_gt + 1))
+        gt_only = 0.1 <= kind < 0.18
+        for _ in range(n_gt):
+            u = rng.random()
+            if variant == "medium":
+                area = 1024.0 if u < 0.15 else float(rng.uniform(1100, 9100))
+            elif variant == "large":
+                area = float(rng.uniform(9300, 60000))
+            else:
+                area = 1024.0 if u < 0.05 else (9216.0 if u < 0.1 else float(rng.uniform(200, 60000)))
+            ratio = rng.uniform(0.4, 1.0)
+            bw, bh = math.sqrt(area * ratio), math.sqrt(area / ratio)
+            bx, by = float(rng.uniform(0, 640 - bw)), float(rng.uniform(0, 480 - bh))
+            t = rng.random()
+            crowd = t < 0.05
+            zero = (not crowd) and t < 0.05 + zero_kp_frac
+            v = np.zeros(17, np.int64) if zero else rng.choice([0, 1, 2], 17, p=[0.3, 0.2, 0.5])
+            if not zero and not v.any():
+                v[0] = 2
+            x = np.round(bx + rng.random(17) * bw)
+            y = np.round(by + rng.random(17) * bh)
+            x[v == 0] = 0
+            y[v == 0] = 0
+            kps = np.stack([x, y, v], 1).reshape(-1)
+            dataset["annotations"].append({
+                "id": ann_id, "image_id": img, "category_id": 1, "iscrowd": int(crowd), "area": area,
+                "bbox": [bx, by, bw, bh], "num_keypoints": int((v > 0).sum()), "keypoints": [int(q) if q == int(q) else float(q) for q in kps]})
+            ann_id += int(rng.integers(1, 4))
+            if rng.random() < 0.1:
+                dataset["annotations"].append({"id": ann_id, "image_id": img, "category_id": 3, "iscrowd": 0, "area": 50.0,
+                                               "bbox": [0, 0, 5, 10], "num_keypoints": 0, "keypoints": [0] * 51})
+                ann_id += 1
+            if gt_only:
+                continue
+            base = np.stack([bx + rng.random(17) * bw, by + rng.random(17) * bh], 1)
+            labelled = v > 0
+            base[labelled, 0], base[labelled, 1] = x[labelled], y[labelled]
+            for _d in range(int(rng.integers(0, 4))):
+                if zero:            # around the box, partly outside it: the grown-box distance
+                    xy = np.stack([rng.uniform(bx - 1.2 * bw, bx + 2.2 * bw, 17), rng.uniform(by - 1.2 * bh, by + 2.2 * bh, 17)], 1)
+                else:
+                    sigma = float(rng.choice([0.0, 0.01, 0.03, 0.06, 0.1, 0.2, 0.5])) * math.sqrt(area)
+                    xy = base + rng.normal(0.0, 1.0, (17, 2)) * sigma
+                det(xy, score(), img)
+        if gt_only:
+            continue
+        n_fp = int(rng.integers(fp[0], fp[1] + 1)) + (25 if rng.random() < crowded_frac else 0)
+        for _ in range(n_fp):
+            u = rng.random()
+            if u < 0.05:                # keypoint extent exactly 32 x 32 or 96 x 96
+                side = 32.0 if rng.random() < 0.5 else 96.0
+                x0, y0 = float(rng.integers(0, 500)), float(rng.integers(0, 350))
+                xy = np.stack([x0 + rng.integers(0, int(side) + 1, 17), y0 + rng.integers(0, int(side) + 1, 17)], 1).astype(np.float64)
+                xy[0] = (x0, y0)
+                xy[1] = (x0 + side, y0 + side)
+            else:
+                cx, cy, s = rng.uniform(0, 640), rng.uniform(0, 480), rng.uniform(5, 200)
+                xy = np.stack([cx + rng.normal(0, 1, 17) * s, cy + rng.normal(0, 1, 17) * s], 1)
+            det(xy, score(), img)
+    order = rng.permutation(len(results))
+    return dataset, [results[i] for i in order]
+
+
+def coco_results_arrays(results):
+    """Results list -> (keypoints float32 [N, 51], scores float64 [N], image ids int64 [N]) as CPU tensors."""
+    import numpy as np
+    kps = np.array([r["keypoints"] for r in results], dtype=np.float32).reshape(-1, 51)
+    scores = np.array([r["score"] for r in results], dtype=np.float64)
+    ids = np.array([r["image_id"] for r in results], dtype=np.int64)
+    return torch.from_numpy(kps), torch.from_numpy(scores), torch.from_numpy(ids)
+
+
+def eval_set_ground_truth(es, keypoints, seed=0, jitter=2.0, zero_kp_frac=0.4):
+    """COCO-shaped GT for an ``EvalSet``, so that the whole eval job can end in AP: image i has id i + 1; every
+    original person of it (not a near-duplicate) becomes a GT whose keypoints are its decoded image-space
+    keypoints (``keypoints`` [N, K, >=2], host) moved by N(0, jitter^2) px, its box the detection box;
+    ``zero_kp_frac`` of them carry no keypoints. Returns (annotation dict, image ids [I])."""
+    import numpy as np
+    rng = np.random.default_rng(seed)
+    kp = np.asarray(keypoints, dtype=np.float64)
+    boxes = es.boxes.numpy()
+    leader = es.leader.numpy()
+    ids = np.arange(1, es.images + 1, dtype=np.int64)
+    anns = []
+    for i in range(es.images):
+        for p in range(int(es.seg[i]), int(es.seg[i + 1])):
+            if leader[p] != p:
+                continue
+            x1, y1, x2, y2 = (float(v) for v in boxes[p])
+            w, h = max(x2 - x1, 1.0), max(y2 - y1, 1.0)
+            zero = rng.random() < zero_kp_frac
+            xy = kp[p, :, :2] + rng.normal(0.0, jitter, (kp.shape[1], 2))
+            v = np.zeros(kp.shape[1]) if zero else np.full(kp.shape[1], 2.0)
+            k = np.stack([np.where(v > 0, xy[:, 0], 0), np.where(v > 0, xy[:, 1], 0), v], 1).reshape(-1)
+            anns.append({"id": len(anns) + 1, "image_id": int(ids[i]), "category_id": 1, "iscrowd": 0,
+                         "area": w * h * 0.7, "bbox": [x1, y1, w, h], "num_keypoints": int((v > 0).sum()),
+                         "keypoints": k.tolist()})
+    return {"images": [{"id": int(i)} for i in ids], "annotations": anns}, ids
