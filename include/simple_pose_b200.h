@@ -158,6 +158,33 @@ int sp_step_f32(const float* joints, const float* pred, const float* trans_inv, 
                 float* pred_xy, float* label_xy, void* workspace, size_t workspace_bytes,
                 int B, int K, int H, int W, double sigma, int ksize, float grad_scale, void* stream);
 
+/* One validation batch in ONE launch: the body of every solver's val() -- processors/dp_pose_hrnet_solver.py:156-161,
+ * dp_pose_resnet_solver.py and ddp_pose_resnet_solver.py alike:
+ *   loss = 0.5 * MSELoss(predicts * mask, targets * mask)       (:156; forward only, val() runs under no_grad)
+ *   acc = HeatMapAcc()(predicts * mask, targets * mask)          (:157)
+ *   pred_kps, scores = decoder(predicts, tran_inv)               (:160; GaussTaylor or Basic KeyPointDecoder)
+ *   kps_to_dict_(pred_kps, scores, img_ids, kps_dict_list)       (:161; as the sp_person_rows_f32 table)
+ * i.e. sp_encode_mse_fwd_bwd_f32 (no grad, argmaxes) + sp_decode_ws_f32(mode) + sp_heatmap_acc_f32 + sp_person_rows_f32.
+ *   joints [B,K,3] f32 heatmap px; pred [B,K,H,W] f32; trans_inv [B,2,3] f32 (NULL = heatmap-space coords);
+ *   mode SP_DECODE_GAUSS_TAYLOR (blur_w [121] f32, ksize must be 11) or SP_DECODE_BASIC (blur_w and ksize unused);
+ *   any other mode: SP_ERR_BAD_ARGUMENT.
+ *   outputs: weights [B,K] (NULL ok), loss (1 f32), acc (1 f32), rows [B, 3K+1] f32 = (x, y, conf) * K then the person
+ *   score mean(conf) + max(conf); coords [B,K,2] / maxval [B,K] (both NULL = rows only); pred_xy / label_xy [B,K,2]
+ *   (the HeatMapAcc argmaxes; both NULL = kept in the workspace).
+ *   distance_thresh, norm_frac: HeatMapAcc's constructor arguments (0.5, 10).
+ * workspace: sp_val_step_workspace_bytes(B, K) bytes, 16-byte aligned, ZERO-FILLED ONCE by the caller. It holds the
+ * reduction workspace, the per-person completion counters and room for the argmax axes; every launch returns the
+ * counters to zero, so it can be reused (and a captured graph replayed) on the same stream.
+ * rows, weights, coords, maxval, pred_xy, label_xy and acc are bit-identical to the composed entry points, the loss up to
+ * the float64 summation order. W % 4 != 0, GaussTaylor with ksize != 11 or maps too large for shared memory:
+ * SP_ERR_UNSUPPORTED (compose the stand-alone calls). */
+size_t sp_val_step_workspace_bytes(int B, int K);
+int sp_val_step_f32(const float* joints, const float* pred, const float* trans_inv, const float* blur_w, int mode,
+                    float* weights, float* loss, float* acc, float* rows, float* coords, float* maxval,
+                    float* pred_xy, float* label_xy, void* workspace, size_t workspace_bytes,
+                    int B, int K, int H, int W, double sigma, int ksize, float distance_thresh, float norm_frac,
+                    void* stream);
+
 /* HeatMapAcc.__call__ epilogue, metrics/pose_metrics.py:225-245: per-joint fraction of persons whose
  * predicted argmax lies within distance_thresh (in units of (W,H)/norm_frac) of the target argmax, over
  * persons whose target argmax has x > 1 and y > 1, averaged over joints that have any. pred_xy, label_xy

@@ -42,6 +42,9 @@ SIGNATURES = {
     "sp_encode_mse_fwd_bwd_f32": (c_int, [c_void] * 9 + [c_size, c_int, c_int, c_int, c_int, c_dbl, c_flt, c_void]),
     "sp_encode_mse_fwd_bwd": (c_int, [c_void, c_void, c_int] + [c_void] * 7 + [c_size, c_int, c_int, c_int, c_int, c_dbl, c_flt, c_void, c_void]),
     "sp_step_f32": (c_int, [c_void] * 13 + [c_size, c_int, c_int, c_int, c_int, c_dbl, c_int, c_flt, c_void]),
+    "sp_val_step_workspace_bytes": (c_size, [c_int, c_int]),
+    "sp_val_step_f32": (c_int, [c_void] * 4 + [c_int] + [c_void] * 9 + [c_size, c_int, c_int, c_int, c_int, c_dbl, c_int,
+                                                                   c_flt, c_flt, c_void]),
     "sp_heatmap_acc_f32": (c_int, [c_void, c_void, c_void, c_int, c_int, c_int, c_int, c_flt, c_flt, c_void]),
     "sp_scale_inplace_f32": (c_int, [c_void, c_ll, c_void, c_void]),
     "sp_decode_f32": (c_int, [c_void, c_void, c_void, c_void, c_void, c_void, c_void, c_void,
@@ -208,13 +211,15 @@ def drop_scratch(device, stream_id=None):
 
 def check_ws(code, device, stream_id, owner=None):
     """``check`` for calls that were handed a workspace: on failure the cached per-stream scratch is dropped and an
-    ``owner`` that keeps its own (``HeatmapHotPath.ws`` / ``.dws``) gets it re-zeroed."""
+    ``owner`` that keeps its own (``HeatmapHotPath.ws`` / ``.dws`` / ``.vws``) gets it re-zeroed."""
     if code != 0:
         drop_scratch(device, stream_id)
         if owner is not None:
             try:
                 owner.ws.zero_()
                 owner.dws.zero_()
+                if getattr(owner, "vws", None) is not None:
+                    owner.vws.zero_()
             except Exception:
                 pass
     check(code)

@@ -2,6 +2,7 @@
 // the PTX wrappers for mbarrier + cp.async.bulk (the 1-D TMA bulk copy, SASS: UBLKCP).
 #pragma once
 #include <cuda_runtime.h>
+#include <math_constants.h>
 #include <stdint.h>
 #include <stdlib.h>
 #include "../../include/simple_pose_b200.h"
@@ -179,5 +180,37 @@ __device__ __forceinline__ bool better(float v, int i, float bv, int bi) {
     if (vn) return i < bi;
     return (v > bv) || (v == bv && i < bi);
 }
+
+// ---- global counter with release (this thread's earlier writes) and acquire (later reads) semantics, device scope
+__device__ __forceinline__ unsigned int atomic_add_acq_rel(unsigned int* p, unsigned int v) {
+    unsigned int old;
+    asm volatile("atom.acq_rel.gpu.global.add.u32 %0, [%1], %2;" : "=r"(old) : "l"(p), "r"(v) : "memory");
+    return old;
+}
+
+// Person score of kps_to_dict_ (metrics/pose_metrics.py:176): mean(conf) + max(conf) over the K joint peaks, fed in
+// joint order. The mean is accumulated in float64 and rounded once (torch's float32 reduction order differs between
+// its CPU and CUDA kernels; this is within 1 ulp of either); a NaN peak makes the score NaN.
+struct PersonScore {
+    double sum;
+    float mx;
+    bool nan;
+    static __device__ __forceinline__ PersonScore start() {
+        PersonScore s;
+        s.sum = 0.0;
+        s.mx = -CUDART_INF_F;
+        s.nan = false;
+        return s;
+    }
+    __device__ __forceinline__ void add(float v) {
+        sum += (double)v;
+        nan |= (v != v);
+        mx = fmaxf(mx, v);
+    }
+    __device__ __forceinline__ float value(int K) const {
+        const float mean = (float)(sum / (double)K);
+        return nan ? CUDART_NAN_F : __fadd_rn(mean, mx);
+    }
+};
 
 }  // namespace sp

@@ -388,28 +388,22 @@ pack_rows_kernel(const float* __restrict__ coords, const float* __restrict__ max
 }
 
 // kps_to_dict_ (metrics/pose_metrics.py:172-179) as one table: rows [N, 3K+1] f32 = (x, y, conf) * K, then the
-// person score mean(conf) + max(conf). The mean is accumulated in float64 and rounded once (torch's float32
-// reduction order differs between its CPU and CUDA kernels; this is within 1 ulp of either).
+// person score mean(conf) + max(conf) (sp::PersonScore, shared with the validation step kernel).
 __global__ void __launch_bounds__(128)
 person_rows_kernel(const float* __restrict__ coords, const float* __restrict__ maxval, float* __restrict__ rows, int N, int K) {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= N) return;
     float* r = rows + (size_t)p * (3 * K + 1);
-    double sum = 0.0;
-    float mx = -CUDART_INF_F;
-    bool nan = false;
+    sp::PersonScore score = sp::PersonScore::start();
     for (int k = 0; k < K; ++k) {
         const float2 c = reinterpret_cast<const float2*>(coords)[(size_t)p * K + k];
         const float v = maxval[(size_t)p * K + k];
         r[3 * k + 0] = c.x;
         r[3 * k + 1] = c.y;
         r[3 * k + 2] = v;
-        sum += (double)v;
-        nan |= (v != v);
-        mx = fmaxf(mx, v);
+        score.add(v);
     }
-    const float mean = (float)(sum / (double)K);
-    r[3 * K] = nan ? CUDART_NAN_F : __fadd_rn(mean, mx);
+    r[3 * K] = score.value(K);
 }
 
 }  // namespace

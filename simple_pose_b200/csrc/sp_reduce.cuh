@@ -16,9 +16,10 @@ struct MseWorkspace {
 };
 
 // Called by ALL threads of every block (gridDim.x <= kMaxPartials, blockDim.x <= THREADS, a multiple
-// of 32). loss = 0.5 * total * inv_count.
+// of 32). loss = 0.5 * total * inv_count. Returns true in every thread of the last block, which has acquired the
+// writes every block made before its call.
 template <int THREADS>
-__device__ __forceinline__ void finish_loss(double block_sum, MseWorkspace* __restrict__ ws, float* __restrict__ loss,
+__device__ __forceinline__ bool finish_loss(double block_sum, MseWorkspace* __restrict__ ws, float* __restrict__ loss,
                                             double inv_count) {
     __shared__ double warp_part[THREADS / 32];
     __shared__ bool am_last;
@@ -34,7 +35,7 @@ __device__ __forceinline__ void finish_loss(double block_sum, MseWorkspace* __re
         am_last = (t == gridDim.x - 1);
     }
     __syncthreads();
-    if (!am_last) return;
+    if (!am_last) return false;
     // last block: add the partials in index order (thread-strided, then a fixed tree)
     __threadfence();
     double s = 0.0;
@@ -50,6 +51,7 @@ __device__ __forceinline__ void finish_loss(double block_sum, MseWorkspace* __re
         ws->ticket = 0u;      // restore the zero state for the next call on this stream
         ws->next_work = 0u;
     }
+    return true;
 }
 
 }  // namespace sp_reduce

@@ -36,10 +36,27 @@ constexpr int kPatchBytes = 1536;    // zero-padded 15 x 15 patch for peaks near
 // k < static_maps, the rest come one at a time from the counter in the caller's workspace (claimed one map ahead, so
 // the atomic's round trip is never waited for). The SMs do not drain HBM at equal rates once the memory system
 // queues (profiles/r1f_fused_timeline.md), and with equal ranges the slowest SM is the critical path.
-template <bool WRITE_GRAD, bool WRITE_TARGETS, bool ACC>
-__global__ void __launch_bounds__(512, 1)
-step_kernel(const sp_dec::DecodeArgs A, const sp_trn::MapIo io, float* __restrict__ loss, MseWorkspace* __restrict__ ws,
-            double inv_count, int nwarps, int static_maps) {
+//
+// The validation form (VAL, val_step_kernel) is the body of val() for both decoder families: no gradient, no target
+// map, HeatMapAcc argmaxes always, the decoder MODE fixed at compile time (GaussTaylor or Basic; Basic reads no blur
+// weights and needs no patch, but keeps the same shared-memory layout and so the same work distribution), and two
+// results that need more than one map:
+//   - the kps_to_dict_ row of a person: after a map's (x, y, conf) is in its row, lane 0 counts the map in the
+//     person's arrival counter (release/acquire); the map that completes the person reads the K peaks back in joint
+//     order, writes the score column and returns the counter to zero;
+//   - the HeatMapAcc value: the last CTA of the loss reduction has acquired every CTA's argmax axes and runs the
+//     stand-alone epilogue on them.
+struct ValOut {
+    unsigned int* arrivals;    // [B] per-person map counters in the caller's workspace, zero between launches
+    float* acc;
+    float norm_x, norm_y, thresh;
+    int B;
+};
+
+template <bool WRITE_GRAD, bool WRITE_TARGETS, bool ACC, int MODE, bool VAL>
+__device__ __forceinline__ void step_body(const sp_dec::DecodeArgs& A, const sp_trn::MapIo& io, float* __restrict__ loss,
+                                          MseWorkspace* __restrict__ ws, double inv_count, int nwarps, int static_maps,
+                                          const ValOut& V) {
     extern __shared__ __align__(128) unsigned char smem[];
     constexpr int KS = 11;
     const int lane = threadIdx.x & 31;
@@ -95,10 +112,11 @@ step_kernel(const sp_dec::DecodeArgs A, const sp_trn::MapIo io, float* __restric
     int m = grid_wide ? (int)blockIdx.x * nwarps + warp : range_lo + warp;
     if (m >= (grid_wide ? A.nmaps : range_hi)) m = -1;
     if (lane == 0 && m >= 0) issue(m);
-    for (int t = threadIdx.x; t < KS * KS; t += blockDim.x) wts[t] = __ldg(A.blur_w + t);
+    if (MODE == SP_DECODE_GAUSS_TAYLOR)
+        for (int t = threadIdx.x; t < KS * KS; t += blockDim.x) wts[t] = __ldg(A.blur_w + t);
     __syncthreads();
     sp_dec::LaneTaps<KS> taps;
-    taps.load(wts, lane);
+    if (MODE == SP_DECODE_GAUSS_TAYLOR) taps.load(wts, lane);
 
     double sum_sq = 0.0;
     uint32_t parity = 0;
@@ -125,13 +143,44 @@ step_kernel(const sp_dec::DecodeArgs A, const sp_trn::MapIo io, float* __restric
                                                                         ex, ey, st, lane, io.half_scale);
                 if (ACC) sp_trn::end_map_acc(io, m, jv, ex, ey, st, lane);
                 sum_sq += (double)st.acc;
-            } else if (A.coords != nullptr) {
+            } else if (VAL || A.coords != nullptr) {
                 // ---- decode (argmax on the raw map, blur at the 13 stencil points, Taylor step, affine)
                 const sp_dec::Peak pk = sp_dec::argmax_smem<false>(a, a, hw, A.W, lane);
                 sp_dec::DirectView view{a};
-                sp_dec::finish_map(A, view, m, pk, lane, T, [&](int px, int py, float ori_max, float& ox, float& oy) {
+                auto gauss_taylor = [&](int px, int py, float ori_max, float& ox, float& oy) {
                     return sp_dec::taylor_refine_smem<KS>(a, wts, patch, taps, A.H, A.W, px, py, ori_max, lane, ox, oy);
-                });
+                };
+                if constexpr (VAL) {
+                    sp_dec::DecodeArgs D = A;
+                    D.mode = MODE;                 // the branch of finish_map is chosen at compile time
+                    if constexpr (MODE == SP_DECODE_BASIC) {
+                        sp_dec::finish_map(D, view, m, pk, lane, T, [](int, int, float, float&, float&) { return false; });
+                    } else {
+                        sp_dec::finish_map(D, view, m, pk, lane, T, gauss_taylor);
+                    }
+                    // lane 0 stored this map's (x, y, conf) in the row; the warp that completes the person reads the K
+                    // peaks in parallel (lane 0's acquire reaches the other lanes through __syncwarp), then every lane
+                    // adds them up in joint order
+                    const int person = m / A.K;
+                    unsigned arrived = 0u;
+                    if (lane == 0) arrived = sp::atomic_add_acq_rel(V.arrivals + person, 1u);
+                    if (__shfl_sync(SP_FULL, arrived, 0) == (unsigned)A.K - 1u) {
+                        __syncwarp();
+                        float* r = A.rows + (size_t)person * A.row_stride;
+                        sp::PersonScore score = sp::PersonScore::start();
+                        for (int k0 = 0; k0 < A.K; k0 += 32) {
+                            const float mine = (k0 + lane < A.K) ? __ldcg(r + 3 * (k0 + lane) + 2) : 0.f;
+                            const int n = min(32, A.K - k0);
+                            for (int j = 0; j < n; ++j) score.add(__shfl_sync(SP_FULL, mine, j));
+                        }
+                        if (lane == 0) {
+                            r[3 * A.K] = score.value(A.K);
+                            V.arrivals[person] = 0u;
+                        }
+                    }
+                } else {
+                    sp_dec::finish_map(A, view, m, pk, lane, T, gauss_taylor);
+                }
             }
         }
         __syncwarp();               // every lane is done with the staged map and the factors
@@ -141,25 +190,37 @@ step_kernel(const sp_dec::DecodeArgs A, const sp_trn::MapIo io, float* __restric
         }
         m = __shfl_sync(SP_FULL, ahead, 0);
     }
-    sp_reduce::finish_loss<512>(sum_sq, ws, loss, inv_count);      // the last block also returns ws->next_work to zero
+    // the last block also returns ws->next_work to zero
+    const bool last = sp_reduce::finish_loss<512>(sum_sq, ws, loss, inv_count);
+    if constexpr (VAL) {
+        // every staged map is consumed: the counters go where the per-warp areas were
+        if (last) sp_trn::heatmap_acc_block<true>(io.pred_xy, io.label_xy, V.acc, V.B, A.K, V.norm_x, V.norm_y, V.thresh,
+                                                  reinterpret_cast<int*>(smem + kHeadBytes + kWtsBytes));
+    }
 }
 
-}  // namespace
+template <bool WRITE_GRAD, bool WRITE_TARGETS, bool ACC>
+__global__ void __launch_bounds__(512, 1)
+step_kernel(const sp_dec::DecodeArgs A, const sp_trn::MapIo io, float* __restrict__ loss, MseWorkspace* __restrict__ ws,
+            double inv_count, int nwarps, int static_maps) {
+    step_body<WRITE_GRAD, WRITE_TARGETS, ACC, SP_DECODE_GAUSS_TAYLOR, false>(A, io, loss, ws, inv_count, nwarps, static_maps,
+                                                                              ValOut{});
+}
 
-extern "C" int sp_step_f32(const float* joints, const float* pred, const float* trans_inv, const float* blur_w,
-                           float* targets, float* weights, float* grad, float* loss, float* coords, float* maxval,
-                           float* pred_xy, float* label_xy, void* workspace, size_t workspace_bytes,
-                           int B, int K, int H, int W, double sigma, int ksize, float grad_scale, void* stream) {
-    SP_RETURN_IF(!joints || !pred || !blur_w || !loss || !workspace, SP_ERR_BAD_ARGUMENT);
-    SP_RETURN_IF((coords == nullptr) != (maxval == nullptr), SP_ERR_BAD_ARGUMENT);      // both NULL: no decode pass
-    SP_RETURN_IF(B <= 0 || K <= 0 || H <= 0 || W <= 0 || !(sigma > 0.0), SP_ERR_BAD_ARGUMENT);
-    SP_RETURN_IF((pred_xy == nullptr) != (label_xy == nullptr), SP_ERR_BAD_ARGUMENT);
-    SP_RETURN_IF((long long)B * K > 0x7fffffffLL || (long long)H * W > (1 << 24), SP_ERR_UNSUPPORTED);
-    SP_RETURN_IF(W % 4 != 0 || ksize != 11, SP_ERR_UNSUPPORTED);      // callers compose the stand-alone kernels instead
-    SP_RETURN_IF(workspace_bytes < sizeof(MseWorkspace), SP_ERR_WORKSPACE);
-    SP_RETURN_IF(!sp_aligned16(workspace) || !sp_aligned16(pred) || (grad && !sp_aligned16(grad)) || (targets && !sp_aligned16(targets)) ||
-                 (coords && !sp_aligned16(coords)) || (pred_xy && (!sp_aligned16(pred_xy) || !sp_aligned16(label_xy))), SP_ERR_BAD_ALIGNMENT);
-    const int nmaps = B * K;
+template <int MODE>
+__global__ void __launch_bounds__(512, 1)
+val_step_kernel(const sp_dec::DecodeArgs A, const sp_trn::MapIo io, float* __restrict__ loss, MseWorkspace* __restrict__ ws,
+                double inv_count, int nwarps, int static_maps, const ValOut V) {
+    step_body<false, false, true, MODE, true>(A, io, loss, ws, inv_count, nwarps, static_maps, V);
+}
+
+// Launch shape of step_kernel / val_step_kernel for B*K = nmaps maps of H x W. SP_ERR_UNSUPPORTED when not even one
+// map fits in shared memory.
+struct StepLayout {
+    int nwarps, grid, static_maps;
+    size_t smem;
+};
+int plan_step(int nmaps, int H, int W, StepLayout& L) {
     const size_t map_bytes = (size_t)H * W * 4;
     const int wpad = (W + 1) & ~1;
     const size_t fac_bytes = (size_t)(wpad + ((H + 1) & ~1)) * sizeof(double);
@@ -185,7 +246,6 @@ extern "C" int sp_step_f32(const float* joints, const float* pred, const float* 
     int grid = sms;
     const int need = (nmaps + nwarps - 1) / nwarps;
     if (grid > need) grid = need;
-    const size_t smem = kHeadBytes + kWtsBytes + (size_t)nwarps * per_warp1;
     // large launches: maps dealt grid-wide; SP_STEP_STATIC_PCT % of a warp's expected share is fixed up front (no atomic),
     // the rest is claimed dynamically. Tried and dropped for this kernel (numbers in DESIGN.md section 4): a second stage per
     // warp (123.5 vs 114.0 us at 1024 x 64x48) and the period-tiled loss pass of the fused training kernel (123 vs 113 us).
@@ -199,23 +259,65 @@ extern "C" int sp_step_f32(const float* joints, const float* pred, const float* 
         static_maps = (int)(share - dynamic);
         if (static_maps < 1) static_maps = 1;
     }
+    L.nwarps = nwarps;
+    L.grid = grid;
+    L.static_maps = static_maps;
+    L.smem = kHeadBytes + kWtsBytes + (size_t)nwarps * per_warp1;
+    return 0;
+}
 
+sp_dec::DecodeArgs step_decode_args(const float* pred, const float* trans_inv, const float* blur_w, float* coords,
+                                    float* maxval, float* rows, int B, int K, int H, int W, int mode) {
     sp_dec::DecodeArgs A;
     A.hm = pred; A.hm_flip = nullptr; A.perm = nullptr; A.trans_inv = trans_inv; A.blur_w = blur_w;
-    A.coords = coords; A.maxval = maxval; A.argmax = nullptr; A.rows = nullptr; A.row_stride = 0;
-    A.nmaps = nmaps; A.K = K; A.H = H; A.W = W; A.ksize = 11; A.mode = SP_DECODE_GAUSS_TAYLOR; A.work = nullptr;
+    A.coords = coords; A.maxval = maxval; A.argmax = nullptr; A.rows = rows; A.row_stride = rows ? 3 * K + 1 : 0;
+    A.nmaps = B * K; A.K = K; A.H = H; A.W = W; A.ksize = 11; A.mode = mode; A.work = nullptr;
+    return A;
+}
+
+sp_trn::MapIo step_io(const float* joints, const float* pred, float* grad, float* targets, float* weights, float* pred_xy,
+                      float* label_xy, int B, int K, int H, int W, double sigma, float grad_scale) {
     const double count = (double)B * (double)K * (double)H * (double)W;
     sp_trn::MapIo io;
     io.joints = joints; io.pred = pred; io.grad = grad; io.targets = targets; io.weights = weights;
     io.pred_xy = reinterpret_cast<float2*>(pred_xy); io.label_xy = reinterpret_cast<float2*>(label_xy);
-    io.nmaps = nmaps; io.H = H; io.W = W; io.reach = (float)(sigma * 3.0); io.denom = 2.0 * (sigma * sigma);
+    io.nmaps = B * K; io.H = H; io.W = W; io.reach = (float)(sigma * 3.0); io.denom = 2.0 * (sigma * sigma);
     io.norm = (float)(2.0 / count); io.half_scale = 0.5f * grad_scale; io.scale_dev = nullptr;
     io.analytic_ok = (sigma >= 0.25 && sigma <= 64.0) ? 1 : 0;
+    return io;
+}
+
+// validation workspace: the reduction workspace, then the per-person arrival counters, then room for the argmax axes
+size_t val_arrivals_offset() { return (sizeof(MseWorkspace) + 15) & ~(size_t)15; }
+size_t val_axes_offset(int B) { return val_arrivals_offset() + (((size_t)B * 4 + 15) & ~(size_t)15); }
+
+}  // namespace
+
+extern "C" int sp_step_f32(const float* joints, const float* pred, const float* trans_inv, const float* blur_w,
+                           float* targets, float* weights, float* grad, float* loss, float* coords, float* maxval,
+                           float* pred_xy, float* label_xy, void* workspace, size_t workspace_bytes,
+                           int B, int K, int H, int W, double sigma, int ksize, float grad_scale, void* stream) {
+    SP_RETURN_IF(!joints || !pred || !blur_w || !loss || !workspace, SP_ERR_BAD_ARGUMENT);
+    SP_RETURN_IF((coords == nullptr) != (maxval == nullptr), SP_ERR_BAD_ARGUMENT);      // both NULL: no decode pass
+    SP_RETURN_IF(B <= 0 || K <= 0 || H <= 0 || W <= 0 || !(sigma > 0.0), SP_ERR_BAD_ARGUMENT);
+    SP_RETURN_IF((pred_xy == nullptr) != (label_xy == nullptr), SP_ERR_BAD_ARGUMENT);
+    SP_RETURN_IF((long long)B * K > 0x7fffffffLL || (long long)H * W > (1 << 24), SP_ERR_UNSUPPORTED);
+    SP_RETURN_IF(W % 4 != 0 || ksize != 11, SP_ERR_UNSUPPORTED);      // callers compose the stand-alone kernels instead
+    SP_RETURN_IF(workspace_bytes < sizeof(MseWorkspace), SP_ERR_WORKSPACE);
+    SP_RETURN_IF(!sp_aligned16(workspace) || !sp_aligned16(pred) || (grad && !sp_aligned16(grad)) || (targets && !sp_aligned16(targets)) ||
+                 (coords && !sp_aligned16(coords)) || (pred_xy && (!sp_aligned16(pred_xy) || !sp_aligned16(label_xy))), SP_ERR_BAD_ALIGNMENT);
+    StepLayout L;
+    const int bad = plan_step(B * K, H, W, L);
+    if (bad != 0) return bad;
+    const sp_dec::DecodeArgs A = step_decode_args(pred, trans_inv, blur_w, coords, maxval, nullptr, B, K, H, W,
+                                                  SP_DECODE_GAUSS_TAYLOR);
+    const sp_trn::MapIo io = step_io(joints, pred, grad, targets, weights, pred_xy, label_xy, B, K, H, W, sigma, grad_scale);
+    const double count = (double)B * (double)K * (double)H * (double)W;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     MseWorkspace* ws = static_cast<MseWorkspace*>(workspace);
     const int sel = (grad ? 4 : 0) | (targets ? 2 : 0) | (pred_xy ? 1 : 0);
 #define SP_LAUNCH_STEP(G, T, AC) \
-    SP_CUDA(sp_launch_smem(step_kernel<G, T, AC>, dim3(grid), dim3(nwarps * 32), smem, st, A, io, loss, ws, 1.0 / count, nwarps, static_maps))
+    SP_CUDA(sp_launch_smem(step_kernel<G, T, AC>, dim3(L.grid), dim3(L.nwarps * 32), L.smem, st, A, io, loss, ws, 1.0 / count, L.nwarps, L.static_maps))
     switch (sel) {
         case 0: SP_LAUNCH_STEP(false, false, false); break;
         case 1: SP_LAUNCH_STEP(false, false, true); break;
@@ -227,5 +329,58 @@ extern "C" int sp_step_f32(const float* joints, const float* pred, const float* 
         default: SP_LAUNCH_STEP(true, true, true); break;
     }
 #undef SP_LAUNCH_STEP
+    return 0;
+}
+
+extern "C" size_t sp_val_step_workspace_bytes(int B, int K) {
+    if (B <= 0 || K <= 0) return val_arrivals_offset();
+    return val_axes_offset(B) + 2 * (size_t)B * K * sizeof(float2);
+}
+
+extern "C" int sp_val_step_f32(const float* joints, const float* pred, const float* trans_inv, const float* blur_w, int mode,
+                               float* weights, float* loss, float* acc, float* rows, float* coords, float* maxval,
+                               float* pred_xy, float* label_xy, void* workspace, size_t workspace_bytes,
+                               int B, int K, int H, int W, double sigma, int ksize, float distance_thresh, float norm_frac,
+                               void* stream) {
+    SP_RETURN_IF(mode != SP_DECODE_GAUSS_TAYLOR && mode != SP_DECODE_BASIC, SP_ERR_BAD_ARGUMENT);
+    SP_RETURN_IF(!joints || !pred || !loss || !acc || !rows || !workspace, SP_ERR_BAD_ARGUMENT);
+    SP_RETURN_IF(mode == SP_DECODE_GAUSS_TAYLOR && !blur_w, SP_ERR_BAD_ARGUMENT);
+    SP_RETURN_IF((coords == nullptr) != (maxval == nullptr), SP_ERR_BAD_ARGUMENT);      // both NULL: rows only
+    SP_RETURN_IF((pred_xy == nullptr) != (label_xy == nullptr), SP_ERR_BAD_ARGUMENT);  // both NULL: in the workspace
+    SP_RETURN_IF(B <= 0 || K <= 0 || H <= 0 || W <= 0 || !(sigma > 0.0) || !(norm_frac > 0.f), SP_ERR_BAD_ARGUMENT);
+    SP_RETURN_IF((long long)B * K > 0x7fffffffLL / 3 || (long long)H * W > (1 << 24), SP_ERR_UNSUPPORTED);
+    SP_RETURN_IF(W % 4 != 0 || (mode == SP_DECODE_GAUSS_TAYLOR && ksize != 11), SP_ERR_UNSUPPORTED);   // compose instead
+    SP_RETURN_IF(workspace_bytes < sp_val_step_workspace_bytes(B, K), SP_ERR_WORKSPACE);
+    SP_RETURN_IF(!sp_aligned16(workspace) || !sp_aligned16(pred) || (coords && !sp_aligned16(coords)) ||
+                 (pred_xy && (!sp_aligned16(pred_xy) || !sp_aligned16(label_xy))), SP_ERR_BAD_ALIGNMENT);
+    StepLayout L;
+    const int bad = plan_step(B * K, H, W, L);
+    if (bad != 0) return bad;
+    // the HeatMapAcc counters reuse the per-warp areas of the last CTA
+    SP_RETURN_IF((size_t)2 * K * sizeof(int) > L.smem - kHeadBytes - kWtsBytes, SP_ERR_UNSUPPORTED);
+    unsigned char* wsb = static_cast<unsigned char*>(workspace);
+    if (!pred_xy) {
+        pred_xy = reinterpret_cast<float*>(wsb + val_axes_offset(B));
+        label_xy = pred_xy + 2 * (size_t)B * K;
+    }
+    const sp_dec::DecodeArgs A = step_decode_args(pred, trans_inv, blur_w, coords, maxval, rows, B, K, H, W, mode);
+    const sp_trn::MapIo io = step_io(joints, pred, nullptr, nullptr, weights, pred_xy, label_xy, B, K, H, W, sigma, 1.f);
+    const double count = (double)B * (double)K * (double)H * (double)W;
+    ValOut V;
+    V.arrivals = reinterpret_cast<unsigned int*>(wsb + val_arrivals_offset());
+    V.acc = acc;
+    V.norm_x = (float)W / norm_frac;           // norm = tensor([W, H], float32) / norm_frac, as sp_heatmap_acc_f32
+    V.norm_y = (float)H / norm_frac;
+    V.thresh = distance_thresh;
+    V.B = B;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    MseWorkspace* ws = static_cast<MseWorkspace*>(workspace);
+    if (mode == SP_DECODE_BASIC) {
+        SP_CUDA(sp_launch_smem(val_step_kernel<SP_DECODE_BASIC>, dim3(L.grid), dim3(L.nwarps * 32), L.smem, st, A, io, loss, ws,
+                               1.0 / count, L.nwarps, L.static_maps, V));
+    } else {
+        SP_CUDA(sp_launch_smem(val_step_kernel<SP_DECODE_GAUSS_TAYLOR>, dim3(L.grid), dim3(L.nwarps * 32), L.smem, st, A, io,
+                               loss, ws, 1.0 / count, L.nwarps, L.static_maps, V));
+    }
     return 0;
 }

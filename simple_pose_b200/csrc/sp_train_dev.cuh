@@ -599,5 +599,44 @@ __device__ __forceinline__ float tile_map(const MapIo& io, int m, const JointVer
     return acc;
 }
 
+// HeatMapAcc epilogue (metrics/pose_metrics.py:227-245) on the [B,K] argmax coordinates, run by ALL threads of one
+// block; counters = 2K ints of shared memory. The per-joint counts do not depend on the order the threads add them in
+// and one thread sums the joints in order, so every block size gives the same bits. COHERENT: read the axes through L2
+// (ld.global.cg) because other CTAs of the same launch wrote them (the caller has acquired their writes).
+template <bool COHERENT>
+__device__ __forceinline__ void heatmap_acc_block(const float2* __restrict__ pred_xy, const float2* __restrict__ label_xy,
+                                                  float* __restrict__ acc, int B, int K, float norm_x, float norm_y,
+                                                  float thresh, int* counters) {
+    int* hit = counters;
+    int* valid = counters + K;
+    for (int k = threadIdx.x; k < 2 * K; k += blockDim.x) counters[k] = 0;
+    __syncthreads();
+    const int n = B * K;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        const float2 l = COHERENT ? __ldcg(label_xy + i) : label_xy[i];
+        if (l.x > 1.f && l.y > 1.f) {
+            const float2 p = COHERENT ? __ldcg(pred_xy + i) : pred_xy[i];
+            const float dx = __fsub_rn(__fdiv_rn(p.x, norm_x), __fdiv_rn(l.x, norm_x));
+            const float dy = __fsub_rn(__fdiv_rn(p.y, norm_y), __fdiv_rn(l.y, norm_y));
+            // torch.norm accumulates float inputs in double on CPU (the pinned oracle); no (dx, dy)
+            // pair of the supported map sizes lands on the threshold, so float vs double is moot
+            const float dist = (float)sqrt((double)dx * (double)dx + (double)dy * (double)dy);
+            const int k = i % K;
+            atomicAdd(&valid[k], 1);
+            if (dist < thresh) atomicAdd(&hit[k], 1);
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float sum = 0.f;
+        int used = 0;
+        for (int k = 0; k < K; ++k) {
+            if (valid[k] < 1) continue;
+            sum = __fadd_rn(sum, __fdiv_rn((float)hit[k], (float)valid[k]));
+            ++used;
+        }
+        acc[0] = used > 0 ? __fdiv_rn(sum, (float)used) : 0.f;
+    }
+}
 
 }  // namespace sp_trn

@@ -208,6 +208,11 @@ def kps_to_dict_(predicts, scores, img_ids, set_in_list):
     """Reference :172-179 with ONE kernel and ONE device->host copy instead of a ``mean``/``max``/``cat``
     chain plus one ``.item()`` and one ``.tolist()`` (two device syncs) per person:
     score = mean + max of the joint peaks, keypoints = [x, y, score] * K."""
-    rows = person_rows(predicts, scores).cpu().tolist()
-    for row, img_id in zip(rows, img_ids):
+    rows_to_dicts(person_rows(predicts, scores), img_ids, set_in_list)
+
+
+def rows_to_dicts(rows, img_ids, set_in_list):
+    """``kps_to_dict_``'s dicts from its [N, 3K+1] rows (``person_rows`` or ``HeatmapHotPath.val_step``), one
+    device->host copy for the whole table."""
+    for row, img_id in zip(rows.cpu().tolist(), img_ids):
         set_in_list.append({"image_id": img_id, "score": float(row[-1]), "category_id": 1, "keypoints": row[:-1]})

@@ -43,6 +43,7 @@ class HeatmapHotPath(object):
         self.blur_w = self.decoder._weights_on(dev)
         self.ksize = int(kernel_size)
         self.pred_xy = self.label_xy = None
+        self.rows = self.acc = self.vws = None       # val_step's outputs and workspace, allocated at its first call
         self._lib = _abi.lib()
         # reduction / work-counter scratch of THIS object (zeroed once; the kernels restore the zero state). Per object
         # rather than per stream: a captured CUDA graph bakes these pointers in and may be replayed on any stream while
@@ -142,6 +143,83 @@ class HeatmapHotPath(object):
         per_warp = 1536 + 8 * (((self.w + 1) & ~1) + ((self.h + 1) & ~1)) + 4 * self.h * self.w
         return self.w % 4 == 0 and self.ksize == 11 and per_warp <= 226 * 1024 - 2048
 
+    VAL_DECODERS = {"gauss_taylor": _abi.SP_DECODE_GAUSS_TAYLOR, "basic": _abi.SP_DECODE_BASIC}
+
+    @staticmethod
+    def val_one_launch_supported(height, width, kernel_size, decoder):
+        """``sp_val_step_f32`` takes W % 4 == 0 and maps that fit in shared memory, and for the GaussTaylor decoder
+        the reference's 11 x 11 blur (the Basic decoder has no blur)."""
+        per_warp = 1536 + 8 * (((width + 1) & ~1) + ((height + 1) & ~1)) + 4 * height * width
+        blur_ok = decoder == "basic" or kernel_size == 11
+        return width % 4 == 0 and blur_ok and per_warp <= 226 * 1024 - 2048
+
+    def val_step(self, joints, pred, trans_inv, decoder="gauss_taylor"):
+        """The body of every solver's ``val()`` on one batch of predicted heatmaps (no gradient): the loss, the
+        ``HeatMapAcc`` value, the solver's decoder (``"gauss_taylor"``: the HRNet solver; ``"basic"``: the ResNet
+        solvers) and the ``kps_to_dict_`` rows. One launch (``sp_val_step_f32``) where the shape allows, otherwise
+        the stand-alone kernels with the same results (the loss up to its float64 summation order). Returns
+        ``(loss, acc, rows)``, this object's buffers: 0-d loss and acc, ``rows`` [B, 3K+1] float32 on the device
+        (``metrics.coco_eval.evaluate_person_rows`` takes them as they are, ``metrics.pose_metrics.rows_to_dicts``
+        turns them into ``kps_to_dict_``'s dicts). ``coords`` / ``maxval`` hold the decoder's output as well."""
+        if decoder not in self.VAL_DECODERS:
+            raise ValueError("decoder must be one of %s, got %r" % (sorted(self.VAL_DECODERS), decoder))
+        mode = self.VAL_DECODERS[decoder]
+        self._checked(joints, (self.batch, self.k, 3), "joints")
+        self._maps(pred, "pred")
+        if trans_inv is not None:
+            self._checked(trans_inv, (self.batch, 2, 3), "trans_inv")
+        dev = self.device
+        if self.pred_xy is None:
+            self.pred_xy = torch.empty((self.batch, self.k, 2), dtype=torch.float32, device=dev)
+            self.label_xy = torch.empty_like(self.pred_xy)
+        if self.rows is None:
+            self.rows = torch.empty((self.batch, 3 * self.k + 1), dtype=torch.float32, device=dev)
+            self.acc = torch.empty((), dtype=torch.float32, device=dev)
+        with torch.cuda.device(dev):
+            stream = _abi.stream_ptr(dev)
+            if self.val_one_launch_supported(self.h, self.w, self.ksize, decoder):
+                if self.vws is None:
+                    nbytes = int(self._lib.sp_val_step_workspace_bytes(self.batch, self.k))
+                    self.vws = torch.zeros((nbytes + 7) // 8, dtype=torch.int64, device=dev)
+                ws = self.vws
+                _abi.check_ws(self._lib.sp_val_step_f32(
+                    joints.data_ptr(), pred.data_ptr(), _abi.ptr(trans_inv), self.blur_w.data_ptr(), mode,
+                    self.weights.data_ptr(), self.loss.data_ptr(), self.acc.data_ptr(), self.rows.data_ptr(),
+                    self.coords.data_ptr(), self.maxval.data_ptr(), self.pred_xy.data_ptr(), self.label_xy.data_ptr(),
+                    ws.data_ptr(), ws.numel() * 8, self.batch, self.k, self.h, self.w, self.sigma, self.ksize,
+                    0.5, 10.0, stream), dev, stream, self)
+                return self.loss, self.acc, self.rows
+            self._val_composed(joints, pred, trans_inv, mode, stream)
+        return self.loss, self.acc, self.rows
+
+    def _val_composed(self, joints, pred, trans_inv, mode, stream):
+        """``val_step`` as the stand-alone kernels: loss + HeatMapAcc argmaxes, decoder, HeatMapAcc epilogue, rows."""
+        ws = self.ws
+        if self.w % 4 == 0:           # the fused loss kernel with its argmaxes, forward only
+            _abi.check_ws(self._lib.sp_encode_mse_fwd_bwd_f32(
+                joints.data_ptr(), pred.data_ptr(), None, None, self.weights.data_ptr(), self.loss.data_ptr(),
+                self.pred_xy.data_ptr(), self.label_xy.data_ptr(), ws.data_ptr(), ws.numel() * 8,
+                self.batch, self.k, self.h, self.w, self.sigma, 1.0, stream), self.device, stream, self)
+        else:                         # encode, forward loss, and the argmaxes of the masked maps as HeatMapAcc takes them
+            self.encode(joints)
+            _abi.check_ws(self._lib.sp_mse_fwd_bwd_f32(pred.data_ptr(), self.targets.data_ptr(), self.weights.data_ptr(),
+                                                       None, self.loss.data_ptr(), ws.data_ptr(), ws.numel() * 8,
+                                                       self.batch, self.k, self.h * self.w, 1.0, 0, stream),
+                          self.device, stream, self)
+            mask = self.weights[..., None, None]
+            for src, dst in ((pred, self.pred_xy), (self.targets, self.label_xy)):
+                _abi.check(self._lib.sp_decode_f32(_abi.dense(src * mask, torch.float32).data_ptr(), None, None, None,
+                                                   None, dst.data_ptr(), self.maxval.data_ptr(), None, self.batch,
+                                                   self.k, self.h, self.w, 0, _abi.SP_DECODE_ARGMAX, stream))
+        _abi.check_ws(self._lib.sp_decode_ws_f32(pred.data_ptr(), None, None, _abi.ptr(trans_inv), self.blur_w.data_ptr(),
+                                                 self.coords.data_ptr(), self.maxval.data_ptr(), None, self.batch, self.k,
+                                                 self.h, self.w, self.ksize, mode, self.dws.data_ptr(),
+                                                 self.dws.numel() * 8, stream), self.device, stream, self)
+        _abi.check(self._lib.sp_heatmap_acc_f32(self.pred_xy.data_ptr(), self.label_xy.data_ptr(), self.acc.data_ptr(),
+                                                self.batch, self.k, self.h, self.w, 0.5, 10.0, stream))
+        _abi.check(self._lib.sp_person_rows_f32(self.coords.data_ptr(), self.maxval.data_ptr(), self.rows.data_ptr(),
+                                                self.batch, self.k, stream))
+
     def step(self, joints, pred, trans_inv, one_launch=None):
         """encode(joints), decode(pred), loss/grad(pred, targets, weights).
 
@@ -170,16 +248,24 @@ class HeatmapHotPath(object):
         that re-runs the step with whatever the buffers hold at that moment, for the price of one graph launch
         instead of the Python -> ctypes -> launch path per kernel (the literal batch-128 configs are bound by
         exactly that). Outputs land in this object's buffers as usual."""
+        return self._capture(lambda: self.step(joints, pred, trans_inv, one_launch))
+
+    def capture_val(self, joints, pred, trans_inv, decoder="gauss_taylor"):
+        """``capture`` for ``val_step``: the returned ``replay`` re-runs the validation step on whatever the input
+        buffers hold; loss, acc and rows land in this object's buffers."""
+        return self._capture(lambda: self.val_step(joints, pred, trans_inv, decoder))
+
+    def _capture(self, run):
         stream = torch.cuda.Stream(self.device)
         stream.wait_stream(torch.cuda.current_stream(self.device))
         with torch.cuda.stream(stream):
             for _ in range(2):                       # warm-up: workspace creation, attribute caches
-                self.step(joints, pred, trans_inv, one_launch)
+                run()
         torch.cuda.current_stream(self.device).wait_stream(stream)
         torch.cuda.synchronize(self.device)
         graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(graph, stream=stream):
-            self.step(joints, pred, trans_inv, one_launch)
+            run()
         self._graph = graph                          # keeps the captured buffers alive
         return graph.replay
 
