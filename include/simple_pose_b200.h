@@ -116,6 +116,28 @@ int sp_mse_fwd_bwd(const void* pred, int pred_dtype, const float* target, const 
                    void* grad, float* loss, void* workspace, size_t workspace_bytes,
                    int B, int K, int HW, float grad_scale, const float* grad_scale_dev, int flags, void* stream);
 
+/* A2 + HeatMapAcc on the targets the loader ships, in the loss kernel's one pass -- what every solver computes per
+ * batch from the same predicts / targets / mask (processors/dp_pose_hrnet_solver.py:106-107 and 123-124 in train(),
+ * :156-157 in val(); the ResNet solvers alike):
+ *   loss = 0.5 * MSELoss(predicts * mask, targets * mask)   (+ backward when grad is given)
+ *   acc = HeatMapAcc()(predicts.mul(mask), targets.mul(mask))                  metrics/pose_metrics.py:212-245
+ * i.e. sp_mse_fwd_bwd + the two masked copies + two sp_decode_f32(SP_DECODE_ARGMAX) + sp_heatmap_acc_f32.
+ *   pred, target [B,K,H,W] (pred_dtype, grad, grad_scale_dev and flags as sp_mse_fwd_bwd; float16 / bfloat16 pred is
+ *   multiplied by the mask in float32, as autocast's pred.mul(mask)); mask [B,K] f32; loss (1 f32) and acc (1 f32)
+ *   are required (forward calls only: the backward-only call stays sp_mse_fwd_bwd with loss == NULL);
+ *   pred_xy / label_xy [B,K,2] f32: heat_map_to_axis of the two masked maps (both NULL = kept in the workspace);
+ *   distance_thresh, norm_frac: HeatMapAcc's constructor arguments (0.5, 10). H and W are separate because the
+ *   coordinates and the thresholds are in (W, H) units. K <= 4096.
+ * workspace: sp_mse_acc_workspace_bytes(B, K) bytes (0 = invalid sizes), 16-byte aligned, ZERO-FILLED ONCE by the
+ * caller: the reduction workspace, the per-map argmax keys and room for the axes; every launch returns it to the
+ * zero state, so it can be reused (and a captured graph replayed) on the same stream.
+ * loss and grad are bit-identical to sp_mse_fwd_bwd, pred_xy / label_xy / acc to the composed calls. */
+size_t sp_mse_acc_workspace_bytes(int B, int K);
+int sp_mse_acc_fwd_bwd(const void* pred, int pred_dtype, const float* target, const float* mask, void* grad,
+                       float* loss, float* acc, float* pred_xy, float* label_xy, void* workspace, size_t workspace_bytes,
+                       int B, int K, int H, int W, float grad_scale, const float* grad_scale_dev,
+                       float distance_thresh, float norm_frac, int flags, void* stream);
+
 /* A1+A2(+HeatMapAcc) fused -- SURVEY section 8f ranks 1 and 2: targets are encoded on the fly and never
  * written (unless `targets` is given), so one pass reads pred and writes grad.
  *   targets, mask = get_heat_map(joints)                        commons/transforms.py:167-191

@@ -39,6 +39,9 @@ SIGNATURES = {
                                    c_int, c_int, c_int, c_flt, c_int, c_void]),
     "sp_mse_fwd_bwd": (c_int, [c_void, c_int, c_void, c_void, c_void, c_void, c_void, c_size,
                                c_int, c_int, c_int, c_flt, c_void, c_int, c_void]),
+    "sp_mse_acc_workspace_bytes": (c_size, [c_int, c_int]),
+    "sp_mse_acc_fwd_bwd": (c_int, [c_void, c_int] + [c_void] * 7 + [c_void, c_size, c_int, c_int, c_int, c_int, c_flt, c_void,
+                                                                     c_flt, c_flt, c_int, c_void]),
     "sp_encode_mse_fwd_bwd_f32": (c_int, [c_void] * 9 + [c_size, c_int, c_int, c_int, c_int, c_dbl, c_flt, c_void]),
     "sp_encode_mse_fwd_bwd": (c_int, [c_void, c_void, c_int] + [c_void] * 7 + [c_size, c_int, c_int, c_int, c_int, c_dbl, c_flt, c_void, c_void]),
     "sp_step_f32": (c_int, [c_void] * 13 + [c_size, c_int, c_int, c_int, c_int, c_dbl, c_int, c_flt, c_void]),

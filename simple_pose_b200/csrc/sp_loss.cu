@@ -22,9 +22,17 @@
 //
 // Arithmetic follows ATen so that grad is bit-identical for finite inputs:
 //   d = fl(m*p) - fl(m*t); grad = ((fl(2/N) * d) * 0.5) * m   (mse_loss_backward, then mul backward)
+//
+// ACC (forward calls of sp_mse_acc_fwd_bwd): the same pass also finds the argmax of both masked maps, m*p and m*t,
+// which is what HeatMapAcc()(pred.mul(mask), target.mul(mask)) decodes (metrics/pose_metrics.py:223-224), and the
+// last block runs the HeatMapAcc epilogue. A map may be split over lanes, warps and blocks (the ring kernel cuts its
+// ranges by chunk count), so every partial argmax becomes a 64-bit key whose unsigned order is sp::better's and the
+// partials meet in one atomicMax per (map, warp that scanned part of it) -- the result cannot depend on the split.
 #include "sp_common.cuh"
 #include "sp_reduce.cuh"
 #include "sp_lowp.cuh"
+#include "sp_decode_dev.cuh"
+#include "sp_train_dev.cuh"
 
 #ifdef SP_TRAIN_TRACE
 __device__ long long* g_loss_trace_ptr = nullptr;     // scratch instrumentation, trace build only
@@ -55,19 +63,90 @@ __device__ __forceinline__ float sq_err_and_grad(float p, float t, float m, floa
     return d;
 }
 
-template <bool VEC4, bool WRITE_GRAD>
+// ---- HeatMapAcc riding along with the loss (ACC) ------------------------------------------------------------------
+struct AccOut {
+    unsigned long long* keys;    // [B*K][2] argmax keys of (m*p, m*t) in the caller's workspace, zero between launches
+    float2* pred_xy;             // [B*K] heat_map_to_axis of m*p / m*t (the caller's buffers or the workspace's)
+    float2* label_xy;
+    float* acc;
+    int B, K, W;
+    float norm_x, norm_y, thresh;
+};
+
+// High word: the value in an order where NaN is above +inf and -0 == +0; low word: ~index, so the smaller index wins
+// among equal values (and among NaNs). Key 0 is below every element: a map nobody scanned.
+__device__ __forceinline__ unsigned long long argmax_key(float v, int i) {
+    unsigned int o = 0xffffffffu;
+    if (v == v) {
+        const unsigned int b = __float_as_uint(v == 0.f ? 0.f : v);
+        o = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+    }
+    return ((unsigned long long)o << 32) | (unsigned int)~i;
+}
+
+// heat_map_to_axis of a merged key; key 0 (a map whose mask is 0: its products are 0 or NaN) gives (0, 0) as well
+__device__ __forceinline__ float2 key_axis(unsigned long long key, int W) {
+    const unsigned int o = (unsigned int)(key >> 32);
+    const float v = (o == 0xffffffffu || o == 0u) ? CUDART_NAN_F : __uint_as_float((o & 0x80000000u) ? (o ^ 0x80000000u) : ~o);
+    return sp_trn::axis_of(v, (int)~(unsigned int)key, W);
+}
+
+// One warp's share of a map seen through QuadBest (each lane visits its quads in increasing order; 4*bq + bsub is the
+// flat index relative to `first`) merged into the map's key. A NaN or an infinity among them: the exact scan of the
+// n elements at `src` (a superset of what the warp saw, starting at flat index `first`) decides instead.
+template <typename PT>
+__device__ __forceinline__ void merge_quads(const sp_trn::QuadBest& b, const PT* src, float mk, int n, int first, int lane,
+                                            unsigned long long* key) {
+    float v;
+    int i;
+    if (__any_sync(SP_FULL, b.poison != b.poison)) {
+        sp_trn::MaskedPredView<PT> view{src, mk};
+        sp_trn::argmax_exact_scan(view, n, lane, v, i);
+    } else {
+        v = sp_trn::warp_max_f32(b.best);
+        if (v == -CUDART_INF_F) return;          // the warp had no element of this map (an infinity is poison)
+        i = (int)__reduce_min_sync(SP_FULL, (b.best == v) ? (unsigned)(4 * b.bq + b.bsub) : 0x7fffffffu);
+    }
+    if (lane == 0) atomicMax(key, argmax_key(v, first + i));
+}
+
+// Scalar paths: this lane's first maximal element by sp::better, merged over the warp, then into the map's key.
+__device__ __forceinline__ void merge_scalar(float bv, int bi, int lane, unsigned long long* key) {
+    const sp_dec::Peak pk = sp_dec::warp_best(bv, bi);
+    if (lane == 0 && pk.index != 0x7fffffff) atomicMax(key, argmax_key(pk.value, pk.index));
+}
+
+// Run by ALL threads of the last block of the loss reduction (it has acquired every block's keys): the keys become
+// heat_map_to_axis coordinates and return to zero, then the HeatMapAcc epilogue of heatmap_acc_kernel / val_step_kernel.
+// counters: 2K ints of shared memory.
+__device__ __forceinline__ void acc_epilogue(const AccOut& A, int* counters) {
+    const int n = A.B * A.K;
+    ulonglong2* keys = reinterpret_cast<ulonglong2*>(A.keys);
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        const ulonglong2 k = __ldcg(keys + i);
+        keys[i] = make_ulonglong2(0ull, 0ull);
+        A.pred_xy[i] = key_axis(k.x, A.W);
+        A.label_xy[i] = key_axis(k.y, A.W);
+    }
+    __syncthreads();
+    sp_trn::heatmap_acc_block<true>(A.pred_xy, A.label_xy, A.acc, A.B, A.K, A.norm_x, A.norm_y, A.thresh, counters);
+}
+
+template <bool VEC4, bool WRITE_GRAD, bool ACC>
 __global__ void __launch_bounds__(kThreads)
 mse_fwd_bwd_kernel(const float* __restrict__ pred, const float* __restrict__ target,
                    const float* __restrict__ mask, float* __restrict__ grad, float* __restrict__ loss,
                    MseWorkspace* __restrict__ ws, int nmaps, int hw, float norm, float half_scale,
-                   double inv_count, int skip_masked) {
+                   double inv_count, int skip_masked, const AccOut A) {
     double block_sum = 0.0;
     sp::grid_dep_wait();
+    const int lane = threadIdx.x & 31;
 
     for (int m = blockIdx.x; m < nmaps; m += gridDim.x) {
         const float mk = __ldg(mask + m);
         const size_t base = (size_t)m * hw;
         float acc = 0.f;
+        const bool track = ACC && mk != 0.f;      // a masked-out map's products are 0 or NaN: (0, 0) either way
         if (skip_masked && mk == 0.f) {
             if (WRITE_GRAD) {
                 if (VEC4) {
@@ -84,6 +163,8 @@ mse_fwd_bwd_kernel(const float* __restrict__ pred, const float* __restrict__ tar
             const float4* t4 = reinterpret_cast<const float4*>(target + base);
             float4* g4 = reinterpret_cast<float4*>(grad + base);
             const int nq = hw >> 2;
+            sp_trn::QuadBest bp, bt;
+            if (ACC) { bp.init(); bt.init(); }
 #pragma unroll 4
             for (int q = threadIdx.x; q < nq; q += kThreads) {
                 const float4 p = ldg_stream(p4 + q);
@@ -95,19 +176,43 @@ mse_fwd_bwd_kernel(const float* __restrict__ pred, const float* __restrict__ tar
                 d = sq_err_and_grad(p.z, t.z, mk, norm, half_scale, g.z); acc = fmaf(d, d, acc);
                 d = sq_err_and_grad(p.w, t.w, mk, norm, half_scale, g.w); acc = fmaf(d, d, acc);
                 if (WRITE_GRAD) g4[q] = g;
+                if (ACC && track) {
+                    bp.push(__fmul_rn(mk, p.x), __fmul_rn(mk, p.y), __fmul_rn(mk, p.z), __fmul_rn(mk, p.w), q);
+                    bt.push(__fmul_rn(mk, t.x), __fmul_rn(mk, t.y), __fmul_rn(mk, t.z), __fmul_rn(mk, t.w), q);
+                }
+            }
+            if (ACC && track) {
+                merge_quads(bp, pred + base, mk, hw, 0, lane, A.keys + 2 * (size_t)m);
+                merge_quads(bt, target + base, mk, hw, 0, lane, A.keys + 2 * (size_t)m + 1);
             }
         } else {
+            float bvp = -CUDART_INF_F, bvt = -CUDART_INF_F;
+            int bip = 0x7fffffff, bit = 0x7fffffff;
             for (int i = threadIdx.x; i < hw; i += kThreads) {
                 float g;
-                const float d = sq_err_and_grad(pred[base + i], target[base + i], mk, norm, half_scale, g);
+                const float pv = pred[base + i], tv = target[base + i];
+                const float d = sq_err_and_grad(pv, tv, mk, norm, half_scale, g);
                 acc = fmaf(d, d, acc);
                 if (WRITE_GRAD) grad[base + i] = g;
+                if (ACC && track) {
+                    const float mp = __fmul_rn(mk, pv), mt = __fmul_rn(mk, tv);
+                    if (sp::better(mp, i, bvp, bip)) { bvp = mp; bip = i; }
+                    if (sp::better(mt, i, bvt, bit)) { bvt = mt; bit = i; }
+                }
+            }
+            if (ACC && track) {
+                merge_scalar(bvp, bip, lane, A.keys + 2 * (size_t)m);
+                merge_scalar(bvt, bit, lane, A.keys + 2 * (size_t)m + 1);
             }
         }
         block_sum += (double)acc;
     }
 
-    finish_loss<kThreads>(block_sum, ws, loss, inv_count);
+    const bool last = finish_loss<kThreads>(block_sum, ws, loss, inv_count);
+    if constexpr (ACC) {
+        extern __shared__ int acc_counters[];     // 2K ints
+        if (last) acc_epilogue(A, acc_counters);
+    }
 }
 
 // Mixed-precision variant (torch.cuda.amp, processors/dp_pose_hrnet_solver.py:111-120): `pred` arrives in the
@@ -117,21 +222,24 @@ mse_fwd_bwd_kernel(const float* __restrict__ pred, const float* __restrict__ tar
 // (GradScaler's scale, read here from device memory so that no host sync is needed) has been applied in
 // float32 -- which is the whole point of loss scaling for float16. Eight elements per thread per step:
 // one 16-byte load of pred (8 x PT; 2 x float4 for float32), two of target, one 16-byte grad store.
-// loss == nullptr: backward only (no reduction); grad == nullptr: forward only.
-template <typename PT, bool VEC8>
+// loss == nullptr: backward only (no reduction); grad == nullptr: forward only. ACC only with loss != nullptr.
+template <typename PT, bool VEC8, bool ACC>
 __global__ void __launch_bounds__(kThreads)
 mse_mixed_kernel(const PT* __restrict__ pred, const float* __restrict__ target, const float* __restrict__ mask,
                  PT* __restrict__ grad, float* __restrict__ loss, MseWorkspace* __restrict__ ws, int nmaps, int hw,
-                 float norm, float half_scale_host, const float* __restrict__ scale_dev, double inv_count, int skip_masked) {
+                 float norm, float half_scale_host, const float* __restrict__ scale_dev, double inv_count, int skip_masked,
+                 const AccOut A) {
     double block_sum = 0.0;
     sp::grid_dep_wait();
     const float half_scale = scale_dev ? __fmul_rn(half_scale_host, __ldg(scale_dev)) : half_scale_host;
     const bool write_grad = grad != nullptr;
+    const int lane = threadIdx.x & 31;
 
     for (int m = blockIdx.x; m < nmaps; m += gridDim.x) {
         const float mk = __ldg(mask + m);
         const size_t base = (size_t)m * hw;
         float acc = 0.f;
+        const bool track = ACC && mk != 0.f;
         if (skip_masked && mk == 0.f) {
             if (write_grad)
                 for (int i = threadIdx.x; i < hw; i += kThreads) grad[base + i] = sp_lowp::from_float<PT>(0.f);
@@ -139,6 +247,8 @@ mse_mixed_kernel(const PT* __restrict__ pred, const float* __restrict__ target, 
         }
         if (VEC8) {
             const int n8 = hw >> 3;
+            sp_trn::QuadBest bp, bt;
+            if (ACC) { bp.init(); bt.init(); }
 #pragma unroll 2
             for (int o = threadIdx.x; o < n8; o += kThreads) {
                 float p[8], g[8];
@@ -152,18 +262,49 @@ mse_mixed_kernel(const PT* __restrict__ pred, const float* __restrict__ target, 
                     acc = fmaf(d, d, acc);
                 }
                 if (write_grad) sp_lowp::store8(grad + base + 8 * (size_t)o, g);
+                if (ACC && track) {       // float(p) * m: the float32 promotion autocast's pred.mul(mask) computes
+#pragma unroll
+                    for (int h = 0; h < 2; ++h) {
+                        bp.push(__fmul_rn(mk, p[4 * h]), __fmul_rn(mk, p[4 * h + 1]), __fmul_rn(mk, p[4 * h + 2]),
+                                __fmul_rn(mk, p[4 * h + 3]), 2 * o + h);
+                        bt.push(__fmul_rn(mk, t[4 * h]), __fmul_rn(mk, t[4 * h + 1]), __fmul_rn(mk, t[4 * h + 2]),
+                                __fmul_rn(mk, t[4 * h + 3]), 2 * o + h);
+                    }
+                }
+            }
+            if (ACC && track) {
+                merge_quads(bp, pred + base, mk, hw, 0, lane, A.keys + 2 * (size_t)m);
+                merge_quads(bt, target + base, mk, hw, 0, lane, A.keys + 2 * (size_t)m + 1);
             }
         } else {
+            float bvp = -CUDART_INF_F, bvt = -CUDART_INF_F;
+            int bip = 0x7fffffff, bit = 0x7fffffff;
             for (int i = threadIdx.x; i < hw; i += kThreads) {
                 float g;
-                const float d = sq_err_and_grad(sp_lowp::to_float(pred[base + i]), target[base + i], mk, norm, half_scale, g);
+                const float pv = sp_lowp::to_float(pred[base + i]), tv = target[base + i];
+                const float d = sq_err_and_grad(pv, tv, mk, norm, half_scale, g);
                 acc = fmaf(d, d, acc);
                 if (write_grad) grad[base + i] = sp_lowp::from_float<PT>(g);
+                if (ACC && track) {
+                    const float mp = __fmul_rn(mk, pv), mt = __fmul_rn(mk, tv);
+                    if (sp::better(mp, i, bvp, bip)) { bvp = mp; bip = i; }
+                    if (sp::better(mt, i, bvt, bit)) { bvt = mt; bit = i; }
+                }
+            }
+            if (ACC && track) {
+                merge_scalar(bvp, bip, lane, A.keys + 2 * (size_t)m);
+                merge_scalar(bvt, bit, lane, A.keys + 2 * (size_t)m + 1);
             }
         }
         block_sum += (double)acc;
     }
-    if (loss != nullptr) finish_loss<kThreads>(block_sum, ws, loss, inv_count);
+    if (loss != nullptr) {
+        const bool last = finish_loss<kThreads>(block_sum, ws, loss, inv_count);
+        if constexpr (ACC) {
+            extern __shared__ int acc_counters[];
+            if (last) acc_epilogue(A, acc_counters);
+        }
+    }
 }
 
 // dynamic smem: [mbarriers 1024 B][per warp: ring x (pred chunk | target chunk)]
@@ -171,12 +312,14 @@ constexpr int kRingBarBytes = 1024;
 
 // A variant that sent the gradient out through the TMA too (written into the drained slot, cp.async.bulk shared -> global)
 // was within 1-2 % either way warm and 12 % slower from a cold cache, so the gradient stays on register stores (DESIGN.md, section 4).
-template <bool WRITE_GRAD>
+// ACC: the argmax is taken over each staged chunk before its slot is re-armed (the exact scan of a chunk holding a NaN
+// or an infinity reads the slot too); the last block's HeatMapAcc counters go where the slots were.
+template <bool WRITE_GRAD, bool ACC>
 __global__ void __launch_bounds__(1024, 1)
 mse_ring_kernel(const float* __restrict__ pred, const float* __restrict__ target, const float* __restrict__ mask,
                 float* __restrict__ grad, float* __restrict__ loss, MseWorkspace* __restrict__ ws,
                 long long nchunks, int chunk_quads, int chunks_per_map, int nwarps, int ring,
-                float norm, float half_scale, double inv_count) {
+                float norm, float half_scale, double inv_count, const AccOut A) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
@@ -220,6 +363,9 @@ mse_ring_kernel(const float* __restrict__ pred, const float* __restrict__ target
         const float4* t4 = reinterpret_cast<const float4*>(slots + (size_t)cs * 2 * chunk_bytes + chunk_bytes);
         float4* g4 = reinterpret_cast<float4*>(grad + i * chunk_floats);
         float acc = 0.f;
+        const bool track = ACC && mk != 0.f;
+        sp_trn::QuadBest bp, bt;
+        if (ACC) { bp.init(); bt.init(); }
 #pragma unroll 3
         for (int q = lane; q < chunk_quads; q += 32) {
             const float4 p = p4[q];
@@ -231,8 +377,18 @@ mse_ring_kernel(const float* __restrict__ pred, const float* __restrict__ target
             d = sq_err_and_grad(p.z, t.z, mk, norm, half_scale, g.z); acc = fmaf(d, d, acc);
             d = sq_err_and_grad(p.w, t.w, mk, norm, half_scale, g.w); acc = fmaf(d, d, acc);
             if (WRITE_GRAD) g4[q] = g;
+            if (ACC && track) {
+                bp.push(__fmul_rn(mk, p.x), __fmul_rn(mk, p.y), __fmul_rn(mk, p.z), __fmul_rn(mk, p.w), q);
+                bt.push(__fmul_rn(mk, t.x), __fmul_rn(mk, t.y), __fmul_rn(mk, t.z), __fmul_rn(mk, t.w), q);
+            }
         }
         sum_sq += (double)acc;
+        if (ACC && track) {
+            const long long map = i / chunks_per_map;
+            const int first = (int)(i - map * chunks_per_map) * (int)chunk_floats;     // the chunk's place in its map
+            merge_quads(bp, reinterpret_cast<const float*>(p4), mk, (int)chunk_floats, first, lane, A.keys + 2 * map);
+            merge_quads(bt, reinterpret_cast<const float*>(t4), mk, (int)chunk_floats, first, lane, A.keys + 2 * map + 1);
+        }
         __syncwarp();
         if (lane == 0) {
             sp::fence_proxy_async_smem();
@@ -248,7 +404,10 @@ mse_ring_kernel(const float* __restrict__ pred, const float* __restrict__ target
         t[0] = trace_t0; t[1] = loss_gtime(); t[2] = smid; t[3] = (long long)(hi - lo);
     }
 #endif
-    finish_loss<1024>(sum_sq, ws, loss, inv_count);
+    const bool last = finish_loss<1024>(sum_sq, ws, loss, inv_count);
+    if constexpr (ACC) {
+        if (last) acc_epilogue(A, reinterpret_cast<int*>(smem_raw + kRingBarBytes));
+    }
 }
 
 __global__ void __launch_bounds__(256)
@@ -271,22 +430,17 @@ scale_inplace_kernel(float* __restrict__ data, long long n, const float* __restr
 
 extern "C" size_t sp_mse_workspace_bytes(void) { return sizeof(MseWorkspace); }
 
-extern "C" int sp_mse_fwd_bwd_f32(const float* pred, const float* target, const float* mask,
-                                  float* grad, float* loss, void* workspace, size_t workspace_bytes,
-                                  int B, int K, int HW, float grad_scale, int flags, void* stream) {
-    SP_RETURN_IF(!pred || !target || !mask || !loss || !workspace, SP_ERR_BAD_ARGUMENT);
-    SP_RETURN_IF(B <= 0 || K <= 0 || HW <= 0, SP_ERR_BAD_ARGUMENT);
-    SP_RETURN_IF((long long)B * K > 0x7fffffffLL, SP_ERR_UNSUPPORTED);
-    SP_RETURN_IF(workspace_bytes < sizeof(MseWorkspace), SP_ERR_WORKSPACE);
-    SP_RETURN_IF(!sp_aligned16(workspace), SP_ERR_BAD_ALIGNMENT);
+// sp_mse_fwd_bwd_f32 after its argument checks; A.acc != nullptr: with the HeatMapAcc argmaxes and epilogue (ACC)
+static int mse_f32(const float* pred, const float* target, const float* mask, float* grad, float* loss, MseWorkspace* ws,
+                   int B, int K, int HW, float grad_scale, int flags, cudaStream_t st, const AccOut& A) {
     const int nmaps = B * K;
     const double count = (double)B * (double)K * (double)HW;
     const float norm = (float)(2.0 / count);       // ATen: norm = 2 / numel, applied in float32
     const float half_scale = 0.5f * grad_scale;    // the 0.5 of the loss expression times upstream grad
     const bool vec4 = (HW % 4 == 0) && sp_aligned16(pred) && sp_aligned16(target) && (!grad || sp_aligned16(grad));
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    MseWorkspace* ws = static_cast<MseWorkspace*>(workspace);
     const int skip = (flags & SP_MSE_SKIP_MASKED) ? 1 : 0;
+    const bool acc = A.acc != nullptr;
+    const size_t counter_bytes = (size_t)2 * K * sizeof(int);      // HeatMapAcc epilogue of the last block
 
     // ring kernel: needs 16-byte rows and a chunk size (in quads) that divides the map
     const SpTuning& tune = sp_tuning();
@@ -307,18 +461,18 @@ extern "C" int sp_mse_fwd_bwd_f32(const float* pred, const float* target, const 
             if (nwarps > 32) nwarps = 32;
             const size_t slot_bytes = (size_t)chunk_quads * 32;      // pred chunk + target chunk
             while (nwarps > 1 && (kRingBarBytes + (size_t)nwarps * ring * slot_bytes > 226 * 1024 || nwarps * ring * 8 > kRingBarBytes)) --nwarps;
-            const size_t smem = kRingBarBytes + (size_t)nwarps * ring * slot_bytes;
+            size_t smem = kRingBarBytes + (size_t)nwarps * ring * slot_bytes;
             if (smem <= 226 * 1024 && nwarps * ring * 8 <= kRingBarBytes) {    // 1 KB spare for static shared memory
                 const long long nchunks = (long long)nmaps * (nq / chunk_quads);
                 int grid = sp_sm_count();
                 if ((long long)grid * nwarps > nchunks) grid = (int)((nchunks + nwarps - 1) / nwarps);
-                if (grad) {
-                    SP_CUDA(sp_launch_smem(mse_ring_kernel<true>, dim3(grid), dim3(nwarps * 32), smem, st, pred, target, mask, grad, loss, ws,
-                                      nchunks, chunk_quads, nq / chunk_quads, nwarps, ring, norm, half_scale, 1.0 / count));
-                } else {
-                    SP_CUDA(sp_launch_smem(mse_ring_kernel<false>, dim3(grid), dim3(nwarps * 32), smem, st, pred, target, mask, grad, loss, ws,
-                                      nchunks, chunk_quads, nq / chunk_quads, nwarps, ring, norm, half_scale, 1.0 / count));
-                }
+                if (acc && smem < kRingBarBytes + counter_bytes) smem = kRingBarBytes + counter_bytes;
+#define SP_LAUNCH_RING(G, AC) \
+    SP_CUDA(sp_launch_smem(mse_ring_kernel<G, AC>, dim3(grid), dim3(nwarps * 32), smem, st, pred, target, mask, grad, loss, ws, \
+                           nchunks, chunk_quads, nq / chunk_quads, nwarps, ring, norm, half_scale, 1.0 / count, A))
+                if (acc) { if (grad) SP_LAUNCH_RING(true, true); else SP_LAUNCH_RING(false, true); }
+                else     { if (grad) SP_LAUNCH_RING(true, false); else SP_LAUNCH_RING(false, false); }
+#undef SP_LAUNCH_RING
                 return 0;
             }
         }
@@ -327,27 +481,64 @@ extern "C" int sp_mse_fwd_bwd_f32(const float* pred, const float* target, const 
     int grid = sp_sm_count() * 8;
     if (grid > nmaps) grid = nmaps;
     if (grid > kMaxPartials) grid = kMaxPartials;
-#define SP_LAUNCH_MSE(V, G) \
-    SP_CUDA(sp_launch(mse_fwd_bwd_kernel<V, G>, dim3(grid), dim3(kThreads), 0, st, pred, target, mask, grad, loss, ws, nmaps, HW, norm, half_scale, 1.0 / count, skip))
-    if (vec4) { if (grad) SP_LAUNCH_MSE(true, true); else SP_LAUNCH_MSE(true, false); }
-    else      { if (grad) SP_LAUNCH_MSE(false, true); else SP_LAUNCH_MSE(false, false); }
+#define SP_LAUNCH_MSE(V, G, AC) \
+    SP_CUDA(sp_launch(mse_fwd_bwd_kernel<V, G, AC>, dim3(grid), dim3(kThreads), AC ? counter_bytes : 0, st, pred, target, mask, grad, \
+                      loss, ws, nmaps, HW, norm, half_scale, 1.0 / count, skip, A))
+    if (acc) {
+        if (vec4) { if (grad) SP_LAUNCH_MSE(true, true, true); else SP_LAUNCH_MSE(true, false, true); }
+        else      { if (grad) SP_LAUNCH_MSE(false, true, true); else SP_LAUNCH_MSE(false, false, true); }
+    } else {
+        if (vec4) { if (grad) SP_LAUNCH_MSE(true, true, false); else SP_LAUNCH_MSE(true, false, false); }
+        else      { if (grad) SP_LAUNCH_MSE(false, true, false); else SP_LAUNCH_MSE(false, false, false); }
+    }
 #undef SP_LAUNCH_MSE
     return 0;
+}
+
+extern "C" int sp_mse_fwd_bwd_f32(const float* pred, const float* target, const float* mask,
+                                  float* grad, float* loss, void* workspace, size_t workspace_bytes,
+                                  int B, int K, int HW, float grad_scale, int flags, void* stream) {
+    SP_RETURN_IF(!pred || !target || !mask || !loss || !workspace, SP_ERR_BAD_ARGUMENT);
+    SP_RETURN_IF(B <= 0 || K <= 0 || HW <= 0, SP_ERR_BAD_ARGUMENT);
+    SP_RETURN_IF((long long)B * K > 0x7fffffffLL, SP_ERR_UNSUPPORTED);
+    SP_RETURN_IF(workspace_bytes < sizeof(MseWorkspace), SP_ERR_WORKSPACE);
+    SP_RETURN_IF(!sp_aligned16(workspace), SP_ERR_BAD_ALIGNMENT);
+    return mse_f32(pred, target, mask, grad, loss, static_cast<MseWorkspace*>(workspace), B, K, HW, grad_scale, flags,
+                   static_cast<cudaStream_t>(stream), AccOut{});
 }
 
 template <typename PT>
 static int launch_mixed(const void* pred, const float* target, const float* mask, void* grad, float* loss, MseWorkspace* ws,
                         int nmaps, int HW, float norm, float half_scale, const float* scale_dev, double inv_count, int skip,
-                        cudaStream_t st) {
+                        cudaStream_t st, const AccOut& A) {
     const bool vec8 = (HW % 8 == 0) && sp_aligned16(pred) && sp_aligned16(target) && (!grad || sp_aligned16(grad));
     int grid = sp_sm_count() * 8;
     if (grid > nmaps) grid = nmaps;
     if (grid > kMaxPartials) grid = kMaxPartials;
     const PT* p = static_cast<const PT*>(pred);
     PT* g = static_cast<PT*>(grad);
-    if (vec8) SP_CUDA(sp_launch(mse_mixed_kernel<PT, true>, dim3(grid), dim3(kThreads), 0, st, p, target, mask, g, loss, ws, nmaps, HW, norm, half_scale, scale_dev, inv_count, skip));
-    else      SP_CUDA(sp_launch(mse_mixed_kernel<PT, false>, dim3(grid), dim3(kThreads), 0, st, p, target, mask, g, loss, ws, nmaps, HW, norm, half_scale, scale_dev, inv_count, skip));
+    const size_t counter_bytes = A.acc ? (size_t)2 * A.K * sizeof(int) : 0;
+#define SP_LAUNCH_MIXED(V8, AC) \
+    SP_CUDA(sp_launch(mse_mixed_kernel<PT, V8, AC>, dim3(grid), dim3(kThreads), counter_bytes, st, p, target, mask, g, loss, ws, \
+                      nmaps, HW, norm, half_scale, scale_dev, inv_count, skip, A))
+    if (A.acc) { if (vec8) SP_LAUNCH_MIXED(true, true); else SP_LAUNCH_MIXED(false, true); }
+    else       { if (vec8) SP_LAUNCH_MIXED(true, false); else SP_LAUNCH_MIXED(false, false); }
+#undef SP_LAUNCH_MIXED
     return 0;
+}
+
+static int mixed_dispatch(const void* pred, int pred_dtype, const float* target, const float* mask, void* grad, float* loss,
+                          MseWorkspace* ws, int B, int K, int HW, float grad_scale, const float* grad_scale_dev, int flags,
+                          cudaStream_t st, const AccOut& A) {
+    const double count = (double)B * (double)K * (double)HW;
+    const float norm = (float)(2.0 / count);
+    const float half_scale = 0.5f * grad_scale;
+    const int skip = (flags & SP_MSE_SKIP_MASKED) ? 1 : 0;
+    if (pred_dtype == SP_DTYPE_F16)
+        return launch_mixed<__half>(pred, target, mask, grad, loss, ws, B * K, HW, norm, half_scale, grad_scale_dev, 1.0 / count, skip, st, A);
+    if (pred_dtype == SP_DTYPE_BF16)
+        return launch_mixed<__nv_bfloat16>(pred, target, mask, grad, loss, ws, B * K, HW, norm, half_scale, grad_scale_dev, 1.0 / count, skip, st, A);
+    return launch_mixed<float>(pred, target, mask, grad, loss, ws, B * K, HW, norm, half_scale, grad_scale_dev, 1.0 / count, skip, st, A);
 }
 
 extern "C" int sp_mse_fwd_bwd(const void* pred, int pred_dtype, const float* target, const float* mask,
@@ -366,17 +557,50 @@ extern "C" int sp_mse_fwd_bwd(const void* pred, int pred_dtype, const float* tar
         SP_RETURN_IF(workspace_bytes < sizeof(MseWorkspace), SP_ERR_WORKSPACE);
         SP_RETURN_IF(!sp_aligned16(workspace), SP_ERR_BAD_ALIGNMENT);
     }
-    const double count = (double)B * (double)K * (double)HW;
-    const float norm = (float)(2.0 / count);
-    const float half_scale = 0.5f * grad_scale;
-    const int skip = (flags & SP_MSE_SKIP_MASKED) ? 1 : 0;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    return mixed_dispatch(pred, pred_dtype, target, mask, grad, loss, static_cast<MseWorkspace*>(workspace), B, K, HW, grad_scale,
+                          grad_scale_dev, flags, static_cast<cudaStream_t>(stream), AccOut{});
+}
+
+// workspace of sp_mse_acc_fwd_bwd: the reduction workspace, the argmax keys (16 bytes per map), room for the axes (16 bytes
+// per map, used when the caller passes no pred_xy / label_xy)
+static size_t acc_keys_offset() { return (sizeof(MseWorkspace) + 15) & ~(size_t)15; }
+
+extern "C" size_t sp_mse_acc_workspace_bytes(int B, int K) {
+    if (B <= 0 || K <= 0 || (long long)B * K > 0x7fffffffLL) return 0;
+    return acc_keys_offset() + 32 * (size_t)B * K;
+}
+
+extern "C" int sp_mse_acc_fwd_bwd(const void* pred, int pred_dtype, const float* target, const float* mask, void* grad,
+                                  float* loss, float* acc, float* pred_xy, float* label_xy, void* workspace,
+                                  size_t workspace_bytes, int B, int K, int H, int W, float grad_scale,
+                                  const float* grad_scale_dev, float distance_thresh, float norm_frac, int flags, void* stream) {
+    SP_RETURN_IF(pred_dtype != SP_DTYPE_F32 && pred_dtype != SP_DTYPE_F16 && pred_dtype != SP_DTYPE_BF16, SP_ERR_BAD_ARGUMENT);
+    SP_RETURN_IF(!pred || !target || !mask || !loss || !acc || !workspace, SP_ERR_BAD_ARGUMENT);
+    SP_RETURN_IF((pred_xy == nullptr) != (label_xy == nullptr), SP_ERR_BAD_ARGUMENT);     // both NULL: kept in the workspace
+    SP_RETURN_IF(B <= 0 || K <= 0 || H <= 0 || W <= 0 || !(norm_frac > 0.f), SP_ERR_BAD_ARGUMENT);
+    SP_RETURN_IF((long long)B * K > 0x7fffffffLL || (long long)H * W > 0x7fffffffLL || K > 4096, SP_ERR_UNSUPPORTED);
+    SP_RETURN_IF(workspace_bytes < sp_mse_acc_workspace_bytes(B, K), SP_ERR_WORKSPACE);
+    SP_RETURN_IF(!sp_aligned16(workspace) || (pred_xy && (!sp_aligned16(pred_xy) || !sp_aligned16(label_xy))), SP_ERR_BAD_ALIGNMENT);
+    unsigned char* wsb = static_cast<unsigned char*>(workspace);
+    if (!pred_xy) {
+        pred_xy = reinterpret_cast<float*>(wsb + acc_keys_offset() + 16 * (size_t)B * K);
+        label_xy = pred_xy + 2 * (size_t)B * K;
+    }
+    AccOut A;
+    A.keys = reinterpret_cast<unsigned long long*>(wsb + acc_keys_offset());
+    A.pred_xy = reinterpret_cast<float2*>(pred_xy);
+    A.label_xy = reinterpret_cast<float2*>(label_xy);
+    A.acc = acc;
+    A.B = B; A.K = K; A.W = W;
+    A.norm_x = (float)W / norm_frac;           // norm = tensor([W, H], float32) / norm_frac, as sp_heatmap_acc_f32
+    A.norm_y = (float)H / norm_frac;
+    A.thresh = distance_thresh;
     MseWorkspace* ws = static_cast<MseWorkspace*>(workspace);
-    if (pred_dtype == SP_DTYPE_F16)
-        return launch_mixed<__half>(pred, target, mask, grad, loss, ws, B * K, HW, norm, half_scale, grad_scale_dev, 1.0 / count, skip, st);
-    if (pred_dtype == SP_DTYPE_BF16)
-        return launch_mixed<__nv_bfloat16>(pred, target, mask, grad, loss, ws, B * K, HW, norm, half_scale, grad_scale_dev, 1.0 / count, skip, st);
-    return launch_mixed<float>(pred, target, mask, grad, loss, ws, B * K, HW, norm, half_scale, grad_scale_dev, 1.0 / count, skip, st);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (pred_dtype == SP_DTYPE_F32 && !grad_scale_dev)             // the float32 fast path, as sp_mse_fwd_bwd
+        return mse_f32(static_cast<const float*>(pred), target, mask, static_cast<float*>(grad), loss, ws, B, K, H * W, grad_scale,
+                       flags, st, A);
+    return mixed_dispatch(pred, pred_dtype, target, mask, grad, loss, ws, B, K, H * W, grad_scale, grad_scale_dev, flags, st, A);
 }
 
 extern "C" int sp_scale_inplace_f32(float* data, long long n, const float* scale_dev, void* stream) {

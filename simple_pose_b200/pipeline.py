@@ -178,10 +178,7 @@ class HeatmapHotPath(object):
         with torch.cuda.device(dev):
             stream = _abi.stream_ptr(dev)
             if self.val_one_launch_supported(self.h, self.w, self.ksize, decoder):
-                if self.vws is None:
-                    nbytes = int(self._lib.sp_val_step_workspace_bytes(self.batch, self.k))
-                    self.vws = torch.zeros((nbytes + 7) // 8, dtype=torch.int64, device=dev)
-                ws = self.vws
+                ws = self._val_ws()
                 _abi.check_ws(self._lib.sp_val_step_f32(
                     joints.data_ptr(), pred.data_ptr(), _abi.ptr(trans_inv), self.blur_w.data_ptr(), mode,
                     self.weights.data_ptr(), self.loss.data_ptr(), self.acc.data_ptr(), self.rows.data_ptr(),
@@ -192,31 +189,36 @@ class HeatmapHotPath(object):
             self._val_composed(joints, pred, trans_inv, mode, stream)
         return self.loss, self.acc, self.rows
 
+    def _val_ws(self):
+        """``vws``: the workspace of ``val_step``, large enough for the one launch and for the composed loss kernel."""
+        if self.vws is None:
+            nbytes = max(int(self._lib.sp_val_step_workspace_bytes(self.batch, self.k)),
+                         int(self._lib.sp_mse_acc_workspace_bytes(self.batch, self.k)))
+            self.vws = torch.zeros((nbytes + 7) // 8, dtype=torch.int64, device=self.device)
+        return self.vws
+
     def _val_composed(self, joints, pred, trans_inv, mode, stream):
-        """``val_step`` as the stand-alone kernels: loss + HeatMapAcc argmaxes, decoder, HeatMapAcc epilogue, rows."""
-        ws = self.ws
-        if self.w % 4 == 0:           # the fused loss kernel with its argmaxes, forward only
+        """``val_step`` as the stand-alone kernels: loss + HeatMapAcc, decoder, rows."""
+        if self.w % 4 == 0:           # the fused loss kernel with its argmaxes, forward only, then the HeatMapAcc epilogue
+            ws = self.ws
             _abi.check_ws(self._lib.sp_encode_mse_fwd_bwd_f32(
                 joints.data_ptr(), pred.data_ptr(), None, None, self.weights.data_ptr(), self.loss.data_ptr(),
                 self.pred_xy.data_ptr(), self.label_xy.data_ptr(), ws.data_ptr(), ws.numel() * 8,
                 self.batch, self.k, self.h, self.w, self.sigma, 1.0, stream), self.device, stream, self)
-        else:                         # encode, forward loss, and the argmaxes of the masked maps as HeatMapAcc takes them
+            _abi.check(self._lib.sp_heatmap_acc_f32(self.pred_xy.data_ptr(), self.label_xy.data_ptr(), self.acc.data_ptr(),
+                                                    self.batch, self.k, self.h, self.w, 0.5, 10.0, stream))
+        else:                         # encode, then the forward loss with HeatMapAcc of the masked maps in the same pass
             self.encode(joints)
-            _abi.check_ws(self._lib.sp_mse_fwd_bwd_f32(pred.data_ptr(), self.targets.data_ptr(), self.weights.data_ptr(),
-                                                       None, self.loss.data_ptr(), ws.data_ptr(), ws.numel() * 8,
-                                                       self.batch, self.k, self.h * self.w, 1.0, 0, stream),
-                          self.device, stream, self)
-            mask = self.weights[..., None, None]
-            for src, dst in ((pred, self.pred_xy), (self.targets, self.label_xy)):
-                _abi.check(self._lib.sp_decode_f32(_abi.dense(src * mask, torch.float32).data_ptr(), None, None, None,
-                                                   None, dst.data_ptr(), self.maxval.data_ptr(), None, self.batch,
-                                                   self.k, self.h, self.w, 0, _abi.SP_DECODE_ARGMAX, stream))
+            ws = self._val_ws()
+            _abi.check_ws(self._lib.sp_mse_acc_fwd_bwd(
+                pred.data_ptr(), _abi.SP_DTYPE_F32, self.targets.data_ptr(), self.weights.data_ptr(), None,
+                self.loss.data_ptr(), self.acc.data_ptr(), self.pred_xy.data_ptr(), self.label_xy.data_ptr(),
+                ws.data_ptr(), ws.numel() * 8, self.batch, self.k, self.h, self.w, 1.0, None, 0.5, 10.0, 0, stream),
+                self.device, stream, self)
         _abi.check_ws(self._lib.sp_decode_ws_f32(pred.data_ptr(), None, None, _abi.ptr(trans_inv), self.blur_w.data_ptr(),
                                                  self.coords.data_ptr(), self.maxval.data_ptr(), None, self.batch, self.k,
                                                  self.h, self.w, self.ksize, mode, self.dws.data_ptr(),
                                                  self.dws.numel() * 8, stream), self.device, stream, self)
-        _abi.check(self._lib.sp_heatmap_acc_f32(self.pred_xy.data_ptr(), self.label_xy.data_ptr(), self.acc.data_ptr(),
-                                                self.batch, self.k, self.h, self.w, 0.5, 10.0, stream))
         _abi.check(self._lib.sp_person_rows_f32(self.coords.data_ptr(), self.maxval.data_ptr(), self.rows.data_ptr(),
                                                 self.batch, self.k, stream))
 

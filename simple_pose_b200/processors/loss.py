@@ -49,16 +49,23 @@ def _check_shapes(pred, target, mask):
 
 
 def mse_forward_backward(pred, target, mask, need_grad=True, grad_scale=1.0, skip_masked=False, need_loss=True,
-                         grad_scale_dev=None):
+                         grad_scale_dev=None, want_acc=False, distance_thresh=0.5, norm_frac=10., axes_out=None):
     """(loss 0-d float32 or None, grad like pred or None); everything on pred's CUDA device.
 
     ``pred`` may be float32, float16 or bfloat16 (``grad`` has the same dtype); ``grad_scale_dev`` is an
     optional 0-d float32 device tensor multiplied into the gradient on the device; ``need_loss=False``
-    is the backward-only call."""
+    is the backward-only call.
+
+    ``want_acc=True`` (forward calls only) also computes ``HeatMapAcc(distance_thresh, norm_frac)(pred.mul(mask),
+    target.mul(mask))`` in the same launch (``sp_mse_acc_fwd_bwd``) and returns ``(loss, grad, acc)``, acc a 0-d
+    float32 device tensor; ``axes_out`` = optional ``(pred_xy, label_xy)`` dense float32 [B, K, 2] tensors that
+    receive the two argmax coordinate tables."""
     dev = _abi.require_cuda(pred, target, mask, grad_scale_dev)
     b, k, hw = _check_shapes(pred, target, mask)
     if not need_loss and not need_grad:
         raise ValueError("nothing to compute")
+    if want_acc and (not need_loss or pred.dim() != 4):
+        raise ValueError("want_acc needs the forward call (need_loss=True) and pred [B, K, H, W]")
     p = _pred_tensor(pred)
     t = _abi.dense(target.detach(), torch.float32)
     m = _abi.dense(mask.detach(), torch.float32)
@@ -66,13 +73,29 @@ def mse_forward_backward(pred, target, mask, need_grad=True, grad_scale=1.0, ski
     loss = torch.empty((), dtype=torch.float32, device=dev) if need_loss else None
     grad = torch.empty_like(p) if need_grad else None
     stream = _abi.stream_ptr(dev)
-    ws = _workspace(dev, stream)
     flags = _abi.SP_MSE_SKIP_MASKED if skip_masked else 0
+    if not want_acc:
+        ws = _workspace(dev, stream)
+        with torch.cuda.device(dev):
+            _abi.check_ws(_abi.lib().sp_mse_fwd_bwd(p.data_ptr(), _DTYPE_CODE[p.dtype], t.data_ptr(), m.data_ptr(),
+                                                    _abi.ptr(grad), _abi.ptr(loss), ws.data_ptr(), ws.numel() * 8, b, k, hw,
+                                                    float(grad_scale), _abi.ptr(s), flags, stream), dev, stream)
+        return loss, grad
+    h, w = int(pred.shape[2]), int(pred.shape[3])
+    pxy, lxy = axes_out if axes_out is not None else (None, None)
+    for a in (pxy, lxy):
+        if a is not None and (a.device != dev or a.dtype != torch.float32 or tuple(a.shape) != (b, k, 2)
+                              or not a.is_contiguous()):
+            raise ValueError("axes_out must be two contiguous float32 [B, K, 2] tensors on %s" % dev)
+    acc = torch.empty((), dtype=torch.float32, device=dev)
+    ws = _abi.scratch(dev, stream, int(_abi.lib().sp_mse_acc_workspace_bytes(b, k)), "mse_acc")
     with torch.cuda.device(dev):
-        _abi.check_ws(_abi.lib().sp_mse_fwd_bwd(p.data_ptr(), _DTYPE_CODE[p.dtype], t.data_ptr(), m.data_ptr(), _abi.ptr(grad),
-                                                _abi.ptr(loss), ws.data_ptr(), ws.numel() * 8, b, k, hw, float(grad_scale),
-                                                _abi.ptr(s), flags, stream), dev, stream)
-    return loss, grad
+        _abi.check_ws(_abi.lib().sp_mse_acc_fwd_bwd(p.data_ptr(), _DTYPE_CODE[p.dtype], t.data_ptr(), m.data_ptr(),
+                                                    _abi.ptr(grad), loss.data_ptr(), acc.data_ptr(), _abi.ptr(pxy),
+                                                    _abi.ptr(lxy), ws.data_ptr(), ws.numel() * 8, b, k, h, w,
+                                                    float(grad_scale), _abi.ptr(s), float(distance_thresh),
+                                                    float(norm_frac), flags, stream), dev, stream)
+    return loss, grad, acc
 
 
 def _scale_saved_grad(ctx, grad, grad_out):
@@ -93,10 +116,16 @@ def _scale_saved_grad(ctx, grad, grad_out):
 
 class _MaskedMSE(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, pred, target, mask, skip_masked, defer_grad, grad_mode):
+    def forward(ctx, pred, target, mask, skip_masked, defer_grad, grad_mode, acc_args):
         need = grad_mode and pred.requires_grad        # grad_mode: torch.is_grad_enabled() at the call site (it is off in here)
         deferred = need and (defer_grad or pred.dtype in (torch.float16, torch.bfloat16))
-        loss, grad = mse_forward_backward(pred, target, mask, need_grad=need and not deferred, skip_masked=skip_masked)
+        if acc_args is None:
+            loss, grad = mse_forward_backward(pred, target, mask, need_grad=need and not deferred, skip_masked=skip_masked)
+        else:                                          # (holder, distance_thresh, norm_frac): HeatMapAcc in the same launch
+            holder, thresh, frac = acc_args
+            loss, grad, holder["acc"] = mse_forward_backward(pred, target, mask, need_grad=need and not deferred,
+                                                             skip_masked=skip_masked, want_acc=True,
+                                                             distance_thresh=thresh, norm_frac=frac)
         ctx.deferred, ctx.skip_masked, ctx.pred_dtype = deferred, skip_masked, pred.dtype
         if deferred:
             ctx.save_for_backward(pred, target, mask)
@@ -106,16 +135,17 @@ class _MaskedMSE(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, grad_out):
+        none = (None,) * 6
         if ctx.deferred:
             pred, target, mask = ctx.saved_tensors
             _, grad = mse_forward_backward(pred, target, mask, need_grad=True, need_loss=False, skip_masked=ctx.skip_masked,
                                            grad_scale_dev=grad_out.detach().to(pred.device).reshape(()))
-            return grad.to(ctx.pred_dtype).view_as(pred), None, None, None, None, None
+            return (grad.to(ctx.pred_dtype).view_as(pred),) + none
         (grad,) = ctx.saved_tensors
         if grad is None:
-            return None, None, None, None, None, None
+            return (None,) + none
         out = _scale_saved_grad(ctx, grad, grad_out)
-        return (out if ctx.pred_dtype == torch.float32 else out.to(ctx.pred_dtype)), None, None, None, None, None
+        return (out if ctx.pred_dtype == torch.float32 else out.to(ctx.pred_dtype),) + none
 
 
 class JointsMSELoss(torch.nn.Module):
@@ -125,15 +155,32 @@ class JointsMSELoss(torch.nn.Module):
     traffic; differs from the reference only when those maps hold NaN/Inf, which the
     reference would propagate into the loss). ``defer_grad=True`` computes the gradient in backward
     instead of forward also for float32 predictions (float16 / bfloat16 always do): nothing the size of
-    ``pred`` is kept between forward and backward and the node may be differentiated repeatedly."""
+    ``pred`` is kept between forward and backward and the node may be differentiated repeatedly.
 
-    def __init__(self, skip_masked=False, defer_grad=False):
+    ``with_acc=True`` returns ``(loss, acc)``: ``acc`` is ``HeatMapAcc(distance_thresh, norm_frac)(pred.mul(mask),
+    target.mul(mask))``, a 0-d float32 device tensor (no host sync), computed by the loss kernel while ``pred`` and
+    ``target`` stream by -- no masked copies, no argmax launches. ``pred`` must be [B, K, H, W]::
+
+        crit = JointsMSELoss(with_acc=True)
+        loss, acc = crit(predicts, targets, mask)     # == 0.5 * MSELoss(...) and HeatMapAcc()(predicts*mask, targets*mask)
+    """
+
+    def __init__(self, skip_masked=False, defer_grad=False, with_acc=False, distance_thresh=0.5, norm_frac=10.):
         super().__init__()
         self.skip_masked = bool(skip_masked)
         self.defer_grad = bool(defer_grad)
+        self.with_acc = bool(with_acc)
+        self.distance_thresh, self.norm_frac = distance_thresh, norm_frac
+        self.acc = None
 
     def forward(self, pred, target, mask):
-        return _MaskedMSE.apply(pred, target, mask, self.skip_masked, self.defer_grad, torch.is_grad_enabled())
+        if not self.with_acc:
+            return _MaskedMSE.apply(pred, target, mask, self.skip_masked, self.defer_grad, torch.is_grad_enabled(), None)
+        holder = {}
+        loss = _MaskedMSE.apply(pred, target, mask, self.skip_masked, self.defer_grad, torch.is_grad_enabled(),
+                                (holder, self.distance_thresh, self.norm_frac))
+        self.acc = holder["acc"]
+        return loss, self.acc
 
 
 def encode_mse_forward_backward(joints, pred, sigma=2.0, need_grad=True, want_targets=False, want_axes=False,
@@ -160,17 +207,18 @@ def encode_mse_forward_backward(joints, pred, sigma=2.0, need_grad=True, want_ta
     stream = _abi.stream_ptr(dev)
     ws = _workspace(dev, stream)
     if w % 4 != 0:
-        # shapes the fused kernel does not take: same results from the separate kernels
+        # shapes the fused kernel does not take: same results from the encoder and the loss kernel, which takes the
+        # HeatMapAcc argmaxes along when they are wanted
         from ..commons.transforms import encode_heat_maps
-        from ..metrics.pose_metrics import BasicKeyPointDecoder
         tg, wt = encode_heat_maps(j, sigma, (w, h))
-        loss, grad = mse_forward_backward(p, tg, wt, need_grad=need_grad, grad_scale=grad_scale, need_loss=need_loss,
-                                          grad_scale_dev=s)
-        out.update(loss=loss, grad=grad, weights=wt, targets=tg if want_targets else None)
         if want_axes:
-            m = wt[..., None, None]
-            out["pred_xy"] = BasicKeyPointDecoder.heat_map_to_axis(p.float() * m)[0]
-            out["label_xy"] = BasicKeyPointDecoder.heat_map_to_axis(tg * m)[0]
+            loss, grad, _ = mse_forward_backward(p, tg, wt, need_grad=need_grad, grad_scale=grad_scale, grad_scale_dev=s,
+                                                 want_acc=True, axes_out=(out["pred_xy"], out["label_xy"]))
+            loss = loss if need_loss else None
+        else:
+            loss, grad = mse_forward_backward(p, tg, wt, need_grad=need_grad, grad_scale=grad_scale, need_loss=need_loss,
+                                              grad_scale_dev=s)
+        out.update(loss=loss, grad=grad, weights=wt, targets=tg if want_targets else None)
         return out
     with torch.cuda.device(dev):
         _abi.check_ws(_abi.lib().sp_encode_mse_fwd_bwd(
