@@ -14,7 +14,8 @@
 // 16-byte global stores and re-arms the slot at once. Measured on B200 (scratch/stream_bench.cu):
 // for a 2-reads-1-write stream ~50-100 KB in flight per SM in few, large requests beats both the
 // classic "many threads, one float4 each" loop (-8 %) and deeper rings (HBM read/write turnarounds).
-// Fallback (mse_fwd_bwd_kernel): any shape / alignment, and the SKIP_MASKED variant.
+// Plain-load kernel (mse_plain_kernel, every dtype of pred): float16 / bfloat16 pred, backward-only calls, a
+// device-side upstream gradient, the SKIP_MASKED variant, any shape / alignment, and SP_LOSS_FORCE_LDG.
 //
 // The sum of squares is accumulated per thread in float32 over a few elements, then in float64;
 // block partials go to the caller's workspace and the last block to finish adds them in a fixed
@@ -48,14 +49,6 @@ namespace {
 
 using namespace sp_reduce;
 constexpr int kThreads = 256;
-
-__device__ __forceinline__ float4 ldg_stream(const float4* p) {
-    float4 r;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];"
-                 : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w)
-                 : "l"(p));
-    return r;
-}
 
 __device__ __forceinline__ float sq_err_and_grad(float p, float t, float m, float norm, float half_scale, float& g) {
     const float d = __fsub_rn(__fmul_rn(m, p), __fmul_rn(m, t));
@@ -132,103 +125,26 @@ __device__ __forceinline__ void acc_epilogue(const AccOut& A, int* counters) {
     sp_trn::heatmap_acc_block<true>(A.pred_xy, A.label_xy, A.acc, A.B, A.K, A.norm_x, A.norm_y, A.thresh, counters);
 }
 
-template <bool VEC4, bool WRITE_GRAD, bool ACC>
-__global__ void __launch_bounds__(kThreads)
-mse_fwd_bwd_kernel(const float* __restrict__ pred, const float* __restrict__ target,
-                   const float* __restrict__ mask, float* __restrict__ grad, float* __restrict__ loss,
-                   MseWorkspace* __restrict__ ws, int nmaps, int hw, float norm, float half_scale,
-                   double inv_count, int skip_masked, const AccOut A) {
-    double block_sum = 0.0;
-    sp::grid_dep_wait();
-    const int lane = threadIdx.x & 31;
-
-    for (int m = blockIdx.x; m < nmaps; m += gridDim.x) {
-        const float mk = __ldg(mask + m);
-        const size_t base = (size_t)m * hw;
-        float acc = 0.f;
-        const bool track = ACC && mk != 0.f;      // a masked-out map's products are 0 or NaN: (0, 0) either way
-        if (skip_masked && mk == 0.f) {
-            if (WRITE_GRAD) {
-                if (VEC4) {
-                    float4* g4 = reinterpret_cast<float4*>(grad + base);
-                    for (int q = threadIdx.x; q < (hw >> 2); q += kThreads) g4[q] = make_float4(0.f, 0.f, 0.f, 0.f);
-                } else {
-                    for (int i = threadIdx.x; i < hw; i += kThreads) grad[base + i] = 0.f;
-                }
-            }
-            continue;
-        }
-        if (VEC4) {
-            const float4* p4 = reinterpret_cast<const float4*>(pred + base);
-            const float4* t4 = reinterpret_cast<const float4*>(target + base);
-            float4* g4 = reinterpret_cast<float4*>(grad + base);
-            const int nq = hw >> 2;
-            sp_trn::QuadBest bp, bt;
-            if (ACC) { bp.init(); bt.init(); }
-#pragma unroll 4
-            for (int q = threadIdx.x; q < nq; q += kThreads) {
-                const float4 p = ldg_stream(p4 + q);
-                const float4 t = ldg_stream(t4 + q);
-                float4 g;
-                float d;
-                d = sq_err_and_grad(p.x, t.x, mk, norm, half_scale, g.x); acc = fmaf(d, d, acc);
-                d = sq_err_and_grad(p.y, t.y, mk, norm, half_scale, g.y); acc = fmaf(d, d, acc);
-                d = sq_err_and_grad(p.z, t.z, mk, norm, half_scale, g.z); acc = fmaf(d, d, acc);
-                d = sq_err_and_grad(p.w, t.w, mk, norm, half_scale, g.w); acc = fmaf(d, d, acc);
-                if (WRITE_GRAD) g4[q] = g;
-                if (ACC && track) {
-                    bp.push(__fmul_rn(mk, p.x), __fmul_rn(mk, p.y), __fmul_rn(mk, p.z), __fmul_rn(mk, p.w), q);
-                    bt.push(__fmul_rn(mk, t.x), __fmul_rn(mk, t.y), __fmul_rn(mk, t.z), __fmul_rn(mk, t.w), q);
-                }
-            }
-            if (ACC && track) {
-                merge_quads(bp, pred + base, mk, hw, 0, lane, A.keys + 2 * (size_t)m);
-                merge_quads(bt, target + base, mk, hw, 0, lane, A.keys + 2 * (size_t)m + 1);
-            }
-        } else {
-            float bvp = -CUDART_INF_F, bvt = -CUDART_INF_F;
-            int bip = 0x7fffffff, bit = 0x7fffffff;
-            for (int i = threadIdx.x; i < hw; i += kThreads) {
-                float g;
-                const float pv = pred[base + i], tv = target[base + i];
-                const float d = sq_err_and_grad(pv, tv, mk, norm, half_scale, g);
-                acc = fmaf(d, d, acc);
-                if (WRITE_GRAD) grad[base + i] = g;
-                if (ACC && track) {
-                    const float mp = __fmul_rn(mk, pv), mt = __fmul_rn(mk, tv);
-                    if (sp::better(mp, i, bvp, bip)) { bvp = mp; bip = i; }
-                    if (sp::better(mt, i, bvt, bit)) { bvt = mt; bit = i; }
-                }
-            }
-            if (ACC && track) {
-                merge_scalar(bvp, bip, lane, A.keys + 2 * (size_t)m);
-                merge_scalar(bvt, bit, lane, A.keys + 2 * (size_t)m + 1);
-            }
-        }
-        block_sum += (double)acc;
-    }
-
-    const bool last = finish_loss<kThreads>(block_sum, ws, loss, inv_count);
-    if constexpr (ACC) {
-        extern __shared__ int acc_counters[];     // 2K ints
-        if (last) acc_epilogue(A, acc_counters);
-    }
-}
-
-// Mixed-precision variant (torch.cuda.amp, processors/dp_pose_hrnet_solver.py:111-120): `pred` arrives in the
-// autocast dtype PT (float16 / bfloat16; float32 also instantiated) and the gradient leaves in PT. The
-// arithmetic is what autocast runs: `pred.mul(mask)` promotes to float32, mse_loss is on autocast's float32
-// list, the backward of the promoted product casts d loss / d pred to PT once, AFTER the upstream gradient
-// (GradScaler's scale, read here from device memory so that no host sync is needed) has been applied in
-// float32 -- which is the whole point of loss scaling for float16. Eight elements per thread per step:
-// one 16-byte load of pred (8 x PT; 2 x float4 for float32), two of target, one 16-byte grad store.
+// The plain-load kernel: one CTA per map at a time, grid-stride over the maps. It serves every call the ring kernel does
+// not take: float16 / bfloat16 `pred`, backward-only calls, a device-side upstream gradient, SKIP_MASKED, any shape and
+// alignment. `pred` arrives in PT (float32, or the autocast dtype float16 / bfloat16 of processors/dp_pose_hrnet_solver.py:
+// 111-120) and the gradient leaves in PT. The arithmetic is what autocast runs: `pred.mul(mask)` promotes to float32,
+// mse_loss is on autocast's float32 list, the backward of the promoted product casts d loss / d pred to PT once, AFTER
+// the upstream gradient (GradScaler's scale, read here from device memory so that no host sync is needed) has been
+// applied in float32 -- which is the whole point of loss scaling for float16.
+// VEC (HW % E == 0, pred / target / grad 16-byte aligned): a step is one 16-byte load of pred, E = 16 / sizeof(PT)
+// elements (4 floats or 8 halves), E / 4 float4 loads of target and one 16-byte grad store.
 // loss == nullptr: backward only (no reduction); grad == nullptr: forward only. ACC only with loss != nullptr.
-template <typename PT, bool VEC8, bool ACC>
+template <typename PT, bool VEC, bool ACC>
 __global__ void __launch_bounds__(kThreads)
-mse_mixed_kernel(const PT* __restrict__ pred, const float* __restrict__ target, const float* __restrict__ mask,
+mse_plain_kernel(const PT* __restrict__ pred, const float* __restrict__ target, const float* __restrict__ mask,
                  PT* __restrict__ grad, float* __restrict__ loss, MseWorkspace* __restrict__ ws, int nmaps, int hw,
                  float norm, float half_scale_host, const float* __restrict__ scale_dev, double inv_count, int skip_masked,
                  const AccOut A) {
+    constexpr int E = 16 / sizeof(PT);
+    constexpr int kLogE = E == 4 ? 2 : 3;
+    constexpr int Q = E / 4;                      // quads per step
+    constexpr int kUnroll = Q == 1 ? 4 : 2;
     double block_sum = 0.0;
     sp::grid_dep_wait();
     const float half_scale = scale_dev ? __fmul_rn(half_scale_host, __ldg(scale_dev)) : half_scale_host;
@@ -239,36 +155,47 @@ mse_mixed_kernel(const PT* __restrict__ pred, const float* __restrict__ target, 
         const float mk = __ldg(mask + m);
         const size_t base = (size_t)m * hw;
         float acc = 0.f;
-        const bool track = ACC && mk != 0.f;
+        const bool track = ACC && mk != 0.f;      // a masked-out map's products are 0 or NaN: (0, 0) either way
         if (skip_masked && mk == 0.f) {
-            if (write_grad)
-                for (int i = threadIdx.x; i < hw; i += kThreads) grad[base + i] = sp_lowp::from_float<PT>(0.f);
+            if (write_grad) {
+                if (VEC) {
+                    uint4* g16 = reinterpret_cast<uint4*>(grad + base);
+                    for (int o = threadIdx.x; o < (hw >> kLogE); o += kThreads) g16[o] = make_uint4(0u, 0u, 0u, 0u);
+                } else {
+                    for (int i = threadIdx.x; i < hw; i += kThreads) grad[base + i] = sp_lowp::from_float<PT>(0.f);
+                }
+            }
             continue;
         }
-        if (VEC8) {
-            const int n8 = hw >> 3;
+        if (VEC) {
+            const float4* t4 = reinterpret_cast<const float4*>(target + base);
+            const int nv = hw >> kLogE;
             sp_trn::QuadBest bp, bt;
             if (ACC) { bp.init(); bt.init(); }
-#pragma unroll 2
-            for (int o = threadIdx.x; o < n8; o += kThreads) {
-                float p[8], g[8];
-                sp_lowp::load8(pred + base + 8 * (size_t)o, p);
-                const float4 t0 = ldg_stream(reinterpret_cast<const float4*>(target + base) + 2 * o);
-                const float4 t1 = ldg_stream(reinterpret_cast<const float4*>(target + base) + 2 * o + 1);
-                const float t[8] = {t0.x, t0.y, t0.z, t0.w, t1.x, t1.y, t1.z, t1.w};
+#pragma unroll kUnroll
+            for (int o = threadIdx.x; o < nv; o += kThreads) {
+                float p[E], t[E], g[E];
+                sp_lowp::load_group(pred + base + E * (size_t)o, p);
 #pragma unroll
-                for (int e = 0; e < 8; ++e) {
+                for (int h = 0; h < Q; ++h) {
+                    const float4 v = sp_trn::ldg_stream4(t4 + Q * o + h);
+                    t[4 * h] = v.x; t[4 * h + 1] = v.y; t[4 * h + 2] = v.z; t[4 * h + 3] = v.w;
+                }
+#pragma unroll
+                for (int e = 0; e < E; ++e) {
                     const float d = sq_err_and_grad(p[e], t[e], mk, norm, half_scale, g[e]);
                     acc = fmaf(d, d, acc);
                 }
-                if (write_grad) sp_lowp::store8(grad + base + 8 * (size_t)o, g);
-                if (ACC && track) {       // float(p) * m: the float32 promotion autocast's pred.mul(mask) computes
+                if (write_grad) sp_lowp::store_group(grad + base + E * (size_t)o, g);
+                // float(p) * m: the float32 promotion autocast's pred.mul(mask) computes. Pushed for untracked maps too
+                // (their state is never merged): a branch on `track` made the ACC calls 0.6-7 % slower.
+                if (ACC) {
 #pragma unroll
-                    for (int h = 0; h < 2; ++h) {
+                    for (int h = 0; h < Q; ++h) {
                         bp.push(__fmul_rn(mk, p[4 * h]), __fmul_rn(mk, p[4 * h + 1]), __fmul_rn(mk, p[4 * h + 2]),
-                                __fmul_rn(mk, p[4 * h + 3]), 2 * o + h);
+                                __fmul_rn(mk, p[4 * h + 3]), Q * o + h);
                         bt.push(__fmul_rn(mk, t[4 * h]), __fmul_rn(mk, t[4 * h + 1]), __fmul_rn(mk, t[4 * h + 2]),
-                                __fmul_rn(mk, t[4 * h + 3]), 2 * o + h);
+                                __fmul_rn(mk, t[4 * h + 3]), Q * o + h);
                     }
                 }
             }
@@ -301,7 +228,7 @@ mse_mixed_kernel(const PT* __restrict__ pred, const float* __restrict__ target, 
     if (loss != nullptr) {
         const bool last = finish_loss<kThreads>(block_sum, ws, loss, inv_count);
         if constexpr (ACC) {
-            extern __shared__ int acc_counters[];
+            extern __shared__ int acc_counters[];     // 2K ints
             if (last) acc_epilogue(A, acc_counters);
         }
     }
@@ -430,21 +357,30 @@ scale_inplace_kernel(float* __restrict__ data, long long n, const float* __restr
 
 extern "C" size_t sp_mse_workspace_bytes(void) { return sizeof(MseWorkspace); }
 
-// sp_mse_fwd_bwd_f32 after its argument checks; A.acc != nullptr: with the HeatMapAcc argmaxes and epilogue (ACC)
-static int mse_f32(const float* pred, const float* target, const float* mask, float* grad, float* loss, MseWorkspace* ws,
-                   int B, int K, int HW, float grad_scale, int flags, cudaStream_t st, const AccOut& A) {
+template <typename PT>
+static auto plain_kernel(bool vec, bool acc) {
+    return vec ? (acc ? mse_plain_kernel<PT, true, true> : mse_plain_kernel<PT, true, false>)
+               : (acc ? mse_plain_kernel<PT, false, true> : mse_plain_kernel<PT, false, false>);
+}
+
+// Every entry point after its argument checks. A.acc != nullptr: with the HeatMapAcc argmaxes and epilogue (ACC).
+static int mse_launch(const void* pred, int pred_dtype, const float* target, const float* mask, void* grad, float* loss,
+                      MseWorkspace* ws, int B, int K, int HW, float grad_scale, const float* grad_scale_dev, int flags,
+                      cudaStream_t st, const AccOut& A) {
     const int nmaps = B * K;
     const double count = (double)B * (double)K * (double)HW;
     const float norm = (float)(2.0 / count);       // ATen: norm = 2 / numel, applied in float32
     const float half_scale = 0.5f * grad_scale;    // the 0.5 of the loss expression times upstream grad
-    const bool vec4 = (HW % 4 == 0) && sp_aligned16(pred) && sp_aligned16(target) && (!grad || sp_aligned16(grad));
+    const int per16 = pred_dtype == SP_DTYPE_F32 ? 4 : 8;           // elements of pred in 16 bytes
+    const bool vec = (HW % per16 == 0) && sp_aligned16(pred) && sp_aligned16(target) && (!grad || sp_aligned16(grad));
     const int skip = (flags & SP_MSE_SKIP_MASKED) ? 1 : 0;
     const bool acc = A.acc != nullptr;
-    const size_t counter_bytes = (size_t)2 * K * sizeof(int);      // HeatMapAcc epilogue of the last block
+    const size_t counter_bytes = acc ? (size_t)2 * K * sizeof(int) : 0;      // HeatMapAcc epilogue of the last block
 
-    // ring kernel: needs 16-byte rows and a chunk size (in quads) that divides the map
+    // ring kernel: float32 forward calls with the upstream gradient on the host; needs 16-byte rows and a chunk size
+    // (in quads) that divides the map
     const SpTuning& tune = sp_tuning();
-    if (vec4 && !skip && sp_knob(tune.loss_force_ldg, 0) == 0) {
+    if (pred_dtype == SP_DTYPE_F32 && loss && !grad_scale_dev && vec && !skip && sp_knob(tune.loss_force_ldg, 0) == 0) {
         const int nq = HW >> 2;
         int want = sp_knob(tune.loss_chunk_quads, 192);           // 3 KB per stream
         if (want < 8) want = 8;
@@ -452,7 +388,7 @@ static int mse_f32(const float* pred, const float* target, const float* mask, fl
         int chunk_quads = 0;
         for (int d = want < nq ? want : nq; d >= 8; --d)
             if (nq % d == 0) { chunk_quads = d; break; }
-        if (chunk_quads * 2 >= (want < nq ? want : nq)) {            // else: awkward map size, use the fallback
+        if (chunk_quads * 2 >= (want < nq ? want : nq)) {            // else: awkward map size, use the plain kernel
             int ring = sp_knob(tune.loss_ring, 3);
             if (ring < 1) ring = 1;
             if (ring > 8) ring = 8;
@@ -481,18 +417,14 @@ static int mse_f32(const float* pred, const float* target, const float* mask, fl
     int grid = sp_sm_count() * 8;
     if (grid > nmaps) grid = nmaps;
     if (grid > kMaxPartials) grid = kMaxPartials;
-#define SP_LAUNCH_MSE(V, G, AC) \
-    SP_CUDA(sp_launch(mse_fwd_bwd_kernel<V, G, AC>, dim3(grid), dim3(kThreads), AC ? counter_bytes : 0, st, pred, target, mask, grad, \
-                      loss, ws, nmaps, HW, norm, half_scale, 1.0 / count, skip, A))
-    if (acc) {
-        if (vec4) { if (grad) SP_LAUNCH_MSE(true, true, true); else SP_LAUNCH_MSE(true, false, true); }
-        else      { if (grad) SP_LAUNCH_MSE(false, true, true); else SP_LAUNCH_MSE(false, false, true); }
-    } else {
-        if (vec4) { if (grad) SP_LAUNCH_MSE(true, true, false); else SP_LAUNCH_MSE(true, false, false); }
-        else      { if (grad) SP_LAUNCH_MSE(false, true, false); else SP_LAUNCH_MSE(false, false, false); }
-    }
-#undef SP_LAUNCH_MSE
-    return 0;
+    auto launch = [&](auto kernel) {
+        SP_CUDA(sp_launch(kernel, dim3(grid), dim3(kThreads), counter_bytes, st, pred, target, mask, grad, loss, ws, nmaps, HW,
+                          norm, half_scale, grad_scale_dev, 1.0 / count, skip, A));
+        return 0;
+    };
+    if (pred_dtype == SP_DTYPE_F16) return launch(plain_kernel<__half>(vec, acc));
+    if (pred_dtype == SP_DTYPE_BF16) return launch(plain_kernel<__nv_bfloat16>(vec, acc));
+    return launch(plain_kernel<float>(vec, acc));
 }
 
 extern "C" int sp_mse_fwd_bwd_f32(const float* pred, const float* target, const float* mask,
@@ -503,42 +435,8 @@ extern "C" int sp_mse_fwd_bwd_f32(const float* pred, const float* target, const 
     SP_RETURN_IF((long long)B * K > 0x7fffffffLL, SP_ERR_UNSUPPORTED);
     SP_RETURN_IF(workspace_bytes < sizeof(MseWorkspace), SP_ERR_WORKSPACE);
     SP_RETURN_IF(!sp_aligned16(workspace), SP_ERR_BAD_ALIGNMENT);
-    return mse_f32(pred, target, mask, grad, loss, static_cast<MseWorkspace*>(workspace), B, K, HW, grad_scale, flags,
-                   static_cast<cudaStream_t>(stream), AccOut{});
-}
-
-template <typename PT>
-static int launch_mixed(const void* pred, const float* target, const float* mask, void* grad, float* loss, MseWorkspace* ws,
-                        int nmaps, int HW, float norm, float half_scale, const float* scale_dev, double inv_count, int skip,
-                        cudaStream_t st, const AccOut& A) {
-    const bool vec8 = (HW % 8 == 0) && sp_aligned16(pred) && sp_aligned16(target) && (!grad || sp_aligned16(grad));
-    int grid = sp_sm_count() * 8;
-    if (grid > nmaps) grid = nmaps;
-    if (grid > kMaxPartials) grid = kMaxPartials;
-    const PT* p = static_cast<const PT*>(pred);
-    PT* g = static_cast<PT*>(grad);
-    const size_t counter_bytes = A.acc ? (size_t)2 * A.K * sizeof(int) : 0;
-#define SP_LAUNCH_MIXED(V8, AC) \
-    SP_CUDA(sp_launch(mse_mixed_kernel<PT, V8, AC>, dim3(grid), dim3(kThreads), counter_bytes, st, p, target, mask, g, loss, ws, \
-                      nmaps, HW, norm, half_scale, scale_dev, inv_count, skip, A))
-    if (A.acc) { if (vec8) SP_LAUNCH_MIXED(true, true); else SP_LAUNCH_MIXED(false, true); }
-    else       { if (vec8) SP_LAUNCH_MIXED(true, false); else SP_LAUNCH_MIXED(false, false); }
-#undef SP_LAUNCH_MIXED
-    return 0;
-}
-
-static int mixed_dispatch(const void* pred, int pred_dtype, const float* target, const float* mask, void* grad, float* loss,
-                          MseWorkspace* ws, int B, int K, int HW, float grad_scale, const float* grad_scale_dev, int flags,
-                          cudaStream_t st, const AccOut& A) {
-    const double count = (double)B * (double)K * (double)HW;
-    const float norm = (float)(2.0 / count);
-    const float half_scale = 0.5f * grad_scale;
-    const int skip = (flags & SP_MSE_SKIP_MASKED) ? 1 : 0;
-    if (pred_dtype == SP_DTYPE_F16)
-        return launch_mixed<__half>(pred, target, mask, grad, loss, ws, B * K, HW, norm, half_scale, grad_scale_dev, 1.0 / count, skip, st, A);
-    if (pred_dtype == SP_DTYPE_BF16)
-        return launch_mixed<__nv_bfloat16>(pred, target, mask, grad, loss, ws, B * K, HW, norm, half_scale, grad_scale_dev, 1.0 / count, skip, st, A);
-    return launch_mixed<float>(pred, target, mask, grad, loss, ws, B * K, HW, norm, half_scale, grad_scale_dev, 1.0 / count, skip, st, A);
+    return mse_launch(pred, SP_DTYPE_F32, target, mask, grad, loss, static_cast<MseWorkspace*>(workspace), B, K, HW, grad_scale,
+                      nullptr, flags, static_cast<cudaStream_t>(stream), AccOut{});
 }
 
 extern "C" int sp_mse_fwd_bwd(const void* pred, int pred_dtype, const float* target, const float* mask,
@@ -546,19 +444,15 @@ extern "C" int sp_mse_fwd_bwd(const void* pred, int pred_dtype, const float* tar
                               int B, int K, int HW, float grad_scale, const float* grad_scale_dev, int flags, void* stream) {
     SP_RETURN_IF(pred_dtype != SP_DTYPE_F32 && pred_dtype != SP_DTYPE_F16 && pred_dtype != SP_DTYPE_BF16, SP_ERR_BAD_ARGUMENT);
     SP_RETURN_IF(!loss && !grad, SP_ERR_BAD_ARGUMENT);
-    if (pred_dtype == SP_DTYPE_F32 && loss && !grad_scale_dev)        // the float32 fast path (TMA ring kernel)
-        return sp_mse_fwd_bwd_f32(static_cast<const float*>(pred), target, mask, static_cast<float*>(grad), loss, workspace,
-                                  workspace_bytes, B, K, HW, grad_scale, flags, stream);
-    SP_RETURN_IF(!pred || !target || !mask, SP_ERR_BAD_ARGUMENT);
+    SP_RETURN_IF(!pred || !target || !mask || (loss && !workspace), SP_ERR_BAD_ARGUMENT);
     SP_RETURN_IF(B <= 0 || K <= 0 || HW <= 0, SP_ERR_BAD_ARGUMENT);
     SP_RETURN_IF((long long)B * K > 0x7fffffffLL, SP_ERR_UNSUPPORTED);
     if (loss) {
-        SP_RETURN_IF(!workspace, SP_ERR_BAD_ARGUMENT);
         SP_RETURN_IF(workspace_bytes < sizeof(MseWorkspace), SP_ERR_WORKSPACE);
         SP_RETURN_IF(!sp_aligned16(workspace), SP_ERR_BAD_ALIGNMENT);
     }
-    return mixed_dispatch(pred, pred_dtype, target, mask, grad, loss, static_cast<MseWorkspace*>(workspace), B, K, HW, grad_scale,
-                          grad_scale_dev, flags, static_cast<cudaStream_t>(stream), AccOut{});
+    return mse_launch(pred, pred_dtype, target, mask, grad, loss, static_cast<MseWorkspace*>(workspace), B, K, HW, grad_scale,
+                      grad_scale_dev, flags, static_cast<cudaStream_t>(stream), AccOut{});
 }
 
 // workspace of sp_mse_acc_fwd_bwd: the reduction workspace, the argmax keys (16 bytes per map), room for the axes (16 bytes
@@ -595,12 +489,8 @@ extern "C" int sp_mse_acc_fwd_bwd(const void* pred, int pred_dtype, const float*
     A.norm_x = (float)W / norm_frac;           // norm = tensor([W, H], float32) / norm_frac, as sp_heatmap_acc_f32
     A.norm_y = (float)H / norm_frac;
     A.thresh = distance_thresh;
-    MseWorkspace* ws = static_cast<MseWorkspace*>(workspace);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (pred_dtype == SP_DTYPE_F32 && !grad_scale_dev)             // the float32 fast path, as sp_mse_fwd_bwd
-        return mse_f32(static_cast<const float*>(pred), target, mask, static_cast<float*>(grad), loss, ws, B, K, H * W, grad_scale,
-                       flags, st, A);
-    return mixed_dispatch(pred, pred_dtype, target, mask, grad, loss, ws, B, K, H * W, grad_scale, grad_scale_dev, flags, st, A);
+    return mse_launch(pred, pred_dtype, target, mask, grad, loss, static_cast<MseWorkspace*>(workspace), B, K, H * W, grad_scale,
+                      grad_scale_dev, flags, static_cast<cudaStream_t>(stream), A);
 }
 
 extern "C" int sp_scale_inplace_f32(float* data, long long n, const float* scale_dev, void* stream) {

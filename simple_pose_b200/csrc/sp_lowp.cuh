@@ -1,6 +1,6 @@
-// float16 / bfloat16 / float32 element access for the mixed-precision (autocast) variants of the loss
-// kernels: eight elements per 16-byte (half types) or 2 x 16-byte (float) access, conversions with
-// round-to-nearest-even exactly as torch's .to(dtype).
+// float16 / bfloat16 / float32 element access for the loss kernels that read `pred` in its own dtype: one
+// 16-byte group (4 floats or 8 halves) per load / store, conversions with round-to-nearest-even exactly as
+// torch's .to(dtype).
 #pragma once
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
@@ -23,13 +23,12 @@ __device__ __forceinline__ uint4 ldg_stream16(const void* p) {
     return r;
 }
 
-// 8 consecutive elements starting at a 16-byte aligned address -> float[8]
-__device__ __forceinline__ void load8(const float* p, float (&out)[8]) {
-    const uint4 a = ldg_stream16(p), b = ldg_stream16(p + 4);
+// the 16 bytes at a 16-byte aligned address -> float[16 / sizeof(T)]
+__device__ __forceinline__ void load_group(const float* p, float (&out)[4]) {
+    const uint4 a = ldg_stream16(p);
     out[0] = __uint_as_float(a.x); out[1] = __uint_as_float(a.y); out[2] = __uint_as_float(a.z); out[3] = __uint_as_float(a.w);
-    out[4] = __uint_as_float(b.x); out[5] = __uint_as_float(b.y); out[6] = __uint_as_float(b.z); out[7] = __uint_as_float(b.w);
 }
-__device__ __forceinline__ void load8(const __half* p, float (&out)[8]) {
+__device__ __forceinline__ void load_group(const __half* p, float (&out)[8]) {
     const uint4 a = ldg_stream16(p);
     const unsigned w[4] = {a.x, a.y, a.z, a.w};
 #pragma unroll
@@ -40,7 +39,7 @@ __device__ __forceinline__ void load8(const __half* p, float (&out)[8]) {
         out[2 * i + 1] = f.y;
     }
 }
-__device__ __forceinline__ void load8(const __nv_bfloat16* p, float (&out)[8]) {
+__device__ __forceinline__ void load_group(const __nv_bfloat16* p, float (&out)[8]) {
     const uint4 a = ldg_stream16(p);
     const unsigned w[4] = {a.x, a.y, a.z, a.w};
 #pragma unroll
@@ -50,11 +49,10 @@ __device__ __forceinline__ void load8(const __nv_bfloat16* p, float (&out)[8]) {
     }
 }
 
-__device__ __forceinline__ void store8(float* p, const float (&v)[8]) {
-    reinterpret_cast<float4*>(p)[0] = make_float4(v[0], v[1], v[2], v[3]);
-    reinterpret_cast<float4*>(p)[1] = make_float4(v[4], v[5], v[6], v[7]);
+__device__ __forceinline__ void store_group(float* p, const float (&v)[4]) {
+    *reinterpret_cast<float4*>(p) = make_float4(v[0], v[1], v[2], v[3]);
 }
-__device__ __forceinline__ void store8(__half* p, const float (&v)[8]) {
+__device__ __forceinline__ void store_group(__half* p, const float (&v)[8]) {
     uint4 r;
     unsigned* w = reinterpret_cast<unsigned*>(&r);
 #pragma unroll
@@ -64,7 +62,7 @@ __device__ __forceinline__ void store8(__half* p, const float (&v)[8]) {
     }
     *reinterpret_cast<uint4*>(p) = r;
 }
-__device__ __forceinline__ void store8(__nv_bfloat16* p, const float (&v)[8]) {
+__device__ __forceinline__ void store_group(__nv_bfloat16* p, const float (&v)[8]) {
     uint4 r;
     unsigned* w = reinterpret_cast<unsigned*>(&r);
 #pragma unroll

@@ -1037,10 +1037,11 @@ def test_fused_label_argmax_ties_and_outside_centres(api):
                                  {"SP_LOSS_WARPS": "32", "SP_LOSS_RING": "2", "SP_LOSS_CHUNK_QUADS": "96"},
                                  {"SP_LOSS_CHUNK_QUADS": "768", "SP_LOSS_RING": "8"},
                                  {"SP_LOSS_CHUNK_QUADS": "100"}, {"SP_NO_PDL": "1"}])
-@pytest.mark.parametrize("b,hw", [(40, (64, 48)), (3, (96, 72)), (9, (20, 12))])
+@pytest.mark.parametrize("b,hw", [(40, (64, 48)), (3, (96, 72)), (9, (20, 12)), (5, (10, 6))])
 def test_loss_kernel_variants_agree(api, env, b, hw):
-    """Every chunk/ring/warp layout of the TMA-ring loss kernel, the plain-load fallback and the
-    non-PDL launch give bit-identical gradients and the same loss (float64 partial order aside)."""
+    """Every chunk/ring/warp layout of the TMA-ring loss kernel, the plain-load kernel, the backward-only
+    call with a device-side scale and the non-PDL launch give bit-identical gradients and the same loss
+    (float64 partial order aside)."""
     h, w = hw
     tgt = synth.heatmaps(b, height=h, width=w, seed=11).to(DEV)
     msk = (torch.rand(b, 17, generator=torch.Generator().manual_seed(12)) > 0.25).float().to(DEV)
@@ -1049,6 +1050,8 @@ def test_loss_kernel_variants_agree(api, env, b, hw):
     base_loss, base_grad = api.loss.mse_forward_backward(pred, tgt, msk)
     fwd_only, none = api.loss.mse_forward_backward(pred, tgt, msk, need_grad=False)
     assert none is None and fwd_only.item() == base_loss.item()
+    _, bwd_only = api.loss.mse_forward_backward(pred, tgt, msk, need_loss=False, grad_scale_dev=torch.tensor(1.0, device=DEV))
+    assert torch.equal(bwd_only, base_grad)
     os.environ.update(env)
     api.abi.reload_tuning()
     try:
