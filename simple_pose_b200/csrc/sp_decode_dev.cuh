@@ -1,11 +1,15 @@
-// Device-side building blocks of the heatmap decoders (argmax with torch.max semantics, the 13-point blur +
-// Taylor refinement, the epilogue with the affine back-projection), shared by the decode kernels
-// (sp_decode.cu) and the one-launch step kernel (sp_step.cu). See sp_decode.cu for the design notes.
+// Device-side building blocks of the heatmap decoders (the vector argmax scan of a staged map, the 13-point blur +
+// Taylor refinement, the epilogue with the affine back-projection), shared by the decode kernels (sp_decode.cu) and
+// the one-launch step kernel (sp_step.cu). The argmax rule itself is in sp_argmax.cuh. See sp_decode.cu for the
+// design notes.
 #pragma once
 #include "sp_common.cuh"
+#include "sp_argmax.cuh"
 #include <math_constants.h>
 
 namespace sp_dec {
+
+using namespace sp_arg;
 
 constexpr int kMaxKsize = 15;
 constexpr int kStencil = 13;
@@ -33,45 +37,12 @@ struct DecodeArgs {
 enum { S_C = 0, S_XP1, S_XM1, S_YP1, S_YM1, S_XP2, S_XM2, S_YP2, S_YM2, S_PP, S_MP, S_PM, S_MM };
 // S_PP = (y+1,x+1), S_MP = (y-1,x+1), S_PM = (y+1,x-1), S_MM = (y-1,x-1)
 
-struct Peak {
-    float value;
-    int index;
-};
-
-// ---------------------------------------------------------------------------------------------
-// warp-wide min/max in one instruction (redux.sync.*.f32, sm_100a; SASS CREDUX)
-// ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ float warp_max_f32(float v) {
-    float r;
-    asm volatile("redux.sync.max.f32 %0, %1, 0xffffffff;" : "=f"(r) : "f"(v));
-    return r;
-}
+// warp-wide min in one instruction (redux.sync.min.f32, sm_100a; SASS CREDUX)
 __device__ __forceinline__ float warp_min_f32(float v) {
     float r;
     asm volatile("redux.sync.min.f32 %0, %1, 0xffffffff;" : "=f"(r) : "f"(v));
     return r;
 }
-
-// ---------------------------------------------------------------------------------------------
-// argmax of a map that is resident in shared (fast path) or global (generic path) memory
-// ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ Peak warp_best(float v, int i) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const float ov = __shfl_xor_sync(SP_FULL, v, o);
-        const int oi = __shfl_xor_sync(SP_FULL, i, o);
-        if (sp::better(ov, oi, v, i)) { v = ov; i = oi; }
-    }
-    Peak p;
-    p.value = v;
-    p.index = i;
-    return p;
-}
-
-struct DirectView {
-    const float* p;
-    __device__ __forceinline__ float at(int i) const { return p[i]; }
-};
 
 // 0.5*(a[y,x] + b[y,W-1-x]) evaluated on the fly (generic path of the flip test)
 struct FlipAvgView {
@@ -84,19 +55,9 @@ struct FlipAvgView {
     }
 };
 
-// exact scalar scan (torch.max semantics incl. NaN); used by the generic path and as the
-// fallback of the vector scan
-template <typename View>
-__device__ __noinline__ Peak argmax_exact(const View map, int hw, int lane) {
-    float bv = -CUDART_INF_F;
-    int bi = 0x7fffffff;
-    for (int i = lane; i < hw; i += 32) {
-        const float v = map.at(i);
-        if (sp::better(v, i, bv, bi)) { bv = v; bi = i; }
-    }
-    return warp_best(bv, bi);
-}
-
+// ---------------------------------------------------------------------------------------------
+// argmax of a map that is resident in shared memory (the generic path runs argmax_exact on the map in place)
+// ---------------------------------------------------------------------------------------------
 // Vector scan over a shared-memory map (hw % 4 == 0). If FLIP, first folds the mirrored partner
 // map into `a` in place (W % 4 == 0 so the mirror of an aligned quad is an aligned quad).
 template <bool FLIP>
@@ -139,8 +100,9 @@ __device__ __forceinline__ Peak argmax_smem(float* a, const float* b, int hw, in
         return argmax_exact(view, hw, lane);
     }
     // all values finite: warp max in one CREDUX, then the smallest quad index that attains it
-    const float gmax = warp_max_f32(best);
-    const unsigned gq = __reduce_min_sync(SP_FULL, (best == gmax) ? (unsigned)bq : 0x7fffffffu);
+    const Peak g = warp_first_max(best, (unsigned)bq);
+    const float gmax = g.value;
+    const unsigned gq = (unsigned)g.index;
     const float4 w = a4[gq];            // broadcast read; first element of the quad equal to the max
     const int sub = (w.x == gmax) ? 0 : (w.y == gmax) ? 1 : (w.z == gmax) ? 2 : 3;
     Peak p;

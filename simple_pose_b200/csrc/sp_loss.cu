@@ -29,11 +29,12 @@
 // last block runs the HeatMapAcc epilogue. A map may be split over lanes, warps and blocks (the ring kernel cuts its
 // ranges by chunk count), so every partial argmax becomes a 64-bit key whose unsigned order is sp::better's and the
 // partials meet in one atomicMax per (map, warp that scanned part of it) -- the result cannot depend on the split.
+// The running argmax, its warp merge, the exact scan and the epilogue are those of sp_argmax.cuh, which the decode,
+// fused training and step kernels use as well.
 #include "sp_common.cuh"
 #include "sp_reduce.cuh"
 #include "sp_lowp.cuh"
-#include "sp_decode_dev.cuh"
-#include "sp_train_dev.cuh"
+#include "sp_argmax.cuh"
 
 #ifdef SP_TRAIN_TRACE
 __device__ long long* g_loss_trace_ptr = nullptr;     // scratch instrumentation, trace build only
@@ -81,31 +82,28 @@ __device__ __forceinline__ unsigned long long argmax_key(float v, int i) {
 __device__ __forceinline__ float2 key_axis(unsigned long long key, int W) {
     const unsigned int o = (unsigned int)(key >> 32);
     const float v = (o == 0xffffffffu || o == 0u) ? CUDART_NAN_F : __uint_as_float((o & 0x80000000u) ? (o ^ 0x80000000u) : ~o);
-    return sp_trn::axis_of(v, (int)~(unsigned int)key, W);
+    return sp_arg::axis_of(v, (int)~(unsigned int)key, W);
 }
 
 // One warp's share of a map seen through QuadBest (each lane visits its quads in increasing order; 4*bq + bsub is the
 // flat index relative to `first`) merged into the map's key. A NaN or an infinity among them: the exact scan of the
 // n elements at `src` (a superset of what the warp saw, starting at flat index `first`) decides instead.
 template <typename PT>
-__device__ __forceinline__ void merge_quads(const sp_trn::QuadBest& b, const PT* src, float mk, int n, int first, int lane,
+__device__ __forceinline__ void merge_quads(const sp_arg::QuadBest& b, const PT* src, float mk, int n, int first, int lane,
                                             unsigned long long* key) {
-    float v;
-    int i;
+    sp_arg::Peak pk;
     if (__any_sync(SP_FULL, b.poison != b.poison)) {
-        sp_trn::MaskedPredView<PT> view{src, mk};
-        sp_trn::argmax_exact_scan(view, n, lane, v, i);
+        pk = sp_arg::argmax_exact(sp_arg::MaskedPredView<PT>{src, mk}, n, lane);
     } else {
-        v = sp_trn::warp_max_f32(b.best);
-        if (v == -CUDART_INF_F) return;          // the warp had no element of this map (an infinity is poison)
-        i = (int)__reduce_min_sync(SP_FULL, (b.best == v) ? (unsigned)(4 * b.bq + b.bsub) : 0x7fffffffu);
+        pk = b.warp_peak();
+        if (pk.value == -CUDART_INF_F) return;   // the warp had no element of this map (an infinity is poison)
     }
-    if (lane == 0) atomicMax(key, argmax_key(v, first + i));
+    if (lane == 0) atomicMax(key, argmax_key(pk.value, first + pk.index));
 }
 
 // Scalar paths: this lane's first maximal element by sp::better, merged over the warp, then into the map's key.
 __device__ __forceinline__ void merge_scalar(float bv, int bi, int lane, unsigned long long* key) {
-    const sp_dec::Peak pk = sp_dec::warp_best(bv, bi);
+    const sp_arg::Peak pk = sp_arg::warp_best(bv, bi);
     if (lane == 0 && pk.index != 0x7fffffff) atomicMax(key, argmax_key(pk.value, pk.index));
 }
 
@@ -122,7 +120,7 @@ __device__ __forceinline__ void acc_epilogue(const AccOut& A, int* counters) {
         A.label_xy[i] = key_axis(k.y, A.W);
     }
     __syncthreads();
-    sp_trn::heatmap_acc_block<true>(A.pred_xy, A.label_xy, A.acc, A.B, A.K, A.norm_x, A.norm_y, A.thresh, counters);
+    sp_arg::heatmap_acc_block<true>(A.pred_xy, A.label_xy, A.acc, A.B, A.K, A.norm_x, A.norm_y, A.thresh, counters);
 }
 
 // The plain-load kernel: one CTA per map at a time, grid-stride over the maps. It serves every call the ring kernel does
@@ -170,7 +168,7 @@ mse_plain_kernel(const PT* __restrict__ pred, const float* __restrict__ target, 
         if (VEC) {
             const float4* t4 = reinterpret_cast<const float4*>(target + base);
             const int nv = hw >> kLogE;
-            sp_trn::QuadBest bp, bt;
+            sp_arg::QuadBest bp, bt;
             if (ACC) { bp.init(); bt.init(); }
 #pragma unroll kUnroll
             for (int o = threadIdx.x; o < nv; o += kThreads) {
@@ -178,7 +176,7 @@ mse_plain_kernel(const PT* __restrict__ pred, const float* __restrict__ target, 
                 sp_lowp::load_group(pred + base + E * (size_t)o, p);
 #pragma unroll
                 for (int h = 0; h < Q; ++h) {
-                    const float4 v = sp_trn::ldg_stream4(t4 + Q * o + h);
+                    const float4 v = sp_lowp::ldg_stream4(t4 + Q * o + h);
                     t[4 * h] = v.x; t[4 * h + 1] = v.y; t[4 * h + 2] = v.z; t[4 * h + 3] = v.w;
                 }
 #pragma unroll
@@ -291,7 +289,7 @@ mse_ring_kernel(const float* __restrict__ pred, const float* __restrict__ target
         float4* g4 = reinterpret_cast<float4*>(grad + i * chunk_floats);
         float acc = 0.f;
         const bool track = ACC && mk != 0.f;
-        sp_trn::QuadBest bp, bt;
+        sp_arg::QuadBest bp, bt;
         if (ACC) { bp.init(); bt.init(); }
 #pragma unroll 3
         for (int q = lane; q < chunk_quads; q += 32) {

@@ -22,6 +22,11 @@ __device__ __forceinline__ uint4 ldg_stream16(const void* p) {
     asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
     return r;
 }
+__device__ __forceinline__ float4 ldg_stream4(const float4* p) {
+    float4 r;
+    asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
+    return r;
+}
 
 // the 16 bytes at a 16-byte aligned address -> float[16 / sizeof(T)]
 __device__ __forceinline__ void load_group(const float* p, float (&out)[4]) {

@@ -17,6 +17,7 @@
 // instead of 5, in one launch instead of three. Results: coords / maxval / targets / weights / grad / acc axes
 // are bit-identical to the stand-alone kernels; the loss differs only in the float64 summation order.
 #include "sp_common.cuh"
+#include "sp_argmax.cuh"
 #include "sp_decode_dev.cuh"
 #include "sp_train_dev.cuh"
 
@@ -145,8 +146,8 @@ __device__ __forceinline__ void step_body(const sp_dec::DecodeArgs& A, const sp_
                 sum_sq += (double)st.acc;
             } else if (VAL || A.coords != nullptr) {
                 // ---- decode (argmax on the raw map, blur at the 13 stencil points, Taylor step, affine)
-                const sp_dec::Peak pk = sp_dec::argmax_smem<false>(a, a, hw, A.W, lane);
-                sp_dec::DirectView view{a};
+                const sp_arg::Peak pk = sp_dec::argmax_smem<false>(a, a, hw, A.W, lane);
+                sp_arg::DirectView view{a};
                 auto gauss_taylor = [&](int px, int py, float ori_max, float& ox, float& oy) {
                     return sp_dec::taylor_refine_smem<KS>(a, wts, patch, taps, A.H, A.W, px, py, ori_max, lane, ox, oy);
                 };
@@ -194,7 +195,7 @@ __device__ __forceinline__ void step_body(const sp_dec::DecodeArgs& A, const sp_
     const bool last = sp_reduce::finish_loss<512>(sum_sq, ws, loss, inv_count);
     if constexpr (VAL) {
         // every staged map is consumed: the counters go where the per-warp areas were
-        if (last) sp_trn::heatmap_acc_block<true>(io.pred_xy, io.label_xy, V.acc, V.B, A.K, V.norm_x, V.norm_y, V.thresh,
+        if (last) sp_arg::heatmap_acc_block<true>(io.pred_xy, io.label_xy, V.acc, V.B, A.K, V.norm_x, V.norm_y, V.thresh,
                                                   reinterpret_cast<int*>(smem + kHeadBytes + kWtsBytes));
     }
 }

@@ -289,7 +289,7 @@ heatmap_acc_kernel(const float2* __restrict__ pred_xy, const float2* __restrict_
                    int B, int K, float norm_x, float norm_y, float thresh) {
     extern __shared__ int counters[];        // hit[K], valid[K]
     sp::grid_dep_wait();
-    sp_trn::heatmap_acc_block<false>(pred_xy, label_xy, acc, B, K, norm_x, norm_y, thresh, counters);
+    sp_arg::heatmap_acc_block<false>(pred_xy, label_xy, acc, B, K, norm_x, norm_y, thresh, counters);
 }
 
 }  // namespace

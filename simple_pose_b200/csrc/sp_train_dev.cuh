@@ -1,61 +1,25 @@
 // Device-side building blocks of the fused encode + masked-MSE (+ HeatMapAcc) pass over a predicted map,
-// shared by the training kernels (sp_train.cu) and the one-launch step kernel (sp_step.cu). See sp_train.cu.
+// shared by the training kernels (sp_train.cu) and the one-launch step kernel (sp_step.cu). The argmax rule and the
+// HeatMapAcc epilogue are in sp_argmax.cuh. See sp_train.cu.
 #pragma once
 #include "sp_common.cuh"
 #include "sp_gauss.cuh"
 #include "sp_reduce.cuh"
 #include "sp_lowp.cuh"
+#include "sp_argmax.cuh"
 #include <math_constants.h>
 
 namespace sp_trn {
 
 using namespace sp_gauss;
 using namespace sp_reduce;
+using namespace sp_arg;
 
 constexpr int kWarps = 8;
 constexpr int kThreads = kWarps * SP_WARP;
 
-__device__ __forceinline__ float4 ldg_stream4(const float4* p) {
-    float4 r;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];"
-                 : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w)
-                 : "l"(p));
-    return r;
-}
-
-__device__ __forceinline__ float warp_max_f32(float v) {
-    float r;
-    asm volatile("redux.sync.max.f32 %0, %1, 0xffffffff;" : "=f"(r) : "f"(v));
-    return r;
-}
-
-// running (value, quad) argmax over the quads a lane visits in increasing order
-struct QuadBest {
-    float best;
-    int bq;
-    int bsub;          // first element of quad bq that equals best
-    float poison;
-    __device__ __forceinline__ void init() { best = -CUDART_INF_F; bq = 0x0fffffff; bsub = 0; poison = 0.f; }
-    __device__ __forceinline__ void push(float a, float b, float c, float d, int q) {
-        const float m4 = sp::fmax_nan(sp::fmax_nan(a, b), sp::fmax_nan(c, d));
-        poison = fmaf(m4, 0.f, poison);
-        if (m4 > best) {
-            best = m4;
-            bq = q;
-            bsub = (a == m4) ? 0 : (b == m4) ? 1 : (c == m4) ? 2 : 3;
-        }
-    }
-};
-
-template <typename PT = float>
-struct MaskedPredView {          // m * pred[i], straight from global memory (exact fallback only)
-    const PT* p;
-    float m;
-    __device__ __forceinline__ float at(int i) const { return __fmul_rn(m, sp_lowp::to_float(p[i])); }
-};
-
 // quad q (4 consecutive elements) of a map stored as float32 / float16 / bfloat16
-__device__ __forceinline__ float4 load_quad(const float* map, int q) { return ldg_stream4(reinterpret_cast<const float4*>(map) + q); }
+__device__ __forceinline__ float4 load_quad(const float* map, int q) { return sp_lowp::ldg_stream4(reinterpret_cast<const float4*>(map) + q); }
 __device__ __forceinline__ float4 load_quad(const __half* map, int q) {
     const uint2 w = __ldg(reinterpret_cast<const uint2*>(map) + q);
     const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&w.x)), b = __half22float2(*reinterpret_cast<const __half2*>(&w.y));
@@ -74,31 +38,6 @@ __device__ __forceinline__ void store_quad(__half* map, int q, float4 v) {
 __device__ __forceinline__ void store_quad(__nv_bfloat16* map, int q, float4 v) {
     const __nv_bfloat162 a = __floats2bfloat162_rn(v.x, v.y), b = __floats2bfloat162_rn(v.z, v.w);
     reinterpret_cast<uint2*>(map)[q] = make_uint2(*reinterpret_cast<const unsigned*>(&a), *reinterpret_cast<const unsigned*>(&b));
-}
-
-template <typename View>
-__device__ __noinline__ void argmax_exact_scan(const View map, int hw, int lane, float& val, int& idx) {
-    float bv = -CUDART_INF_F;
-    int bi = 0x7fffffff;
-    for (int i = lane; i < hw; i += 32) {
-        const float v = map.at(i);
-        if (sp::better(v, i, bv, bi)) { bv = v; bi = i; }
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const float ov = __shfl_xor_sync(SP_FULL, bv, o);
-        const int oi = __shfl_xor_sync(SP_FULL, bi, o);
-        if (sp::better(ov, oi, bv, bi)) { bv = ov; bi = oi; }
-    }
-    val = bv;
-    idx = bi;
-}
-
-// heat_map_to_axis on an index/value pair: (x, y) as floats, zeroed when the max is not > 0
-__device__ __forceinline__ float2 axis_of(float val, int idx, int W) {
-    if (!(val > 0.f)) return make_float2(0.f, 0.f);
-    const int y = idx / W;
-    return make_float2((float)(idx - y * W), (float)y);
 }
 
 struct MapIo {                 // per-launch constants of the fused kernel
@@ -210,6 +149,31 @@ __device__ __forceinline__ void run_quads(const MapIo& io, int m, const float4* 
     else                   run_quads_impl<WRITE_GRAD, WRITE_TARGETS, ACC, SMEM_PRED, false, PT>(io, m, chunk, q_begin, q_end, jv, ex, ey, st, lane, half_scale);
 }
 
+// Position of x factor i in the period-tiled kernel's layout: the four factors of a quad are split
+// into two planes of (e0, e1) and (e2, e3) pairs, so that the 16-byte shared loads of eight
+// consecutive lanes (consecutive quads of a row) cover 128 contiguous bytes. With the four doubles
+// of a quad contiguous (32-byte lane stride) every such load was a 2-way bank conflict.
+template <int QPR>
+__device__ __forceinline__ int ex_slot(int i) {
+    return QPR > 0 ? (((i >> 2) << 1) + (i & 1) + ((i & 2) ? 2 * QPR : 0)) : i;
+}
+
+// heat_map_to_axis of the masked target fl(mk * t) of a drawn map, found analytically: the factors decrease
+// monotonically away from the centre, so every maximiser of the rounded products lies in the 3x3 block around
+// the nearest in-map pixel. ex is laid out as ex_slot<QPR>.
+template <int QPR>
+__device__ __forceinline__ float2 analytic_target_axis(const MapIo& io, const JointVerdict& jv, float mk, const double* ex,
+                                                       const double* ey, int lane) {
+    const int W = io.W;
+    const int xn = min(max(__float2int_rn(jv.mx), 0), W - 1), yn = min(max(__float2int_rn(jv.my), 0), io.H - 1);
+    const int yy = yn - 1 + lane / 3, xx = xn - 1 + lane % 3;
+    const bool in = lane < 9 && yy >= 0 && yy < io.H && xx >= 0 && xx < W;
+    float v = -CUDART_INF_F;
+    if (in) v = __fmul_rn(mk, __double2float_rn(__dmul_rn(ex[ex_slot<QPR>(xx)], ey[yy])));
+    const Peak pk = warp_first_max(v, in ? (unsigned)(yy * W + xx) : 0x7fffffffu);
+    return axis_of(pk.value, pk.index, W);
+}
+
 // HeatMapAcc coordinates of both masked maps (heat_map_to_axis). The winning quad of the predicted
 // map is re-read from global memory (L2-resident: it has just streamed through), so the staged
 // copy may already have been recycled.
@@ -221,34 +185,15 @@ __device__ __forceinline__ void end_map_acc(const MapIo& io, int m, const JointV
     float2 pxy = make_float2(0.f, 0.f), lxy = make_float2(0.f, 0.f);
     if (st.track) {
         const PT* src = reinterpret_cast<const PT*>(io.pred) + (size_t)m * hw;
-        float pv;
-        int pi;
-        if (__any_sync(SP_FULL, st.bp.poison != st.bp.poison)) {
-            MaskedPredView<PT> view{src, mk};
-            argmax_exact_scan(view, hw, lane, pv, pi);
-        } else {
-            // every lane tracked the first maximal element of its own quads: the smallest flat index
-            // among the lanes that hold the warp-wide maximum is torch.max's answer
-            pv = warp_max_f32(st.bp.best);
-            pi = (int)__reduce_min_sync(SP_FULL, (st.bp.best == pv) ? (unsigned)(4 * st.bp.bq + st.bp.bsub) : 0x7fffffffu);
-        }
-        pxy = axis_of(pv, pi, W);
+        const Peak pp = __any_sync(SP_FULL, st.bp.poison != st.bp.poison) ? argmax_exact(MaskedPredView<PT>{src, mk}, hw, lane)
+                                                                            : st.bp.warp_peak();
+        pxy = axis_of(pp.value, pp.index, W);
         // target map: fl(m * t); always finite
         if (st.analytic_t) {
-            // factors decrease monotonically away from the centre, so every maximiser of the
-            // rounded products lies in the 3x3 block around the nearest in-map pixel
-            const int xn = min(max(__float2int_rn(jv.mx), 0), W - 1), yn = min(max(__float2int_rn(jv.my), 0), io.H - 1);
-            const int yy = yn - 1 + lane / 3, xx = xn - 1 + lane % 3;
-            const bool in = lane < 9 && yy >= 0 && yy < io.H && xx >= 0 && xx < W;
-            float v = -CUDART_INF_F;
-            if (in) v = __fmul_rn(mk, __double2float_rn(__dmul_rn(ex[xx], ey[yy])));
-            const float gmax = warp_max_f32(v);
-            const unsigned gi = __reduce_min_sync(SP_FULL, (in && v == gmax) ? (unsigned)(yy * W + xx) : 0x7fffffffu);
-            lxy = axis_of(gmax, (int)gi, W);
+            lxy = analytic_target_axis<0>(io, jv, mk, ex, ey, lane);
         } else if (jv.draw) {
-            const float gmax = warp_max_f32(st.bt.best);
-            const unsigned gi = __reduce_min_sync(SP_FULL, (st.bt.best == gmax) ? (unsigned)(4 * st.bt.bq + st.bt.bsub) : 0x7fffffffu);
-            lxy = axis_of(gmax, (int)gi, W);
+            const Peak pt = st.bt.warp_peak();
+            lxy = axis_of(pt.value, pt.index, W);
         }
     }
     if (lane == 0) {
@@ -269,15 +214,6 @@ __device__ __forceinline__ Joint3 load_joint(const MapIo& io, int m) {
         j.v = __ldg(io.joints + 3 * (size_t)m + 2);
     }
     return j;
-}
-
-// Position of x factor i in the period-tiled kernel's layout: the four factors of a quad are split
-// into two planes of (e0, e1) and (e2, e3) pairs, so that the 16-byte shared loads of eight
-// consecutive lanes (consecutive quads of a row) cover 128 contiguous bytes. With the four doubles
-// of a quad contiguous (32-byte lane stride) every such load was a 2-way bank conflict.
-template <int QPR>
-__device__ __forceinline__ int ex_slot(int i) {
-    return QPR > 0 ? (((i >> 2) << 1) + (i & 1) + ((i & 2) ? 2 * QPR : 0)) : i;
 }
 
 // joint -> verdict, weight store, float64 factors into this warp's shared-memory slice
@@ -555,35 +491,24 @@ __device__ __forceinline__ float tile_map(const MapIo& io, int m, const JointVer
         if (track) {
             const float* src = io.pred + (size_t)m * hw;
             if (__any_sync(SP_FULL, best != best)) {
-                float pv;
-                int pi;
-                MaskedPredView<float> view{src, mk};
-                argmax_exact_scan(view, hw, lane, pv, pi);
-                if (lane == 0) io.pred_xy[m] = axis_of(pv, pi, io.W);
+                const Peak pk = argmax_exact(MaskedPredView<float>{src, mk}, hw, lane);
+                if (lane == 0) io.pred_xy[m] = axis_of(pk.value, pk.index, io.W);
             } else {
                 // every lane kept the first quad holding its own maximum: the smallest quad among
                 // the lanes that hold the warp-wide maximum contains torch.max's answer
-                const float gmax = warp_max_f32(best);
-                const int gq = (int)__reduce_min_sync(SP_FULL, (best == gmax) ? (unsigned)bq : 0x7fffffffu);
+                const Peak g = warp_first_max(best, (unsigned)bq);
                 pd.m = m;
-                pd.quad = gq;
-                pd.gmax = gmax;
+                pd.quad = g.index;
+                pd.gmax = g.value;
                 pd.mk = mk;
-                pd.v = __ldg(reinterpret_cast<const float4*>(src) + gq);
+                pd.v = __ldg(reinterpret_cast<const float4*>(src) + g.index);
             }
             if (analytic_t) {
-                const int W = io.W;
-                const int xn = min(max(__float2int_rn(jv.mx), 0), W - 1), yn = min(max(__float2int_rn(jv.my), 0), io.H - 1);
-                const int yy = yn - 1 + lane / 3, xx = xn - 1 + lane % 3;
-                const bool in = lane < 9 && yy >= 0 && yy < io.H && xx >= 0 && xx < W;
-                float v = -CUDART_INF_F;
-                if (in) v = __fmul_rn(mk, __double2float_rn(__dmul_rn(ex[ex_slot<QPR>(xx)], ey[yy])));
-                const float gmax = warp_max_f32(v);
-                const unsigned gi = __reduce_min_sync(SP_FULL, (in && v == gmax) ? (unsigned)(yy * W + xx) : 0x7fffffffu);
-                lxy = axis_of(gmax, (int)gi, W);
+                lxy = analytic_target_axis<QPR>(io, jv, mk, ex, ey, lane);
             } else if (track_t) {
-                const float gmax = warp_max_f32(tbest);
-                const int gq = (int)__reduce_min_sync(SP_FULL, (tbest == gmax) ? (unsigned)tbq : 0x7fffffffu);
+                const Peak g = warp_first_max(tbest, (unsigned)tbq);
+                const float gmax = g.value;
+                const int gq = g.index;
                 const int y = gq / QPR, x4 = 4 * (gq - y * QPR);
                 int sub = 3;
 #pragma unroll
@@ -597,46 +522,6 @@ __device__ __forceinline__ float tile_map(const MapIo& io, int m, const JointVer
         if (lane == 0) io.label_xy[m] = lxy;
     }
     return acc;
-}
-
-// HeatMapAcc epilogue (metrics/pose_metrics.py:227-245) on the [B,K] argmax coordinates, run by ALL threads of one
-// block; counters = 2K ints of shared memory. The per-joint counts do not depend on the order the threads add them in
-// and one thread sums the joints in order, so every block size gives the same bits. COHERENT: read the axes through L2
-// (ld.global.cg) because other CTAs of the same launch wrote them (the caller has acquired their writes).
-template <bool COHERENT>
-__device__ __forceinline__ void heatmap_acc_block(const float2* __restrict__ pred_xy, const float2* __restrict__ label_xy,
-                                                  float* __restrict__ acc, int B, int K, float norm_x, float norm_y,
-                                                  float thresh, int* counters) {
-    int* hit = counters;
-    int* valid = counters + K;
-    for (int k = threadIdx.x; k < 2 * K; k += blockDim.x) counters[k] = 0;
-    __syncthreads();
-    const int n = B * K;
-    for (int i = threadIdx.x; i < n; i += blockDim.x) {
-        const float2 l = COHERENT ? __ldcg(label_xy + i) : label_xy[i];
-        if (l.x > 1.f && l.y > 1.f) {
-            const float2 p = COHERENT ? __ldcg(pred_xy + i) : pred_xy[i];
-            const float dx = __fsub_rn(__fdiv_rn(p.x, norm_x), __fdiv_rn(l.x, norm_x));
-            const float dy = __fsub_rn(__fdiv_rn(p.y, norm_y), __fdiv_rn(l.y, norm_y));
-            // torch.norm accumulates float inputs in double on CPU (the pinned oracle); no (dx, dy)
-            // pair of the supported map sizes lands on the threshold, so float vs double is moot
-            const float dist = (float)sqrt((double)dx * (double)dx + (double)dy * (double)dy);
-            const int k = i % K;
-            atomicAdd(&valid[k], 1);
-            if (dist < thresh) atomicAdd(&hit[k], 1);
-        }
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        float sum = 0.f;
-        int used = 0;
-        for (int k = 0; k < K; ++k) {
-            if (valid[k] < 1) continue;
-            sum = __fadd_rn(sum, __fdiv_rn((float)hit[k], (float)valid[k]));
-            ++used;
-        }
-        acc[0] = used > 0 ? __fdiv_rn(sum, (float)used) : 0.f;
-    }
 }
 
 }  // namespace sp_trn
