@@ -405,7 +405,13 @@ def heat_map_acc(predicts, targets, distance_thresh=0.5, norm_frac=10.):
     that have at least one such person."""
     p, _ = argmax_coords(predicts)
     t, _ = argmax_coords(targets)
-    norm = torch.tensor([predicts.shape[-1], predicts.shape[-2]], dtype=torch.float) / norm_frac
+    return heat_map_acc_from_axes(p, t, predicts.shape[-2], predicts.shape[-1], distance_thresh, norm_frac)
+
+
+def heat_map_acc_from_axes(p, t, height, width, distance_thresh=0.5, norm_frac=10.):
+    """The epilogue of ``heat_map_acc`` (metrics/pose_metrics.py:225-245) on the two [B,K,2] float32
+    ``argmax_coords`` tables ``p`` (predictions) and ``t`` (targets) of [B,K,height,width] maps."""
+    norm = torch.tensor([width, height], dtype=torch.float) / norm_frac
     ok = (t[..., 0] > 1) & (t[..., 1] > 1)
     dist = torch.norm(p / norm - t / norm, dim=-1)
     dist[~ok] = -1.

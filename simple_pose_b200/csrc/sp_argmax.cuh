@@ -98,8 +98,9 @@ __device__ __forceinline__ float2 axis_of(float val, int idx, int W) {
 }
 
 // HeatMapAcc epilogue (metrics/pose_metrics.py:227-245) on the [B,K] argmax coordinates, run by ALL threads of one
-// block; counters = 2K ints of shared memory. The per-joint counts do not depend on the order the threads add them in
-// and one thread sums the joints in order, so every block size gives the same bits. COHERENT: read the axes through L2
+// block; counters = 2K ints of shared memory. Every step is a correctly rounded float32 operation in the oracle's order
+// (divide, subtract, the distance below, compare), so each verdict is the oracle's. The per-joint counts do not depend
+// on the order the threads add them in and one thread sums the joints in order, so every block size gives the same bits. COHERENT: read the axes through L2
 // (ld.global.cg) because other CTAs of the same launch wrote them (the caller has acquired their writes).
 template <bool COHERENT>
 __device__ __forceinline__ void heatmap_acc_block(const float2* __restrict__ pred_xy, const float2* __restrict__ label_xy,
@@ -116,9 +117,11 @@ __device__ __forceinline__ void heatmap_acc_block(const float2* __restrict__ pre
             const float2 p = COHERENT ? __ldcg(pred_xy + i) : pred_xy[i];
             const float dx = __fsub_rn(__fdiv_rn(p.x, norm_x), __fdiv_rn(l.x, norm_x));
             const float dy = __fsub_rn(__fdiv_rn(p.y, norm_y), __fdiv_rn(l.y, norm_y));
-            // torch.norm accumulates float inputs in double on CPU (the pinned oracle); no (dx, dy)
-            // pair of the supported map sizes lands on the threshold, so float vs double is moot
-            const float dist = (float)sqrt((double)dx * (double)dx + (double)dy * (double)dy);
+            // torch.norm(d, dim=-1) of a float32 pair on the CPU (the pinned oracle) is sqrtf(fmaf(dy, dy, dx * dx)),
+            // in float32 (tests/test_heatmap_acc_norm_cpu.py pins it). A double sum rounded once differs in the last
+            // bit for about one offset in nine, and some of those lie on the threshold: at 100 x 100 with the defaults,
+            // pred (0, 3) and label (3, 7) are 0.49999997 apart, a hit, where the double form gives 0.5, a miss.
+            const float dist = __fsqrt_rn(__fmaf_rn(dy, dy, __fmul_rn(dx, dx)));
             const int k = i % K;
             atomicAdd(&valid[k], 1);
             if (dist < thresh) atomicAdd(&hit[k], 1);

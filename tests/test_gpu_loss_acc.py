@@ -278,7 +278,7 @@ def test_loss_acc_against_the_oracle(b, hw):
     got = one_pass(pred, target, mask, True)
     p, t, m = pred.cpu(), target.cpu(), mask.cpu()[..., None, None]
     ref_acc = O.heat_map_acc(p * m, t * m)
-    assert abs(got["acc"].item() - float(ref_acc)) <= 1e-6
+    assert got["acc"].item() == float(ref_acc)             # float32 values: equal as doubles iff equal as floats
     ref_loss = O.masked_mse_loss(p, t, mask.cpu())
     assert abs(got["loss"].item() - ref_loss.item()) <= 1e-5 * abs(ref_loss.item())
 

@@ -145,7 +145,7 @@ def test_fused_encode_loss_native_half_precision_pred(dtype):
     loss, acc = crit(p, joints.to(DEV))
     (loss * scale).backward()
     assert abs(loss.item() - ref_loss.item()) <= 1e-5 * abs(ref_loss.item())
-    assert abs(acc.item() - float(ref_acc)) <= 1e-6
+    assert acc.item() == float(ref_acc)
     assert torch.equal(crit.weights.cpu(), msk)
     d = half_ulp_distance(p.grad.cpu(), ref_grad)
     assert p.grad.dtype == dtype and int(d.max()) <= 1 and float((d != 0).float().mean()) < 1e-3
@@ -209,7 +209,7 @@ def test_train_loop_of_the_hrnet_solver(amp, fused_targets):
         ref_loss, ref_grad = reference_loss_and_grad(p_host, tgt, msk, scale)
         assert abs(loss.item() - ref_loss.item()) <= 1e-5 * abs(ref_loss.item())
         ref_acc = O.heat_map_acc(p_host.float() * msk[..., None, None], tgt * msk[..., None, None])
-        assert abs(acc.item() - float(ref_acc)) <= 1e-6
+        assert acc.item() == float(ref_acc)
         g = captured["grad"]
         assert g.dtype == predicts.dtype and g.shape == predicts.shape
         if amp:
@@ -250,7 +250,7 @@ def test_val_loop_of_the_hrnet_solver():
             ref_loss = O.masked_mse_loss(p_host, t_host, m_host)
             assert abs(loss.item() - ref_loss.item()) <= 1e-5 * abs(ref_loss.item())
             ref_acc = O.heat_map_acc(p_host * m_host[..., None, None], t_host * m_host[..., None, None])
-            assert abs(acc.item() - float(ref_acc)) <= 1e-6
+            assert acc.item() == float(ref_acc)
             want_xy, want_conf = O.gauss_taylor_decode(p_host, tran_inv.cpu())
             mag = float(tran_inv[:, 0, 0].abs().max())
             assert (pred_kps.cpu() - want_xy).abs().max().item() <= 1e-4 * mag + 1e-3

@@ -169,7 +169,7 @@ def test_val_step_against_the_oracle(decoder, b, hw):
     ref_loss = O.masked_mse_loss(p_host, tgt, msk)
     assert abs(loss.item() - ref_loss.item()) <= 1e-5 * abs(ref_loss.item())
     ref_acc = O.heat_map_acc(p_host * msk[..., None, None], tgt * msk[..., None, None])
-    assert abs(acc.item() - float(ref_acc)) <= 1e-6
+    assert acc.item() == float(ref_acc)
     want_xy, want_conf = (O.gauss_taylor_decode if decoder == "gauss_taylor" else O.basic_decode)(p_host, t_inv)
     mag = float(t_inv[:, 0, 0].abs().max())
     assert (hp.coords.cpu() - want_xy).abs().max().item() <= 1e-4 * mag + 1e-3
@@ -222,7 +222,7 @@ def test_val_loop_of_the_resnet_solvers():
             ref_loss = creterion(predicts.clone(), targets, mask)
             ref_acc = acc_func(predicts.mul(mask[..., None, None]), targets.mul(mask[..., None, None]))
             assert abs(loss.item() - ref_loss.item()) <= 1e-5 * abs(ref_loss.item())
-            assert abs(acc.item() - ref_acc.item()) <= 1e-6
+            assert acc.item() == ref_acc.item()
             pred_kps, scores = decoder(predicts, tran_inv)
             ref_rows.append(person_rows(pred_kps, scores))
     got, want = torch.cat(val_rows), torch.cat(ref_rows)
